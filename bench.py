@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the environment-step hot path (BASELINE.json config 2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs E] [--dump-outputs DIR]
 
 Workload (per GPU, weak scaling): ``MultiAgentInvManagement`` 4-stage chain in preset MA_6 mode
 (hyperparams.py:482-484), 65 536 environments, replayed Poisson(5) demand, host-random uniform
@@ -586,6 +586,9 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
     elapsed = e0.elapsed_time(e1) * 1e-3
+    # device copies of the last timed episode's outputs, taken before the replays below overwrite the buffers; they reach
+    # the host only after the clocks have been sampled
+    dumped = sample_outputs(obs0, obs_all, rew, final_stats) if args.dump_outputs and rank == 0 else None
     if os.environ.get("IMX_BENCH_DEBUG"):
         print(f"[rank {rank}] elapsed {elapsed * 1e3:.3f} ms for {args.steps} steps", file=sys.stderr, flush=True)
     # keep the GPU busy a little longer so that the 100 ms clock sampler sees the kernel under load
@@ -697,8 +700,38 @@ def run_ours(args):
             "episode_stats": {"n": float(final_stats[0].item()), "mean_return": float((final_stats[1] / final_stats[0]).item())},
         }
         print(json.dumps(line), flush=True)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_ENVS = 4096
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def sample_outputs(obs0, obs_all, rew, stats):
+    """Device copies of what the last timed episode returned to its caller: the reset observations, the 30 periods'
+    observations and rewards, and the episode statistics accumulated over the timed steps.  Per-env arrays keep a fixed,
+    seeded sample of DUMP_ENVS envs (all of them when there are fewer), the same in every run, so that two builds can be
+    compared output for output."""
+    import torch
+    N = obs0.shape[0]
+    keep = np.sort(np.random.default_rng(0).choice(N, size=min(N, DUMP_ENVS), replace=False))
+    idx = torch.as_tensor(keep, device=obs0.device)
+    return {"obs_reset": obs0.index_select(0, idx), "obs": obs_all.index_select(1, idx), "reward": rew.index_select(1, idx),
+            "episode_stats": stats.clone()}
+
+
+def write_outputs(out_dir, sampled):
+    """sample_outputs' arrays as float64 DIR/<name>.npy files."""
+    arrays = {k: v.double().cpu().numpy() for k, v in sampled.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs would write {total} bytes (limit {DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def large_n_roofline(torch, dev, peak, N=4 * 1024 * 1024, periods=8):
@@ -786,7 +819,13 @@ def main():
     ap.add_argument("--skip-large", action="store_true")
     ap.add_argument("--skip-configs", action="store_true", help="skip BASELINE configs 3 / 4 / 5 (the `configs` object of the line)")
     ap.add_argument("--large-only", action="store_true", help="only the 4 Mi-env roofline point (used for the ncu capture)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last timed episode's observations, "
+                    "rewards and episode statistics (a fixed sample of envs, float64) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.large_only or args.impl == "reference"):
+        ap.error("--dump-outputs writes the outputs of the timed GPU path; it does not apply to --large-only or --impl reference")
     if args.large_only:
         import torch
         peak = float(json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"]) if os.path.exists(os.path.join(ROOT, "MEASURED_PEAKS.json")) else 6650.0

@@ -1,5 +1,5 @@
-"""TEST INFRASTRUCTURE — loader for the UNMODIFIED reference envs (only works where
-/root/reference exists, i.e. in the build container, never on the GPU box).
+"""TEST INFRASTRUCTURE — loader for the UNMODIFIED reference envs (only works where a checkout of the
+reference is present: IMX_REFERENCE_ROOT, default oracle/_ref, which git ignores).
 
 The reference (MarwanMousa/MARL-for-IM) is pure Python and needs `gym` and
 `ray.rllib` only for two base classes and `gym.spaces.Box`; neither package is
@@ -19,7 +19,7 @@ import sys
 import types
 import warnings
 
-REFERENCE_ROOT = os.environ.get("IMX_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("IMX_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def reference_available() -> bool:

@@ -1,6 +1,6 @@
 """Shared trajectory runners for the parity tests.
 
-``run_reference`` drives the UNMODIFIED reference env (build container only),
+``run_reference`` drives the UNMODIFIED reference env (only where its source tree is present, see oracle/ref_import.py),
 ``run_oracle`` drives oracle/im_oracle.py; both return the same dict of arrays so the
 tests can compare them (and the CUDA path) field by field:
 

@@ -140,9 +140,13 @@ int imx_destroy(imx_env* env);
  * does this for the variants its batch size selects; call imx_prepare() to force the rest.
  *   flags: IMX_PREPARE_STEP (observation-writing step / step_many / rollout kernels), IMX_PREPARE_NOOBS (the
  *          obs_dev = NULL specialisation), IMX_PREPARE_HOST (staging buffers + stream of the *_host calls),
- *          IMX_PREPARE_DFO (scratch of the dfo objective), IMX_PREPARE_CC (imx_step_cc's specialisation and scratch);
- *          0 = all.  Synchronous; may take seconds (NVRTC). */
-enum imx_prepare_flags { IMX_PREPARE_STEP = 1, IMX_PREPARE_NOOBS = 2, IMX_PREPARE_HOST = 4, IMX_PREPARE_DFO = 8, IMX_PREPARE_CC = 16 };
+ *          IMX_PREPARE_DFO (scratch of the dfo objective), IMX_PREPARE_CC (imx_step_cc's specialisation and scratch),
+ *          IMX_PREPARE_EPISODE (imx_replay_episode's two episode kernels, with and without observations, and the scratch
+ *          buffers of its unfused form: [T][N](m) rewards, [N][m][O] observations, [N][m] profits, [N](m) returns);
+ *          0 = the first five (STEP | NOOBS | HOST | DFO | CC; not EPISODE, so existing callers compile nothing more).
+ *          Synchronous; may take seconds (NVRTC). */
+enum imx_prepare_flags { IMX_PREPARE_STEP = 1, IMX_PREPARE_NOOBS = 2, IMX_PREPARE_HOST = 4, IMX_PREPARE_DFO = 8, IMX_PREPARE_CC = 16,
+                         IMX_PREPARE_EPISODE = 32 };
 int imx_prepare(imx_env* env, int flags);
 
 /* Derived sizes: O (observation length per agent), S (int32 state words per env), R, L, NB. */
@@ -191,6 +195,25 @@ int imx_step(imx_env* env, const double* actions_dev, void* obs_dev, double* rew
  *   array_acquisition records of the LP replay loops, DSHLP_4.py:918-923). */
 int imx_step_many(imx_env* env, const double* actions_dev, int K, void* obs_dev, double* reward_dev,
                   const imx_info_out* info, void* stream);
+
+/* One whole episode on a stored plan: reset(customer_demand) + T step() calls + the episode's returns / statistics
+ * (+ the evaluation loops' accumulators), i.e. the LP scripts' replay loop (DSHLP_4.py:896-928).  Bit-identical to
+ *   imx_reset(env, demand_dev, delay_mask_dev, noisy, episode, NULL, s);
+ *   imx_step_many(env, actions_dev, T, obs_dev, reward, NULL, s);                 (reward: reward_dev or scratch)
+ *   imx_episode_stats(env, reward, T, return_dev, stats_dev, accumulate, s);       (when return_dev or stats_dev)
+ *   imx_eval_accumulate(env, obs[t], reward[t], profit[t], eval_acc_dev, t == 0, s) for t < T   (when eval_acc_dev)
+ * actions_dev [T][N][m]; obs_dev [T][N][m][O] or NULL; reward_dev [T][N][m] / [T][N] or NULL; return_dev [N][m] / [N] or NULL;
+ * stats_dev [3 + 2m] / [3] or NULL; eval_acc_dev [N][4 + m] or NULL.  Leaves the env at period T with the final state
+ * (every state field, the split's error flags).  demand_dev / delay_mask_dev / noisy / episode as in imx_reset: NULL draws
+ * from the same Philox streams.  Works from any current period (it is a reset).
+ * Where the runtime-specialised kernels serve the whole batch with one tile per CTA (N a multiple of the tile, 16-byte aligned
+ * buffers, the tile's [E][R][T] trace fitting in shared memory) this is ONE kernel launch, plus the two statistics launches of
+ * imx_return_stats when stats_dev is given; imx_kernel_variant() then returns 4.  That kernel reads the trace and the mask in
+ * place, so on that path IMX_F_DEMAND and IMX_F_DELAY_MASK are NOT rewritten.  Elsewhere the library runs the composition
+ * itself; its scratch buffers are allocated on first use, or by imx_prepare(IMX_PREPARE_EPISODE) — needed under capture. */
+int imx_replay_episode(imx_env* env, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
+                       const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
+                       double* stats_dev, int accumulate, double* eval_acc_dev, void* stream);
 
 /* dfo_func's loop  —  base_restock_policy.py:24-45 with base_stock_policy :4-21 fused in: a whole
  * K = T period episode per env in ONE kernel, state on chip.
@@ -276,13 +299,14 @@ int imx_poisson_cdf(const imx_env* env, double* out, int cap);
 
 /* Which kernel served the last step()/rollout of this handle: 0 ahead-of-time direct kernel,
  * 1 ahead-of-time TMA-staged kernel, 2 runtime-specialised (NVRTC, same sources, flags as literals),
- * 3 runtime-specialised persistent pipeline (imx_step_pipe.cuh). */
+ * 3 runtime-specialised persistent pipeline (imx_step_pipe.cuh), 4 the one-launch episode kernel (imx_replay_episode). */
 int imx_kernel_variant(const imx_env* env);
 /* Last message of the runtime-specialisation layer (why it is unavailable, or a compile log). */
 const char* imx_jit_log(void);
 /* Compiles the specialised kernels for `cfg` with NVRTC for sm_100a WITHOUT a GPU (build check; also warms the on-disk
  * cubin cache).  variant: 0 = the step / step_many / rollout / pipelined kernels, 1 = the same without observations
- * (obs_dev = NULL), 2 = with the centralised-critic rows (imx_step_cc).
+ * (obs_dev = NULL), 2 = with the centralised-critic rows (imx_step_cc), 3 = imx_replay_episode's episode kernel,
+ * 4 = the same without observations.
  * Returns the cubin size in bytes, or a negative error; `log` receives the compiler log. */
 int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap);
 

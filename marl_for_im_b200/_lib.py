@@ -12,6 +12,7 @@ MAX_NODES, MAX_CHILDREN, MAX_DELAY, MAX_HIST = 32, 8, 8, 8
 ABI_VERSION = 3          # IMX_ABI_VERSION of include/imx_b200.h this binding mirrors
 KIND = {"IM": 0, "MAIM": 1, "IM_div": 2, "MAIM_div": 3}
 DIST = {"replay": 0, "custom": 0, "poisson": 1, "uniform": 2}
+PREPARE_EPISODE = 32    # IMX_PREPARE_EPISODE: imx_replay_episode's kernels and scratch (imx_prepare)
 F_INV, F_BACKLOG, F_ORDER_U, F_PIPE, F_HIST_D, F_HIST_O, F_CARRY, F_BACKLOG_TO, F_ERROR, F_DEMAND, F_DELAY_MASK = range(11)
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libimx_b200.so")
@@ -62,6 +63,7 @@ SYMBOLS = {
     "imx_reset": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P]),
     "imx_step": (C.c_int, [_P, _P, _P, _P, C.POINTER(ImxInfoOut), _P]),
     "imx_step_many": (C.c_int, [_P, _P, C.c_int, _P, _P, C.POINTER(ImxInfoOut), _P]),
+    "imx_replay_episode": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, C.c_int, _P, _P]),
     "imx_rollout_basestock": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, C.c_int, _P]),
     "imx_prepare": (C.c_int, [_P, C.c_int]),
     "imx_step_cc": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_double, C.c_double, _P, _P]),

@@ -144,8 +144,15 @@ struct imx_env {
     const imxjit::Kernels* jit_cc = nullptr;      // specialised with the centralised-critic rows emitted by the step (imx_step_cc)
     int jit_cc_state = 0;
     TileLayout tile_cc = {};             // tile_jit + the [E][m][W] critic-row region
-    void* d_obs_scratch = nullptr;       // [N][m][O] observations of the unfused imx_step_cc fallback when the caller passes none
-    int last_variant = 0;                // 0 AOT direct, 1 AOT TMA, 2 runtime-specialised TMA
+    void* d_obs_scratch = nullptr;       // [N][m][O] observations of the unfused imx_step_cc / imx_replay_episode when the caller passes none
+    const imxjit::Kernels* jit_ep = nullptr;        // the one-launch episode kernel (imx_replay_episode) with observations ...
+    const imxjit::Kernels* jit_ep_noobs = nullptr;  // ... and without
+    int jit_ep_state = 0, jit_ep_noobs_state = 0;
+    double* d_ep_rewards = nullptr;      // [T][N](m) rewards of the unfused imx_replay_episode when the caller passes none
+    double* d_ep_profit = nullptr;       // [N][m] one period's profits (unfused imx_replay_episode with evaluation accumulators)
+    double* d_ep_ret = nullptr;          // [N](m) returns of imx_replay_episode when only the statistics are wanted
+    double* d_ep_stats = nullptr;        // [3 + 2m] statistics of the unfused imx_replay_episode when only the returns are wanted
+    int last_variant = 0;                // 0 AOT direct, 1 AOT TMA, 2 runtime-specialised TMA, 3 pipelined, 4 one-launch episode
     reset_fn_t reset_fn = nullptr;
     rollout_fn_t rollout_fn = nullptr;
     int step_grid_cap = 0, rollout_grid_cap = 0;
@@ -257,7 +264,8 @@ static int pipe_stages_for(const imx_env* e, const TileLayout& L) {
     return s;
 }
 
-static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1, int has_cc = 0) {
+// episode != 0: the module holds the one-launch episode kernel only (imx_replay_episode)
+static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1, int has_cc = 0, int episode = 0) {
     std::vector<std::string>& defs = sp.defines;
     const imx_config& c = e->cfg;
     const bool always_std = (c.kind == IMX_KIND_MAIM_DIV);
@@ -315,6 +323,7 @@ static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1
     defs.push_back("IMX_HOST_SIZEOF_STEPARGS=" + std::to_string(sizeof(StepArgs)));
     defs.push_back("IMX_HOST_SIZEOF_TILELAYOUT=" + std::to_string(sizeof(TileLayout)));
     defs.push_back("IMX_HOST_SIZEOF_ROLLOUTARGS=" + std::to_string(sizeof(RolloutArgs)));
+    defs.push_back("IMX_HOST_SIZEOF_EPISODEARGS=" + std::to_string(sizeof(EpisodeArgs)));
     const int mp = e->step_dense ? e->m : m_pad_of(e);     // step kernel: power-of-two tile width (see select_kernels)
     const int pmax = (e->need_hd || e->need_ho) ? e->P : 1;
     const int maxc = e->maxc > 1 ? e->maxc : 1;
@@ -389,6 +398,11 @@ static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1
         if (pr && atoi(pr) > 0) defs.push_back("IMX_PIPE_MAXNREG=" + std::to_string(atoi(pr)));
         sp.name[3] = "imx::step_kernel_pipe" + targs;
     }
+    sp.name[4] = "";
+    if (episode) {
+        for (int k = 0; k < 4; ++k) sp.name[k] = "";
+        sp.name[4] = "imx::step_kernel_tma_episode" + targs;
+    }
 }
 
 static void jit_smem(const imx_env* e, int smem[imxjit::N_KERNELS]) {
@@ -396,6 +410,7 @@ static void jit_smem(const imx_env* e, int smem[imxjit::N_KERNELS]) {
     smem[1] = e->tile_jit.total2 <= 200 * 1024 ? e->tile_jit.total2 : e->tile_jit.total;
     smem[2] = 0;
     smem[3] = pipe_stages_for(e, e->tile_jit) * e->tile_jit.total;
+    smem[4] = 0;
 }
 
 // Loads the specialised kernels for this handle (large batches, or IMX_JIT=1).  Called from imx_create() /
@@ -442,6 +457,38 @@ static void ensure_jit_cc(imx_env* e) {
     if (smem[3] > 200 * 1024) smem[3] = 0;
     e->jit_cc = imxjit::get(sp, smem, e->cfg.device);
     if (e->jit_cc) e->jit_cc_state = 1;
+}
+
+// Shared-memory layout of the episode kernel: tile_jit's multi-period layout, then the episode regions of EpisodeArgs that the
+// call needs (the returns and the accumulators adjacent: the kernel zeroes [off_ret, off_prof) in one loop) — a launch reserves
+// no bytes it does not use, since resident CTAs per SM bound this latency-bound loop.  Returns the total bytes.
+static int64_t episode_layout(const imx_env* e, EpisodeArgs& EA, bool ret = true, bool eval = true) {
+    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1;
+    int64_t off = e->tile_jit.total2;
+    auto take = [&](int64_t bytes) { const int64_t o = off; off += (bytes + 127) & ~(int64_t)127; return (int32_t)(o < (1 << 30) ? o : 0); };
+    EA.off_edem = take(E * e->R * e->T * 4);
+    EA.off_ret = take(ret ? E * cols * 8 : 0);
+    EA.off_eval = take(eval ? E * (EVAL_FIXED + e->m) * 8 : 0);
+    EA.off_prof = take(eval ? E * e->m * 8 : 0);
+    EA.total = (int32_t)(off < (1 << 30) ? off : 0);
+    return off;
+}
+
+// The episode kernel, with (obs) or without observations.  Compiled by imx_prepare(IMX_PREPARE_EPISODE) or on first use
+// outside stream capture; unavailable where the specialised kernels are (small batches) or the layout exceeds 200 KB.
+static void ensure_jit_episode(imx_env* e, bool obs) {
+    int& st = obs ? e->jit_ep_state : e->jit_ep_noobs_state;
+    if (st != 0) return;
+    st = -1;
+    ensure_jit(e);
+    EpisodeArgs EA;
+    if (e->jit_state != 1 || episode_layout(e, EA) > 200 * 1024) return;
+    imxjit::Spec sp;
+    jit_spec(e, e->TL, sp, obs ? 1 : 0, 0, 1);
+    const int smem[imxjit::N_KERNELS] = {0, 0, 0, 0, EA.total};
+    const imxjit::Kernels* k = imxjit::get(sp, smem, e->cfg.device);
+    (obs ? e->jit_ep : e->jit_ep_noobs) = k;
+    if (k) st = 1;
 }
 
 static bool stream_is_capturing(cudaStream_t s) {
@@ -880,6 +927,7 @@ extern "C" int imx_destroy(imx_env* e) {
     cudaFree(e->d_nodes); cudaFree(e->d_state); cudaFree(e->d_err);
     cudaFree(e->d_demand_T); cudaFree(e->d_mask_T); cudaFree(e->d_cdf); cudaFree(e->d_guide); cudaFree(e->d_tab); cudaFree(e->d_stats_partial);
     cudaFree(e->d_dfo_rewards); cudaFree(e->d_obs_scratch);
+    cudaFree(e->d_ep_rewards); cudaFree(e->d_ep_profit); cudaFree(e->d_ep_ret); cudaFree(e->d_ep_stats);
     cudaFree(e->d_act_h); cudaFree(e->d_obs_h); cudaFree(e->d_rew_h); cudaFree(e->d_dem_h); cudaFree(e->d_mask_h);
     delete e;
     return 0;
@@ -1199,6 +1247,7 @@ static int ensure_host_path(imx_env* e);
 extern "C" int imx_prepare(imx_env* e, int flags) {
     if (!e) return fail(-1, "null env");
     IMX_CUDA(cudaSetDevice(e->cfg.device));
+    // (0 keeps meaning the five flags it always meant: IMX_PREPARE_EPISODE compiles two more modules and is asked for explicitly)
     if (flags == 0) flags = IMX_PREPARE_STEP | IMX_PREPARE_NOOBS | IMX_PREPARE_HOST | IMX_PREPARE_DFO | IMX_PREPARE_CC;
     if (flags & IMX_PREPARE_STEP) ensure_jit(e);
     if (flags & IMX_PREPARE_NOOBS) ensure_jit_noobs(e);
@@ -1209,6 +1258,16 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
     }
     if ((flags & IMX_PREPARE_DFO) && !e->multi && !e->d_dfo_rewards)
         IMX_CUDA(cudaMalloc(&e->d_dfo_rewards, (size_t)e->T * e->N * sizeof(double)));
+    if (flags & IMX_PREPARE_EPISODE) {                     // both episode modules + every scratch buffer of the unfused form
+        ensure_jit_episode(e, true);
+        ensure_jit_episode(e, false);
+        const size_t cols = e->multi ? e->m : 1, cells = (size_t)e->N * e->m;
+        if (!e->d_ep_rewards) IMX_CUDA(cudaMalloc(&e->d_ep_rewards, (size_t)e->T * e->N * cols * sizeof(double)));
+        if (!e->d_ep_profit) IMX_CUDA(cudaMalloc(&e->d_ep_profit, cells * sizeof(double)));
+        if (!e->d_ep_ret) IMX_CUDA(cudaMalloc(&e->d_ep_ret, (size_t)e->N * cols * sizeof(double)));
+        if (!e->d_ep_stats) IMX_CUDA(cudaMalloc(&e->d_ep_stats, (3 + 2 * (size_t)e->m) * sizeof(double)));
+        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, cells * e->O * (e->cfg.obs_f32 ? 4 : 8)));
+    }
     IMX_CUDA(cudaDeviceSynchronize());
     return 0;
 }
@@ -1244,6 +1303,131 @@ extern "C" int imx_step_many(imx_env* e, const double* actions_dev, int K, void*
         if (rc) return rc;
         j += adv;
     }
+    return 0;
+}
+
+static int launch_return_stats(imx_env* e, const double* src, int periods, bool fused, double* ret_out, double* stats_dev, int accumulate,
+                               cudaStream_t s);
+
+// A whole stored-plan episode: reset + T steps + returns / statistics / evaluation accumulators.  One launch of the episode
+// kernel (plus the two statistics launches over the returns) wherever the runtime-specialised build serves the whole batch
+// with one tile per CTA; otherwise the composition of the existing calls, with the same results.
+extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
+                                  const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
+                                  double* stats_dev, int accumulate, double* eval_acc_dev, void* stream) {
+    IMX_NVTX("imx_replay_episode");
+
+    if (!e || !actions_dev) return fail(-1, "null argument");
+    if ((noisy || delay_mask_dev) && !e->has_carry) return fail(-1, "noisy delay requested but the env was created with noisy_delay = 0");
+    if (!demand_dev && e->cfg.demand_dist == IMX_DIST_REPLAY_ONLY)
+        return fail(-1, "imx_replay_episode without a demand trace needs demand_dist poisson or uniform");
+    IMX_CUDA(cudaSetDevice(e->cfg.device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool capturing = stream_is_capturing(s);
+    const int64_t N = e->N;
+    const int m = e->m;
+    const size_t cols = e->multi ? m : 1, cells = (size_t)N * m, es = e->cfg.obs_f32 ? 4 : 8;
+    if (!capturing) ensure_jit_episode(e, obs_dev != nullptr);
+    const imxjit::Kernels* jk = obs_dev ? e->jit_ep : e->jit_ep_noobs;
+    EpisodeArgs EA;
+    memset(&EA, 0, sizeof(EA));
+    const int64_t smem = episode_layout(e, EA, return_dev || stats_dev, eval_acc_dev != nullptr);
+    const int64_t E = e->tile_jit.E;
+    const auto aligned16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
+    // the legality of imx_step_many's fused form (whole tiles, N % 4, 16-byte aligned buffers, a layout that fits), and the
+    // replayed trace's per-tile block [E][R][T] must be a whole number of 16-byte units
+    // divergent networks (measured, profiles/r3_replay_episode.jsonl): the episode kernel is ahead where the period body is the
+    // env-per-thread one and observations are written (div2 +3 %), and where it is lane-mapped without observations (div1 +1 to
+    // +6 %); in the other two cases its larger resident layout costs more than the bookkeeping it saves (div2 without observations
+    // -7 to -12 %, div1 with observations -6 % at 32 768 envs), so the composition serves them
+    const bool pays = !e->div || (e->step_et ? obs_dev != nullptr : obs_dev == nullptr);
+    const bool fused = pays && jk && jk->step_episode && e->step_path != 1 && e->fuse_periods && N % 4 == 0 && N % E == 0 && E % 2 == 0 &&
+                       smem <= 200 * 1024 && aligned16(actions_dev) && aligned16(obs_dev) && aligned16(reward_dev) && aligned16(return_dev) &&
+                       aligned16(eval_acc_dev) && (!demand_dev || (aligned16(demand_dev) && (E * e->R * e->T) % 4 == 0));
+    // internal buffers are allocated here (never under capture: imx_prepare(IMX_PREPARE_EPISODE) allocates them up front),
+    // before anything is launched
+    auto scratch = [&](void** p, size_t bytes) -> int {
+        if (*p) return 0;
+        if (capturing) return fail(-1, "imx_replay_episode needs an internal buffer under stream capture: call imx_prepare(IMX_PREPARE_EPISODE) first");
+        IMX_CUDA(cudaMalloc(p, bytes));
+        return 0;
+    };
+    int rc = 0;
+    if (fused) {
+        double* ret = return_dev;
+        if (!ret && stats_dev) {                              // the statistics read the returns: keep them in a scratch row
+            if ((rc = scratch((void**)&e->d_ep_ret, (size_t)N * cols * sizeof(double)))) return rc;
+            ret = e->d_ep_ret;
+        }
+        StepArgs A;
+        fill_args(e, A);
+        A.t = 0;
+        A.noisy = (noisy || delay_mask_dev) ? 1 : 0;
+        A.periods = e->T;
+        A.act_stride = (int64_t)cells;
+        A.obs_stride_bytes = (int64_t)(cells * e->O * es);
+        A.rew_stride = (int64_t)(N * cols);
+        A.actions = actions_dev;
+        A.obs = (double*)obs_dev;
+        A.reward = reward_dev;
+        EA.demand = demand_dev;
+        EA.mask = delay_mask_dev;
+        EA.ret = ret;
+        EA.eval = eval_acc_dev;
+        EA.gen = make_gen(e, episode);
+        EA.delay_thr = e->cfg.noisy_delay_threshold;
+        EA.rescaled = (e->cfg.kind == IMX_KIND_MAIM_DIV || e->cfg.standardise_state) ? 1 : 0;
+        void* params[] = {(void*)&A, (void*)&e->tile_jit, (void*)&EA};
+        CUlaunchConfig lc;
+        memset(&lc, 0, sizeof(lc));
+        lc.gridDimX = (unsigned)(N / E); lc.gridDimY = 1; lc.gridDimZ = 1;
+        lc.blockDimX = (unsigned)e->jit_threads; lc.blockDimY = 1; lc.blockDimZ = 1;
+        lc.sharedMemBytes = (unsigned)smem;
+        lc.hStream = (CUstream)s;
+        CUlaunchAttribute at[1];
+        at[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
+        at[0].value.programmaticStreamSerializationAllowed = 1;
+        lc.attrs = at;
+        lc.numAttrs = e->use_pdl ? 1 : 0;
+        const CUresult cr = imxjit::g_api.LaunchKernelEx(&lc, jk->step_episode, params, nullptr);
+        if (cr != CUDA_SUCCESS) return fail(-3, "launch of the episode kernel failed (CUresult %d)", (int)cr);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        e->last_variant = 4;
+        e->t = e->T;
+        e->episode = episode;
+        e->noisy_now = A.noisy;
+        return stats_dev ? launch_return_stats(e, ret, 1, false, nullptr, stats_dev, accumulate, s) : 0;
+    }
+    // the composition: imx_reset + imx_step_many (per-period steps with the profit diagnostics when the accumulators are
+    // wanted) + imx_episode_stats
+    double* rew = reward_dev;
+    if (!rew && (rc = scratch((void**)&e->d_ep_rewards, (size_t)e->T * N * cols * sizeof(double)))) return rc;
+    if (!rew) rew = e->d_ep_rewards;
+    if (eval_acc_dev) {
+        if ((rc = scratch((void**)&e->d_ep_profit, cells * sizeof(double)))) return rc;
+        if (!obs_dev && (rc = scratch(&e->d_obs_scratch, cells * e->O * es))) return rc;
+    }
+    double* st = stats_dev;
+    if (!st && return_dev) {
+        if ((rc = scratch((void**)&e->d_ep_stats, (3 + 2 * (size_t)m) * sizeof(double)))) return rc;
+        st = e->d_ep_stats;
+        accumulate = 0;
+    }
+    if ((rc = imx_reset(e, demand_dev, delay_mask_dev, noisy, episode, nullptr, stream))) return rc;
+    const size_t rstride = (size_t)N * cols;
+    if (!eval_acc_dev) {
+        if ((rc = imx_step_many(e, actions_dev, e->T, obs_dev, rew, nullptr, stream))) return rc;
+    } else {
+        for (int t = 0; t < e->T; ++t) {
+            imx_info_out info;
+            memset(&info, 0, sizeof(info));
+            info.profit_dev = e->d_ep_profit;
+            void* ob = obs_dev ? (void*)((unsigned char*)obs_dev + (size_t)t * cells * e->O * es) : e->d_obs_scratch;
+            if ((rc = launch_step(e, actions_dev + (size_t)t * cells, (double*)ob, rew + (size_t)t * rstride, &info, s))) return rc;
+            if ((rc = imx_eval_accumulate(e, ob, rew + (size_t)t * rstride, e->d_ep_profit, eval_acc_dev, t == 0, stream))) return rc;
+        }
+    }
+    if (st) return imx_episode_stats(e, rew, e->T, return_dev, st, accumulate, stream);
     return 0;
 }
 
@@ -1529,7 +1713,8 @@ extern "C" const char* imx_jit_log(void) { return imxjit::g_last_log.c_str(); }
 
 extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap) {
     if (!cfg) return fail(-1, "null argument");
-    if (variant < 0 || variant > 2) return fail(-1, "variant must be 0 (step), 1 (no observations) or 2 (critic rows)");
+    if (variant < 0 || variant > 4)
+        return fail(-1, "variant must be 0 (step), 1 (no observations), 2 (critic rows), 3 (episode) or 4 (episode without observations)");
     imx_env tmp;
     tmp.cfg = *cfg;
     const int rc = derive(&tmp);
@@ -1554,7 +1739,9 @@ extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* l
     build_tables(&tmp, &TL);
     imxjit::Spec sp;
     if (variant == 2 && !tmp.multi) return fail(-1, "the critic rows exist for the multi-agent kinds only");
-    jit_spec(&tmp, TL, sp, variant == 1 ? 0 : 1, variant == 2 ? 1 : 0);
+    EpisodeArgs EA;
+    if (variant >= 3 && episode_layout(&tmp, EA) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
+    jit_spec(&tmp, TL, sp, (variant == 1 || variant == 4) ? 0 : 1, variant == 2 ? 1 : 0, variant >= 3 ? 1 : 0);
     std::string lg;
     std::vector<char> cubin;
     const size_t n = imxjit::compile_only(sp, lg, &cubin);

@@ -165,6 +165,11 @@ __device__ __forceinline__ double rescale(double v, double vmax, double a, doubl
 __device__ __forceinline__ double rev_scale(double x, double vmax, double a, double bma) {
     return __ddiv_rn(__dmul_rn(__dsub_rn(x, a), vmax), bma);
 }
+// the evaluation loops' rev_scale with every operation of the host expression (the trailing "+ 0" turns -0 into +0):
+// (((x - a) * (max - 0)) / (b - a)) + 0                                                 MAIM_env.py:509-519
+__device__ __forceinline__ double rev_scale_dev(double x, double vmax, double a, double bma) {
+    return __dadd_rn(__ddiv_rn(__dmul_rn(__dsub_rn(x, a), __dsub_rn(vmax, 0.0)), bma), 0.0);
+}
 // order clipping: MAIM kinds round then clip (MAIM_env.py:344-347), IM kinds clip then round
 // (IM_env.py:300-302); rint() is round-half-to-even like np.round.
 __device__ __forceinline__ int decode_order(double x, double om, bool std_actions, bool multi, double a, double bma,

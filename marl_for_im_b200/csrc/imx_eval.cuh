@@ -34,11 +34,6 @@ struct EvalArgs {
     double a, bma;
 };
 
-// rev_scale(x, 0, max, a, b) = (((x - a) * (max - 0)) / (b - a)) + 0            MAIM_env.py:509-519
-__device__ __forceinline__ double rev_scale_dev(double x, double vmax, double a, double bma) {
-    return __dadd_rn(__ddiv_rn(__dmul_rn(__dsub_rn(x, a), __dsub_rn(vmax, 0.0)), bma), 0.0);
-}
-
 __global__ void __launch_bounds__(256) eval_accumulate_kernel(const __grid_constant__ EvalArgs E) {
     const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= E.N) return;

@@ -39,6 +39,31 @@ struct TileLayout {
     int32_t off_cc;            // centralised-critic rows [E][m][W] (layouts built for imx_step_cc only; inside `total`)
 };
 
+// One whole stored-plan episode per launch (imx_replay_episode, step_kernel_tma_episode): what the kernel needs beyond the
+// multi-period StepArgs.  The episode regions of shared memory sit behind TileLayout.total2 (the per-period demand rows of
+// that layout are unused: the episode's whole trace is resident instead).
+struct EpisodeArgs {
+    const int32_t* __restrict__ demand;   // replayed trace [N][R][T] read in place (one bulk copy per tile), or null: Philox draws
+    const uint8_t* __restrict__ mask;     // replayed noisy-delay outcomes [N][T][m], or null: Philox draws (when A.noisy)
+    double* __restrict__ ret;             // episode returns [N][m] / [N], or null
+    double* __restrict__ eval;            // evaluation-loop accumulators [N][4 + m], or null
+    DemandGen gen;                        // the Philox stream imx_reset would draw this episode from
+    double delay_thr;                     // noisy_delay_threshold of the Philox delay draws
+    int32_t off_edem;                     // [E][R][T] int32 demand of the tile's envs
+    int32_t off_ret;                      // [E][m] / [E] float64 returns
+    int32_t off_eval;                     // [E][4 + m] float64 accumulators
+    int32_t off_prof;                     // [E][m] float64 profits of the current period (eval only)
+    int32_t total;                        // dynamic shared memory bytes
+    int32_t rescaled;                     // the state is standardised: the accumulators undo the scaling (rev_scale)
+};
+
+// Noisy-delay outcome of (local env n, node i, period t) in an episode launch: the replayed mask, or the draw
+// mask_generate_kernel makes for imx_reset(noisy = 1) of the same episode.
+__device__ __forceinline__ bool episode_delayed(const EpisodeArgs& EA, int64_t n, int m, int T, int i, int t) {
+    if (EA.mask) return EA.mask[(n * T + t) * m + i] != 0;
+    return draw_delay(EA.gen.seed, EA.gen.env_offset + n, i, t, EA.gen.episode, EA.delay_thr);
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
@@ -158,6 +183,8 @@ struct TileSmem {
     int32_t *inv, *bl, *ou, *pipe, *hd, *ho, *carry, *bt;   // state, updated in place
     unsigned char* obs;         // [E][m][O] observation tile (float64 or float32)
     double* rew;                // [E][m] / [E] reward tile
+    double* prof;               // [E][m] profits of the period, or null (episode kernel with evaluation accumulators)
+    double* ret;                // [E][m] / [E] episode returns, or null (episode kernel): reward added in place, period by period
 };
 
 // Per-thread constants of the lanes = stages mapping.
@@ -201,7 +228,8 @@ __device__ __forceinline__ LaneCtx<MAXC> make_lane_ctx(const StepArgs& A, int ti
 // writes (a multi-period launch waits there for the previous period's bulk stores).  No barriers or fences in here:
 // the caller orders the tile's loads before and its stores after.
 //   j = period index inside the launch (diagnostics block, MANY only), t = period being simulated, n0 = first env of the tile
-template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, typename BeforeStore>
+//   EP: episode kernel — S.dem is the tile's whole [E][R][T] trace, and the profits go to S.prof when it is set
+template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, bool EP = false, typename BeforeStore>
 __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout& TLY, const TileSmem& S, const LaneCtx<MAXC>& L,
                                             int t, int j, int64_t n0, bool delayed, BeforeStore&& before_store) {
     const NodeParams& np = L.np;
@@ -243,7 +271,7 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
             for (int jj = 0; jj < PMAX; ++jj)
                 if (jj < KF(P)) ho[jj] = S.ho[cell * KF(P) + jj];
         }
-        if (np.retailer_idx >= 0) cust = S.dem[np.retailer_idx * E + e_loc];
+        if (np.retailer_idx >= 0) cust = EP ? S.dem[(e_loc * KF(R) + np.retailer_idx) * KF(T) + t] : S.dem[np.retailer_idx * E + e_loc];
         if (KF(has_carry)) carry = S.carry[cell];
         if constexpr (DIV) {
             if (np.bt_off >= 0) {
@@ -378,6 +406,11 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
         }
         if (KF(multi)) S.rew[cell] = reward_out;
         else if (i == 0) S.rew[e_loc] = reward_out;
+        if (EP && S.prof) S.prof[cell] = profit;
+        if (EP && S.ret) {                           // stats_slice_kernel<true>'s order: from 0, period by period
+            if (KF(multi)) S.ret[cell] = __dadd_rn(S.ret[cell], reward_out);
+            else if (i == 0) S.ret[e_loc] = __dadd_rn(S.ret[e_loc], reward_out);
+        }
 #ifdef IMX_OBS_ROTATE
         {
             if (KHAS(obs)) {
@@ -484,9 +517,10 @@ __device__ __forceinline__ void cc_build(const StepArgs& A, const TileLayout& TL
 // Used for the divergent networks, whose lanes = nodes kernels are issue-bound (profiles/r2_ncu_div2_step_kernel_lanes.txt).
 #if defined(IMX_JIT) && defined(IMX_STEP_ET) && IMX_STEP_ET
 #define IMX_USE_STEP_ET 1
-template <int M, int DMAX, int PMAX, int MAXC, bool DIV, typename BeforeStore>
+// EP: episode kernel (as in tile_period; the noisy-delay outcomes come from episode_delayed)
+template <int M, int DMAX, int PMAX, int MAXC, bool DIV, bool EP = false, typename BeforeStore>
 __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayout& TLY, const TileSmem& S, int e, int t, int64_t n0,
-                                               BeforeStore&& before_store) {
+                                               BeforeStore&& before_store, const EpisodeArgs* EA = nullptr) {
     constexpr int INV_MAX[M] = {IMX_L_inv_max}, ORDER_MAX[M] = {IMX_L_order_max}, DEMAND_MAX[M] = {IMX_L_demand_max};
     constexpr int DELAY[M] = {IMX_L_delay}, PIPE_OFF[M] = {IMX_L_pipe_off};
     constexpr int NCHILD[M] = {IMX_L_nchild}, RETAILER[M] = {IMX_L_retailer_idx}, BT_OFF[M] = {IMX_L_bt_off};
@@ -519,7 +553,7 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
 #pragma unroll
     for (int j = 0; j < M; ++j) {
         if (RETAILER[j] >= 0) {
-            demand[j] = min(S.dem[RETAILER[j] * E + e], INV_MAX[j]);
+            demand[j] = min(EP ? S.dem[(e * KF(R) + RETAILER[j]) * KF(T) + t] : S.dem[RETAILER[j] * E + e], INV_MAX[j]);
         } else if (DIV) {
             int sum = 0;
 #pragma unroll
@@ -534,7 +568,10 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
         if (t >= DELAY[j]) {
             a += pipe[j][0];
             if (KF(noisy)) {                         // noisy delay (MAIM_env.py:449-457): hold this period's arrival back by one period
-                if (t < KF(T) - 1 && A.mask_T[((int64_t)t * A.N + n0 + e) * M + j] != 0) { cr[j] = a; a = 0; }
+                if (t < KF(T) - 1 && (EP ? episode_delayed(*EA, n0 + e, M, KF(T), j, t) : A.mask_T[((int64_t)t * A.N + n0 + e) * M + j] != 0)) {
+                    cr[j] = a;
+                    a = 0;
+                }
             }
         }
         acq[j] = a;
@@ -629,6 +666,7 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
                 if (k < NCHILD[j]) S.bt[e * KF(NB) + BT_OFF[j] + k] = bt[j][k];
         }
         if (KF(multi)) S.rew[c0 + j] = reward[j];
+        if (EP && S.prof) S.prof[c0 + j] = profit[j];
         if (KHAS(obs)) {
             NodeParams np;                           // the integer maxima write_obs_row scales with (compile-time values)
             np.inv_max = INV_MAX[j]; np.order_max = ORDER_MAX[j]; np.demand_max = DEMAND_MAX[j];
@@ -637,16 +675,66 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
         }
     }
     if (!KF(multi)) S.rew[e] = reward[0];
+    if (EP && S.ret) {                               // stats_slice_kernel<true>'s order: from 0, period by period
+#pragma unroll
+        for (int j = 0; j < (KF(multi) ? M : 1); ++j) S.ret[e * (KF(multi) ? M : 1) + j] = __dadd_rn(S.ret[e * (KF(multi) ? M : 1) + j], reward[j]);
+    }
     if (DIV && err_code != 0) A.err[n0 + e] = err_code;
 }
 #else
 #define IMX_USE_STEP_ET 0
 #endif
 
+// Episode kernel with evaluation accumulators, after each period: thread e repeats eval_accumulate_kernel's float64 operations
+// in its order on the observation elements the step writes (obs[i][0] = inventory, obs[i][1] = backlog: rounded to float32 and
+// widened for float32 observations) and on the period's profits.
+__device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs& EA, unsigned char* smem, int e) {
+    const int m = KF(m);
+    const int cols = KF(multi) ? m : 1;
+    const double* rew = reinterpret_cast<const double*>(smem + KT(off_rew)) + e * cols;
+    {
+        double* row = reinterpret_cast<double*>(smem + EA.off_eval) + e * (4 + m);
+        const int32_t* inv = reinterpret_cast<const int32_t*>(smem + KT(off_inv)) + e * m;
+        const int32_t* bl = reinterpret_cast<const int32_t*>(smem + KT(off_bl)) + e * m;
+        const double* prof = reinterpret_cast<const double*>(smem + EA.off_prof) + e * m;
+        double ep = row[0], step_inv = 0.0, step_bl = 0.0, cust = 0.0;
+        if (!KF(multi)) ep = __dadd_rn(ep, rew[0]);
+        for (int i = 0; i < m; ++i) {
+            const double inv_max = (double)__ldg(&A.nodes[i].inv_max);
+            double x0, x1;
+            if (KF(std_state)) {
+                const double* tabrow = KHAS(tab) ? A.tab + (size_t)i * 4 * KF(TL) : nullptr;
+                x0 = scaled(KHAS(tab), tabrow, KF(TL), TAB_INV, inv[i], inv_max, A.a, A.bma);
+                x1 = scaled(KHAS(tab), tabrow, KF(TL), TAB_DEM, bl[i], (double)__ldg(&A.nodes[i].demand_max), A.a, A.bma);
+            } else {
+                x0 = (double)inv[i];
+                x1 = (double)bl[i];
+            }
+            if (KF(obs_f32)) { x0 = (double)(float)x0; x1 = (double)(float)x1; }
+            if (EA.rescaled) {
+                x0 = rev_scale_dev(x0, inv_max, A.a, A.bma);         // the loops use inv_max for BOTH fields
+                x1 = rev_scale_dev(x1, inv_max, A.a, A.bma);
+            }
+            if (KF(multi)) ep = __dadd_rn(ep, rew[i]);
+            row[4 + i] = __dadd_rn(row[4 + i], prof[i]);
+            step_inv = __dadd_rn(step_inv, x0);
+            step_bl = __dadd_rn(step_bl, x1);
+            if (i == 0) cust = x1;
+        }
+        row[0] = ep;
+        row[1] = __dadd_rn(row[1], step_inv);
+        row[2] = __dadd_rn(row[2], step_bl);
+        row[3] = __dadd_rn(row[3], cust);
+    }
+}
+
 // MANY = false: one period per launch (the loop below folds away); MANY = true: A.periods periods per launch with the
 // tile's state resident in shared memory (imx_step_many) — separate kernels because the loop costs registers.
-template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY>
-__device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& TLY) {
+// EPISODE (with MANY): a whole episode from period 0 (imx_replay_episode) — the state starts as reset_kernel writes it instead
+// of being loaded, the tile's demand trace is resident for the whole episode, rewards are stored only when A.reward is set,
+// and returns / evaluation accumulators are kept in shared memory and stored once.
+template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, bool EPISODE = false>
+__device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs* EA = nullptr) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t bar[2];         // bar[b]: inputs of the periods with parity b (bar[0] also the state)
 
@@ -676,15 +764,18 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     const uint32_t b_cell4 = (uint32_t)E * m * 4u, b_cell8 = (uint32_t)E * m * 8u;
     const uint32_t b_pipe = (uint32_t)E * KF(L) * 4u, b_hist = b_cell4 * (uint32_t)KF(P);
     const uint32_t b_bt = (uint32_t)E * KF(NB) * 4u, b_dem = (uint32_t)E * 4u;
-    const uint32_t b_in = b_cell8 + (uint32_t)KF(R) * b_dem;       // per-period inputs: actions + demand rows
+    // per-period inputs: actions + demand rows (the episode kernel's demand is resident for the whole launch)
+    const uint32_t b_in = b_cell8 + (EPISODE ? 0u : (uint32_t)KF(R) * b_dem);
+    const uint32_t b_edem = (uint32_t)E * KF(R) * KF(T) * 4u;     // the tile's [E][R][T] trace (episode kernel)
 
     // per-period inputs of period j (actions block j, demand rows of period t0 + j) into input buffer j & 1
     auto load_inputs = [&](int j) {
         double* sa = reinterpret_cast<double*>(smem + ((j & 1) ? KT(off_act2) : KT(off_act)));
         int32_t* sd = reinterpret_cast<int32_t*>(smem + ((j & 1) ? KT(off_dem2) : KT(off_dem)));
         bulk_load_g2s(sa, A.actions + (int64_t)j * A.act_stride + n0 * m, b_cell8, &bar[j & 1]);
-        for (int r = 0; r < KF(R); ++r)
-            bulk_load_g2s(sd + r * E, A.demand_T + ((int64_t)(A.t + j) * KF(R) + r) * A.N + n0, b_dem, &bar[j & 1]);
+        if (!EPISODE)
+            for (int r = 0; r < KF(R); ++r)
+                bulk_load_g2s(sd + r * E, A.demand_T + ((int64_t)(A.t + j) * KF(R) + r) * A.N + n0, b_dem, &bar[j & 1]);
     };
 
     pdl_launch_dependents();
@@ -697,9 +788,15 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     if (tid == 0) {
 #if defined(IMX_JIT) && !defined(IMX_NO_ACT_PREFETCH)
         bulk_prefetch_l2(A.actions + n0 * m, b_cell8);
-        for (int r = 0; r < KF(R); ++r) bulk_prefetch_l2(A.demand_T + ((int64_t)A.t * KF(R) + r) * A.N + n0, b_dem);
+        if (!EPISODE)
+            for (int r = 0; r < KF(R); ++r) bulk_prefetch_l2(A.demand_T + ((int64_t)A.t * KF(R) + r) * A.N + n0, b_dem);
 #endif
         pdl_wait();                                  // state written by the previous step must be complete and visible
+        if (EPISODE) {                               // no state to load: the actions of period 0 (+ the replayed trace)
+            mbar_expect_tx(&bar[0], b_in + (EA->demand ? b_edem : 0u));
+            load_inputs(0);
+            if (EA->demand) bulk_load_g2s(smem + EA->off_edem, EA->demand + n0 * KF(R) * KF(T), b_edem, &bar[0]);
+        } else {
         uint32_t bytes = b_in + 3u * b_cell4 + b_pipe;
         if (KF(need_hd)) bytes += b_hist;
         if (KF(need_ho)) bytes += b_hist;
@@ -715,6 +812,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
         if (KF(need_ho)) bulk_load_g2s(s_ho, A.hist_o + n0 * m * KF(P), b_hist, &bar[0]);
         if (KF(has_carry)) bulk_load_g2s(s_carry, A.carry + n0 * m, b_cell4, &bar[0]);
         if (DIV && KF(NB) > 0) bulk_load_g2s(s_bt, A.bt + n0 * KF(NB), b_bt, &bar[0]);
+        }
         if (K > 1) {                                 // period 1's inputs land while period 0 computes
             mbar_expect_tx(&bar[1], b_in);
             load_inputs(1);
@@ -724,6 +822,28 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     // per-lane constants (overlaps the bulk loads)
     const LaneCtx<MAXC> L = make_lane_ctx<M_PAD, MAXC, DIV>(A, tid);
     pdl_wait();
+    if (EPISODE) {
+        // reset(): inv = init_inv, every other state word 0 (reset_kernel), the watchdog flags cleared, returns and accumulators
+        // at 0, and a Philox trace drawn into the demand region exactly as demand_generate_kernel draws it
+        const int nthr = (int)blockDim.x;
+        const int state_words = (KT(off_dem) - KT(off_inv)) / 4;     // inv .. bt are consecutive regions
+        for (int k = tid; k < state_words; k += nthr) s_inv[k] = (k < E * m) ? __ldg(&A.nodes[k % m].init_inv) : 0;
+        double* s_acc = reinterpret_cast<double*>(smem + EA->off_ret);  // returns, then accumulators
+        for (int k = tid; k < (EA->off_prof - EA->off_ret) / 8; k += nthr) s_acc[k] = 0.0;
+        for (int k = tid; k < E; k += nthr) A.err[n0 + k] = 0;
+        if (!EA->demand) {
+            int32_t* s_d = reinterpret_cast<int32_t*>(smem + EA->off_edem);
+            const int pairs = (KF(T) + 1) / 2;
+            for (int k = tid; k < E * KF(R) * pairs; k += nthr) {
+                const int p = k % pairs, er = k / pairs;             // er = e * R + r
+                int d0, d1;
+                draw_demand_pair(EA->gen, n0 + er / KF(R), er % KF(R), 2 * p, d0, d1);
+                s_d[er * KF(T) + 2 * p] = d0;
+                if (2 * p + 1 < KF(T)) s_d[er * KF(T) + 2 * p + 1] = d1;
+            }
+        }
+        __syncthreads();
+    }
 
     for (int j = 0; j < K; ++j) {
     const int t = A.t + j;                           // period being simulated
@@ -733,11 +853,14 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     unsigned char* s_obs = smem + KT(off_obs);       // ONE output buffer: period j - 1's bulk stores have long finished
     double* s_rew = reinterpret_cast<double*>(smem + KT(off_rew));   // reading it when period j's dynamics are done (waited below)
     bool delayed = false;
-    if (KF(noisy) && ok) delayed = A.mask_T[((int64_t)t * A.N + n0 + e_loc) * m + i] != 0;
+    if (KF(noisy) && ok)
+        delayed = EPISODE ? episode_delayed(*EA, n0 + e_loc, m, KF(T), i, t) : A.mask_T[((int64_t)t * A.N + n0 + e_loc) * m + i] != 0;
 
     mbar_wait(&bar[b], (uint32_t)((j >> 1) & 1));
 
-    const TileSmem S = {s_act, s_dem, s_inv, s_bl, s_ou, s_pipe, s_hd, s_ho, s_carry, s_bt, s_obs, s_rew};
+    const TileSmem S = {s_act, EPISODE ? reinterpret_cast<const int32_t*>(smem + EA->off_edem) : s_dem, s_inv, s_bl, s_ou, s_pipe, s_hd,
+                        s_ho, s_carry, s_bt, s_obs, s_rew, (EPISODE && EA->eval) ? reinterpret_cast<double*>(smem + EA->off_prof) : nullptr,
+                        (EPISODE && EA->ret) ? reinterpret_cast<double*>(smem + EA->off_ret) : nullptr};
     auto before_store = [&]() {
         if (MANY && j > 0) {                         // the previous period's stores must be done reading the output buffer
             if (tid == 0) bulk_wait_read_all();
@@ -745,10 +868,10 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
         }
     };
 #if IMX_USE_STEP_ET
-    tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV>(A, TLY, S, tid, t, n0, before_store);
+    tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV, EPISODE>(A, TLY, S, tid, t, n0, before_store, EA);
     (void)L; (void)delayed;
 #else
-    tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, MANY>(A, TLY, S, L, t, j, n0, delayed, before_store);
+    tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, MANY, EPISODE>(A, TLY, S, L, t, j, n0, delayed, before_store);
 #endif
     if (!MANY && KHAS(cc)) cc_build<MAXC>(A, TLY, S, smem, L, (int)blockDim.x);
     fence_proxy_async_smem();          // every writer orders its generic-proxy stores before the bulk copies
@@ -756,7 +879,8 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     if (tid == 0) {
         if (!MANY && KHAS(cc)) bulk_store_only(reinterpret_cast<unsigned char*>(A.cc) + n0 * m * A.cc_W * es, smem + KT(off_cc), (uint32_t)E * m * A.cc_W * es);
         if (KHAS(obs)) bulk_store_only(reinterpret_cast<unsigned char*>(A.obs) + (int64_t)j * A.obs_stride_bytes + n0 * m * O * es, s_obs, (uint32_t)E * m * O * es);
-        bulk_store_only(A.reward + (int64_t)j * A.rew_stride + (KF(multi) ? n0 * m : n0), s_rew, KF(multi) ? b_cell8 : (uint32_t)E * 8u);
+        if (!EPISODE || A.reward)
+            bulk_store_only(A.reward + (int64_t)j * A.rew_stride + (KF(multi) ? n0 * m : n0), s_rew, KF(multi) ? b_cell8 : (uint32_t)E * 8u);
         if (j == K - 1) {              // the tile's state leaves the SM once per launch
             bulk_store_only(A.inv + n0 * m, s_inv, b_cell4);
             bulk_store_only(A.backlog + n0 * m, s_bl, b_cell4);
@@ -773,7 +897,19 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
             load_inputs(j + 2);
         }
     }
+    // (reads this period's reward / state / profit tiles: the next period overwrites them only behind its before_store barrier)
+    if (EPISODE && EA->eval && tid < E) episode_env_pass(A, TLY, *EA, smem, tid);
     }   // periods
+    if (EPISODE && (EA->ret || EA->eval)) {      // returns and accumulator rows leave the SM once per episode
+        fence_proxy_async_smem();
+        __syncthreads();
+        if (tid == 0) {
+            const int cols = KF(multi) ? m : 1;
+            if (EA->ret) bulk_store_only(EA->ret + n0 * cols, smem + EA->off_ret, (uint32_t)E * cols * 8u);
+            if (EA->eval) bulk_store_only(EA->eval + n0 * (4 + m), smem + EA->off_eval, (uint32_t)E * (4 + m) * 8u);
+            bulk_commit();
+        }
+    }
     if (tid == 0) bulk_wait_read_all();  // shared memory must outlive the bulk engine's reads
 }
 
@@ -800,6 +936,13 @@ __global__ void IMX_STEP_BOUNDS step_kernel_tma(const __grid_constant__ StepArgs
 template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV>
 __global__ void IMX_MANY_BOUNDS step_kernel_tma_many(const __grid_constant__ StepArgs A, const __grid_constant__ TileLayout TLY) {
     step_tile<M_PAD, DMAX, PMAX, MAXC, DIV, true>(A, TLY);
+}
+
+// A whole stored-plan episode per launch (imx_replay_episode): reset + A.periods = T periods + returns / accumulators.
+template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV>
+__global__ void IMX_MANY_BOUNDS step_kernel_tma_episode(const __grid_constant__ StepArgs A, const __grid_constant__ TileLayout TLY,
+                                                        const __grid_constant__ EpisodeArgs EA) {
+    step_tile<M_PAD, DMAX, PMAX, MAXC, DIV, true, true>(A, TLY, &EA);
 }
 
 }  // namespace imx

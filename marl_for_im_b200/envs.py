@@ -641,6 +641,58 @@ class _ImxEnvBase:
             return obs_out, reward_out, self._shape_done(done), info
         return obs_out, reward_out, (self._shape_done(done))
 
+    def replay_episode(self, actions, customer_demand=None, delay_mask=None, noisy_delay=None, want_obs=False, want_rewards=False,
+                       returns=True, stats=None, accumulate=False, eval_acc=False):
+        """A whole episode on a stored plan ``actions [T, N, m]``: ``reset(customer_demand)`` + T ``step()`` calls + the episode's
+        returns, statistics and evaluation-loop accumulators (the LP scripts' replay loop, DSHLP_4.py:896-928) in one call —
+        one kernel launch where the batch allows it, without materialising per-period rewards or observations unless asked.
+
+        customer_demand: [N, R, T] / [N, T] / one trace, or None (Philox, the stream ``reset()`` draws from).  Noisy delays follow
+        the env's sticky ``noisy_delay`` flag unless ``noisy_delay`` is given; ``delay_mask`` replays them ([N, T, m] / [T, m]).
+        stats: None (not wanted), True (a new vector) or a float64 tensor ``[3 (+ 2m)]`` to write, or with ``accumulate=True``
+        to add into.  Returns ``dict(returns, stats, obs [T, N, m, O], rewards [T, N(, m)], eval [N, 4 + m])`` with None for
+        what was not asked; ``eval`` is what ``eval_accumulate`` builds over the episode (``eval_stats`` / ``eval_summary``
+        take it as is).  Leaves the env at period T with the final state."""
+        if not self.batched:
+            raise _lib.ImxError("replay_episode is a batched-mode call (construct the env with num_envs=N)")
+        N, m, O, T = self.num_envs, self.num_nodes, self.obs_len, self.num_periods
+        act = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions, dtype=np.float64))
+        act = act.to(device=self.device, dtype=torch.float64)
+        if act.numel() != T * N * m:
+            raise ValueError(f"actions must hold a whole episode: [T={T}, N={N}, m={m}]")
+        act = act.reshape(T, N, m).contiguous()
+        demand_dev = self._demand_to_device(customer_demand) if customer_demand is not None else None
+        want_noisy = (bool(self.noisy_delay) if noisy_delay is None else bool(noisy_delay)) or delay_mask is not None
+        mask_dev = None
+        if want_noisy:
+            if not self._has_carry:
+                self._create_handle(True)
+            if delay_mask is not None:
+                mask_dev = self._mask_to_device(delay_mask)
+        cols = (m,) if self.MULTI else ()
+        f64 = dict(dtype=torch.float64, device=self.device)
+        obs = torch.empty((T, N, m, O), dtype=self.obs_dtype, device=self.device) if want_obs else None
+        rew = torch.empty((T, N) + cols, **f64) if want_rewards else None
+        ret = torch.empty((N,) + cols, **f64) if returns else None
+        if stats is True:
+            stats = torch.zeros(3 + (2 * m if self.MULTI else 0), **f64)
+        elif stats is False:
+            stats = None
+        if stats is not None and (stats.dtype != torch.float64 or not stats.is_contiguous() or stats.numel() != 3 + (2 * m if self.MULTI else 0)):
+            raise ValueError("stats must be a contiguous float64 tensor of 3 (+ 2m for the multi-agent kinds) entries")
+        ev = torch.empty((N, 4 + m), **f64) if eval_acc else None
+        self._episode += 1
+        p = lambda x: C.c_void_p(x.data_ptr()) if x is not None else None   # noqa: E731
+        _lib.check(self._lib.imx_replay_episode(self._handle, p(demand_dev), p(mask_dev), int(want_noisy), self._episode, p(act),
+                                                p(obs), p(rew), p(ret), p(stats), int(bool(accumulate)), p(ev), self._stream()))
+        self._keepalive = (act, demand_dev, mask_dev)
+        if obs is not None:
+            self.last_obs = obs[T - 1]
+            self.state = self._shape_obs(obs[T - 1])
+        if rew is not None:
+            self.last_reward = rew[T - 1]
+        return {"returns": ret, "stats": stats, "obs": obs, "rewards": rew, "eval": ev}
+
     # ------------------------------------------------------------------ drop-in mode histories
     def _alloc_histories(self):
         T, m = self.num_periods, self.num_nodes

@@ -84,6 +84,11 @@ typedef struct imx_config {
     uint64_t seed;                /* Philox key                                               */
     int64_t num_envs;             /* N: envs in this handle (this rank's shard)              */
     int64_t env_offset;           /* global index of local env 0 (Philox counter; makes results independent of sharding) */
+    /* Capacities above 2^28 are refused, and so is any config whose int32 state could wrap (DESIGN.md §6): with dmax_i the
+     * most node i can be asked for in one period (a retailer's inv_max, the downstream stage's order_max, the sum of the
+     * children's order_max), demand_max must fit int32, and T * dmax_i must too wherever the backlog is uncapped
+     * (standardise_state = 0 on IM / IM_DIV / MAIM) and for every divergent node with more than one child (its ledger).
+     * With noisy_delay, inv_max_i + T * order_max_i (twice that for a divergent node other than 0) must fit int32 (the carry). */
     int32_t inv_init[IMX_MAX_NODES];
     int32_t inv_max[IMX_MAX_NODES];
     int32_t order_max[IMX_MAX_NODES];

@@ -655,9 +655,12 @@ static int derive(imx_env* e) {
             if (c.num_children[i] == 0) { e->retailer_idx[i] = e->R; e->retailers[e->R++] = i; }
             e->sell[i] = (double)(e->depth[i] + 2);            // MAIM_div_env.py:55-61
             e->buy[i] = (double)(e->depth[i] + 1);
-            int dm = c.inv_max[i], s = 0;                      // MAIM_div_env.py:91-99
+            int64_t s = 0;                                     // MAIM_div_env.py:91-99
             for (int k = 0; k < c.num_children[i]; ++k) s += c.order_max[c.children[i][k]];
-            e->demand_max[i] = s > dm ? s : dm;
+            if (s > INT32_MAX)
+                return fail(-1, "demand_max[%d] = %lld (the sum of its children's order_max) exceeds INT32_MAX: the int32 state "
+                                "cannot hold it", i, (long long)s);
+            e->demand_max[i] = s > c.inv_max[i] ? (int)s : c.inv_max[i];
         }
         if (c.order_max[0] > c.inv_max[0]) return fail(-1, "order_max[0] must not exceed inv_max[0]");   // MAIM_div_env.py:235
     } else {
@@ -674,6 +677,35 @@ static int derive(imx_env* e) {
     }
 
     const bool std_state = (c.kind == IMX_KIND_MAIM_DIV) ? true : (c.standardise_state != 0);
+    // Domain of the int32 state (the reference's integers are unbounded).  A node's demand in one period is at most dmax_i:
+    // the clipped customer demand of a retailer, a serial stage's downstream order, a split node's children's orders.  An
+    // uncapped backlog (standardise_state = 0 on IM, IM_div and MAIM) grows by at most dmax_i a period, and so does a split node's
+    // per-child ledger (IMX_F_BACKLOG_TO, never capped, negative entries bounded by earlier positive ones): both stay below
+    // T * dmax_i, which must fit int32.  Every other int32 quantity is bounded by a capacity (<= 2^28) or by these.
+    for (int i = 0; i < m; ++i) {
+        int64_t dmax = (e->retailer_idx[i] >= 0) ? c.inv_max[i] : e->div ? 0 : c.order_max[i - 1];
+        if (e->div)
+            for (int k = 0; k < c.num_children[i]; ++k) dmax += c.order_max[c.children[i][k]];
+        const int64_t bound = (int64_t)e->T * dmax;
+        if (bound > INT32_MAX && !std_state)
+            return fail(-1, "num_periods * the largest per-period demand of node %d = %lld exceeds INT32_MAX: its uncapped backlog "
+                            "(standardise_state = 0) could wrap the int32 state", i, (long long)bound);
+        if (bound > INT32_MAX && e->div && c.num_children[i] > 1)
+            return fail(-1, "num_periods * the largest per-period demand of node %d = %lld exceeds INT32_MAX: its per-child backlog "
+                            "ledger could wrap the int32 state", i, (long long)bound);
+        // The noisy-delay carry (IMX_F_CARRY) holds every arrival of a run of delayed periods, and acquisition adds it to the
+        // inventory.  A node receives no more over the episode than it orders (T * order_max_i): its supplier ships at most
+        // the backlog plus demand it owes, or the factory fills the order itself.  A divergent child can receive up to twice
+        // that, since the split subtracts what it ships from the parent's ledger twice when it drains a backlog, and the
+        // ledger may then go negative by as much as it was positive.
+        if (c.noisy_delay) {
+            const int64_t arrivals = (int64_t)e->T * c.order_max[i] * ((e->div && i > 0) ? 2 : 1);
+            if (arrivals + c.inv_max[i] > INT32_MAX)
+                return fail(-1, "with noisy delays, inv_max[%d] + the most node %d can receive over num_periods (%lld) exceeds "
+                                "INT32_MAX: goods held back over consecutive delayed periods could wrap the int32 state", i, i,
+                                (long long)arrivals);
+        }
+    }
     // quirk 2: MAIM kinds in mode (td=F, pd=T, pa=F) never write the demand-history slots
     e->write_hd = !(e->multi && c.prev_demand && !c.prev_actions && !c.time_dependency);
     e->need_hd = c.prev_demand && e->write_hd && !(e->multi && !std_state);

@@ -142,10 +142,14 @@ static int decode_order(const orc_cfg* c, int i, double x) {
     return (int)x;
 }
 
+/* dm * mult saturated at INT32_MAX: a pass count never exceeds the int32 amount it hands out, so the saturated limit fires
+ * exactly where the reference's unbounded product would */
+static int wd_limit(int dm, int mult) { return dm > INT32_MAX / mult ? INT32_MAX : dm * mult; }
+
 /* returns the watchdog code (0 ok) */
 static int split(const orc_cfg* c, orc_state* s, int i, int ship, int demand, int backlog, const int* order, int* st) {
     const int nc = c->nchild[i];
-    const int dm = c->demand_max[i];
+    const int lim1 = wd_limit(c->demand_max[i], c->wd_mult1), lim = wd_limit(c->demand_max[i], c->wd_mult);
     int* bt = s->bt[i];
     int od[ORC_MAX_CHILDREN];
     int amt = ship;
@@ -159,7 +163,7 @@ static int split(const orc_cfg* c, orc_state* s, int i, int ship, int demand, in
                 for (int k = 0; k < nc; ++k) sum += bt[k];
                 if (!(sum > 0 && amt > 0)) break;
                 for (int k = 0; k < nc; ++k) if (bt[k] > 0) { st[k]++; bt[k]--; amt--; }
-                if (++cnt > dm * c->wd_mult1) return 1;
+                if (++cnt > lim1) return 1;
             }
             if (amt > 0 && demand > 0) {
                 int out[ORC_MAX_CHILDREN];
@@ -170,7 +174,7 @@ static int split(const orc_cfg* c, orc_state* s, int i, int ship, int demand, in
                     for (int k = 0; k < nc; ++k) sum += out[k];
                     if (!(amt > 0 && sum > 0)) break;
                     for (int k = 0; k < nc; ++k) if (out[k] > 0) { st[k]++; out[k]--; amt--; }
-                    if (++cnt > dm * c->wd_mult) return 2;
+                    if (++cnt > lim) return 2;
                 }
                 for (int k = 0; k < nc; ++k) bt[k] += out[k];
             }
@@ -185,13 +189,15 @@ static int split(const orc_cfg* c, orc_state* s, int i, int ship, int demand, in
                 for (int k = 0; k < nc; ++k) sum += bt[k];
                 if (!(sum > 0 && amt > 0)) break;
                 for (int k = 0; k < nc; ++k) if (bt[k] > 0) { st[k]++; bt[k]--; amt--; }
-                if (++cnt > dm * c->wd_mult) return 3;
+                if (++cnt > lim) return 3;
             }
         } else {
             int cnt = 0;
             while (amt > 0) {
-                for (int k = 0; k < nc; ++k) if (st[k] < od[k] + bt[k]) { st[k]++; amt--; }
-                if (++cnt > dm * c->wd_mult) return 4;
+                int gave = 0;
+                for (int k = 0; k < nc; ++k) if (st[k] < od[k] + bt[k]) { st[k]++; amt--; gave = 1; }
+                if (!gave) return 4;                     /* nobody can take a unit: the reference spins into its watchdog */
+                if (++cnt > lim) return 4;
             }
         }
         for (int k = 0; k < nc; ++k) bt[k] += od[k] - st[k];

@@ -26,7 +26,9 @@
  *
  * Data layout (row-major, env index slowest unless stated)
  *   actions  [N][m] float64      reward (MAIM kinds) [N][m] float64, (IM kinds) [N] float64
- *   obs      [N][m][O] float64   row i of env n = agent i's observation vector (float32 when cfg.obs_f32)
+ *            (float32 with IMX_IO_ACTIONS_F32: action pointers are in the handle's action type)
+ *   obs      [N][m][O] float64   row i of env n = agent i's observation vector (float32 when cfg.obs_f32, bfloat16 with
+ *                                IMX_IO_OBS_BF16: every observation pointer is void*, in the handle's observation type)
  *   demand   [N][R][T] int32     replayed customer demand, R = number of retailers (serial: 1)
  *   mask     [N][T][m] uint8     replayed noisy-delay Bernoulli outcomes (u <= threshold)
  *   state    int32 structure-of-arrays, see imx_state_field()
@@ -42,7 +44,9 @@
 extern "C" {
 #endif
 
-#define IMX_ABI_VERSION 3     /* 3: obs pointers are void* (float64, or float32 with cfg.obs_f32) everywhere; imx_rollout_basestock gained
+#define IMX_ABI_VERSION 3     /* 3 (later, source-compatible): imx_config.reserved0 became io_flags (bfloat16 observations, float32
+                                 actions); action pointers are const void* (imx_replay_episode's keeps its spelling); imx_round_bf16.
+                                 3: obs pointers are void* (float64, or float32 with cfg.obs_f32) everywhere; imx_rollout_basestock gained
                                  delay_mask_dev / noisy and takes pmf [N][R][T]; imx_prepare; imx_step_cc.
                                  2: imx_config gained obs_f32 + noisy_demand_threshold; imx_step_many, imx_eval_*; imx_cc_observe takes void* */
 #define IMX_MAX_NODES 32     /* agents (stages / nodes) per env: one lane each            */
@@ -52,6 +56,11 @@ extern "C" {
 
 enum imx_kind { IMX_KIND_IM = 0, IMX_KIND_MAIM = 1, IMX_KIND_IM_DIV = 2, IMX_KIND_MAIM_DIV = 3 };
 enum imx_demand_dist { IMX_DIST_REPLAY_ONLY = 0, IMX_DIST_POISSON = 1, IMX_DIST_UNIFORM = 2 };
+/* imx_config.io_flags: per-handle I/O element types (the default, 0, is float64 actions and float64 / cfg.obs_f32 observations).
+ *   IMX_IO_OBS_BF16     observations are bfloat16: each element is the round-to-nearest-even bfloat16 of the float32 element
+ *                       cfg.obs_f32 writes (= torch's float64 -> bfloat16 conversion of the reference's value).  Not with obs_f32.
+ *   IMX_IO_ACTIONS_F32  actions are float32; results are bit-identical to passing the same values widened to float64. */
+enum imx_io_flags { IMX_IO_OBS_BF16 = 1, IMX_IO_ACTIONS_F32 = 2 };
 
 /* Per-config constants.  The host mirrors the reference constructors
  * (IM_env.py:7-162, MAIM_env.py:8-173, IM_div_env.py:9-199, MAIM_div_env.py:9-237): it applies
@@ -75,7 +84,7 @@ typedef struct imx_config {
     int32_t uniform_high;
     int32_t device;               /* CUDA device ordinal                                      */
     int32_t obs_f32;              /* 1: observations are written as float32 (= the float32 cast of the reference's float64 value; RLlib casts anyway), obs buffers are [N][m][O] float */
-    int32_t reserved0;
+    int32_t io_flags;             /* enum imx_io_flags; unused bits must be 0 (imx_create refuses them)                */
     double a, b;                  /* rescale interval (IM_DIV: the host passes -1, 1)        */
     double mu;                    /* IMX_DIST_POISSON mean                                   */
     double noisy_delay_threshold; /* used when the mask is generated (Philox) instead of replayed */
@@ -186,7 +195,7 @@ int imx_reset(imx_env* env, const int32_t* demand_dev, const uint8_t* delay_mask
  * MAIM_div_env.py:441-630: order clipping, demand propagation, acquisition, shipment (+ split),
  * backlog / pipeline / inventory update, profit reward, observation build.  One kernel launch.
  * done = imx_period(env) >= T after the call.  info may be NULL. */
-int imx_step(imx_env* env, const double* actions_dev, void* obs_dev, double* reward_dev,
+int imx_step(imx_env* env, const void* actions_dev, void* obs_dev, double* reward_dev,
              const imx_info_out* info, void* stream);
 
 /* K consecutive step() calls on pre-computed actions  —  the replay loops that drive an env with a stored plan
@@ -198,7 +207,7 @@ int imx_step(imx_env* env, const double* actions_dev, void* obs_dev, double* rew
  *   actions_dev [K][N][m], obs_dev [K][N][m][O] or NULL, reward_dev [K][N][m] (MAIM kinds) / [K][N];
  *   info: NULL, or diagnostics arrays of K consecutive [N][m] blocks each (the array_profit / array_demand / array_ship /
  *   array_acquisition records of the LP replay loops, DSHLP_4.py:918-923). */
-int imx_step_many(imx_env* env, const double* actions_dev, int K, void* obs_dev, double* reward_dev,
+int imx_step_many(imx_env* env, const void* actions_dev, int K, void* obs_dev, double* reward_dev,
                   const imx_info_out* info, void* stream);
 
 /* One whole episode on a stored plan: reset(customer_demand) + T step() calls + the episode's returns / statistics
@@ -207,7 +216,8 @@ int imx_step_many(imx_env* env, const double* actions_dev, int K, void* obs_dev,
  *   imx_step_many(env, actions_dev, T, obs_dev, reward, NULL, s);                 (reward: reward_dev or scratch)
  *   imx_episode_stats(env, reward, T, return_dev, stats_dev, accumulate, s);       (when return_dev or stats_dev)
  *   imx_eval_accumulate(env, obs[t], reward[t], profit[t], eval_acc_dev, t == 0, s) for t < T   (when eval_acc_dev)
- * actions_dev [T][N][m]; obs_dev [T][N][m][O] or NULL; reward_dev [T][N][m] / [T][N] or NULL; return_dev [N][m] / [N] or NULL;
+ * actions_dev [T][N][m] in the handle's action type (float32 with IMX_IO_ACTIONS_F32: pass the float32 buffer cast to
+ * const double*; this declaration keeps its earlier spelling); obs_dev [T][N][m][O] or NULL; reward_dev [T][N][m] / [T][N] or NULL; return_dev [N][m] / [N] or NULL;
  * stats_dev [3 + 2m] / [3] or NULL; eval_acc_dev [N][4 + m] or NULL.  Leaves the env at period T with the final state
  * (every state field, the split's error flags).  demand_dev / delay_mask_dev / noisy / episode as in imx_reset: NULL draws
  * from the same Philox streams.  Works from any current period (it is a reset).
@@ -272,31 +282,32 @@ int imx_eval_stats(imx_env* env, const double* acc_dev, double* stats_dev, int a
 /* central_critic_observer + FillInActions  —  models/CC_Model.py:165-214 (and the hand-built CC
  * observation of CC_inv_management.py:516-528): for every agent the flat vector
  * [opponent_action (m-1) | opponent_obs (m-1)*O | own_obs O], W = imx_cc_obs_len() values.
- *   obs_dev      [N][m][O] in the element type this env writes (float64, or float32 with cfg.obs_f32)
- *   actions_dev  [N][m] float64 actions of the same step, clipped to [clip_lo, clip_hi]; NULL = zeros
- *   out_dev      [N][m][W] float64, or float32 when out_is_f32 != 0 (RLlib casts observations to float32) */
+ *   obs_dev      [N][m][O] in the element type this env writes (float64, float32 with cfg.obs_f32, bfloat16 with IMX_IO_OBS_BF16)
+ *   actions_dev  [N][m] actions of the same step in the handle's action type, clipped to [clip_lo, clip_hi]; NULL = zeros
+ *   out_dev      [N][m][W] float64 (out_is_f32 = 0), float32 (1: RLlib casts observations to float32) or bfloat16 (2: the
+ *                round-to-nearest-even of the float32 value) */
 int imx_cc_obs_len(const imx_env* env);
-int imx_cc_observe(imx_env* env, const void* obs_dev, const double* actions_dev, double clip_lo, double clip_hi,
+int imx_cc_observe(imx_env* env, const void* obs_dev, const void* actions_dev, double clip_lo, double clip_hi,
                    void* out_dev, int out_is_f32, void* stream);
 
 /* step(action) + central_critic_observer in ONE kernel: the step kernel's epilogue assembles the critic rows of
  * imx_cc_observe from the observation tile it has just built in shared memory and from this step's action tile, and
  * writes them with one bulk store per tile next to obs / reward / state (no second pass over [N][m][O]).
  *   obs_dev     [N][m][O] or NULL (the rows still contain every agent's observation)
- *   cc_dev      [N][m][W], W = imx_cc_obs_len(), in the observation element type (float64, or float32 with cfg.obs_f32)
+ *   cc_dev      [N][m][W], W = imx_cc_obs_len(), in the observation element type (float64, float32 or bfloat16)
  *   fill_actions non-zero: opponent-action slots = this step's actions clipped to [clip_lo, clip_hi] (FillInActions,
  *               models/CC_Model.py:165-193; the evaluation loops' hand-built rows, CC_inv_management.py:516-528); zero: zeros, as
  *               central_critic_observer leaves them at sampling time (:196-214)
  * Fused wherever the runtime-specialised TMA kernels serve the whole batch (N a multiple of the tile size, 16-byte aligned
  * buffers); otherwise imx_step followed by imx_cc_observe — same bytes either way.  Multi-agent kinds only. */
-int imx_step_cc(imx_env* env, const double* actions_dev, void* obs_dev, void* cc_dev, int fill_actions, double clip_lo,
+int imx_step_cc(imx_env* env, const void* actions_dev, void* obs_dev, void* cc_dev, int fill_actions, double clip_lo,
                 double clip_hi, double* reward_dev, void* stream);
 
 /* End-to-end convenience calls on HOST buffers (pinned memory recommended): copy in, launch, copy
- * out, synchronise.  These are what a per-step Python caller pays for. */
+ * out, synchronise.  These are what a per-step Python caller pays for.  Actions and observations in the handle's types. */
 int imx_reset_host(imx_env* env, const int32_t* demand_host, const uint8_t* delay_mask_host, int noisy,
                    uint64_t episode, void* obs_host);
-int imx_step_host(imx_env* env, const double* actions_host, void* obs_host, double* reward_host);
+int imx_step_host(imx_env* env, const void* actions_host, void* obs_host, double* reward_host);
 
 /* Poisson CDF table the Philox demand generator inverts (cdf[k] = P(X <= k), last entry a
  * sentinel > 1).  Returns the table length; copies min(len, cap) entries when out != NULL. */
@@ -314,6 +325,10 @@ const char* imx_jit_log(void);
  * 4 = the same without observations.
  * Returns the cubin size in bytes, or a negative error; `log` receives the compiler log. */
 int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap);
+
+/* The host's float32 -> bfloat16 rounding (round to nearest even; a NaN stays a NaN), which builds the bfloat16 copy of the
+ * rescale tables: out[k] = bit pattern of in[k] rounded, as torch.Tensor.to(torch.bfloat16) rounds.  Needs no GPU. */
+int imx_round_bf16(const float* in, uint16_t* out, int64_t n);
 
 /* Number of kernels this library has launched since load (bench.py's gpu_launches claim). */
 int64_t imx_launch_count(void);

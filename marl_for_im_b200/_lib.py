@@ -13,6 +13,7 @@ ABI_VERSION = 3          # IMX_ABI_VERSION of include/imx_b200.h this binding mi
 KIND = {"IM": 0, "MAIM": 1, "IM_div": 2, "MAIM_div": 3}
 DIST = {"replay": 0, "custom": 0, "poisson": 1, "uniform": 2}
 PREPARE_EPISODE = 32    # IMX_PREPARE_EPISODE: imx_replay_episode's kernels and scratch (imx_prepare)
+IO_OBS_BF16, IO_ACTIONS_F32 = 1, 2   # imx_config.io_flags: bfloat16 observations, float32 actions
 F_INV, F_BACKLOG, F_ORDER_U, F_PIPE, F_HIST_D, F_HIST_O, F_CARRY, F_BACKLOG_TO, F_ERROR, F_DEMAND, F_DELAY_MASK = range(11)
 
 LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "libimx_b200.so")
@@ -25,7 +26,7 @@ class ImxConfig(C.Structure):
         ("standardise_state", C.c_int32), ("standardise_actions", C.c_int32), ("independent", C.c_int32),
         ("share_network", C.c_int32), ("noisy_delay", C.c_int32), ("demand_dist", C.c_int32),
         ("uniform_low", C.c_int32), ("uniform_high", C.c_int32), ("device", C.c_int32),
-        ("obs_f32", C.c_int32), ("reserved0", C.c_int32),
+        ("obs_f32", C.c_int32), ("io_flags", C.c_int32),
         ("a", C.c_double), ("b", C.c_double), ("mu", C.c_double), ("noisy_delay_threshold", C.c_double), ("noisy_demand_threshold", C.c_double),
         ("seed", C.c_uint64), ("num_envs", C.c_int64), ("env_offset", C.c_int64),
         ("inv_init", C.c_int32 * MAX_NODES), ("inv_max", C.c_int32 * MAX_NODES),
@@ -80,6 +81,7 @@ SYMBOLS = {
     "imx_kernel_variant": (C.c_int, [_P]),
     "imx_jit_log": (C.c_char_p, []),
     "imx_jit_compile_check": (C.c_int, [C.POINTER(ImxConfig), C.c_int, C.c_char_p, C.c_int]),
+    "imx_round_bf16": (C.c_int, [_P, _P, C.c_int64]),
     "imx_launch_count": (C.c_int64, []),
 }
 

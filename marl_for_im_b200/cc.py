@@ -31,11 +31,12 @@ def cc_observe(env, obs, actions=None, clip=(-1.0, 1.0), dtype=torch.float64):
     if actions is not None:
         act = env._actions_to_device(actions)
     W = env._lib.imx_cc_obs_len(env._handle)
+    out_type = {torch.float64: 0, torch.float32: 1, torch.bfloat16: 2}.get(dtype)    # imx_cc_observe's out_is_f32 codes
+    if out_type is None:
+        raise ValueError("dtype must be float64, float32 or bfloat16")
     out = torch.empty((N, m, W), dtype=dtype, device=env.device)
-    if dtype not in (torch.float64, torch.float32):
-        raise ValueError("dtype must be float64 or float32")
     _lib.check(env._lib.imx_cc_observe(env._handle, C.c_void_p(obs.data_ptr()), C.c_void_p(act.data_ptr()) if act is not None else None,
-                                       float(clip[0]), float(clip[1]), C.c_void_p(out.data_ptr()), int(dtype == torch.float32), env._stream()))
+                                       float(clip[0]), float(clip[1]), C.c_void_p(out.data_ptr()), out_type, env._stream()))
     return out
 
 

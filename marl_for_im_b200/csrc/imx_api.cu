@@ -109,7 +109,7 @@ struct imx_env {
     int TL = 0;
     // host-call staging (allocated on first use)
     cudaStream_t hstream = nullptr;
-    double *d_act_h = nullptr, *d_obs_h = nullptr, *d_rew_h = nullptr;
+    double *d_act_h = nullptr, *d_obs_h = nullptr, *d_rew_h = nullptr;   // (sized for float64; a float32 handle uses the first half)
     int32_t* d_dem_h = nullptr;
     uint8_t* d_mask_h = nullptr;
     // episode bookkeeping
@@ -160,6 +160,15 @@ struct imx_env {
     int m_pad = 0;
 };
 
+// The per-handle I/O element types (imx_config.obs_f32 / io_flags): every size the host derives from them comes from here.
+static int obs_type_of(const imx_config& c) { return (c.io_flags & IMX_IO_OBS_BF16) ? OBS_BF16 : c.obs_f32 ? OBS_F32 : OBS_F64; }
+static int obs_elem_bytes(const imx_env* e) { return imx::obs_elem_bytes(obs_type_of(e->cfg)); }
+static int act_elem_bytes(const imx_env* e) { return (e->cfg.io_flags & IMX_IO_ACTIONS_F32) ? 4 : 8; }
+// bytes one step moves per env: state read + written, demand, actions, rewards, observations
+static int64_t bytes_per_env(const imx_env* e) {
+    return 8 * (int64_t)e->S + 4 * e->R + (int64_t)e->m * (act_elem_bytes(e) + 8 + e->O * obs_elem_bytes(e));
+}
+
 // --------------------------------------------------------------------------------------
 // kernel dispatch tables: the template instantiations live in imx_kernels_inst.cu, one object per
 // (tile width, network family), compiled in parallel by the build
@@ -187,7 +196,10 @@ static void pick_kernels(imx_env* e, int m_pad, bool div) {
         else imx_pick_kernels_32_0(small, few, &ks);
     }
     e->step_fn = ks.step_fn; e->tma_fn = ks.tma_fn; e->tma_many_fn = ks.tma_many_fn; e->rollout_fn = ks.rollout_fn;
-    e->reset_fn = small ? reset_kernel<4, 1> : reset_kernel<8, 8>;
+    const int ot = obs_type_of(e->cfg);
+    if (ot == OBS_BF16) e->reset_fn = small ? reset_kernel<4, 1, OBS_BF16> : reset_kernel<8, 8, OBS_BF16>;
+    else if (ot == OBS_F32) e->reset_fn = small ? reset_kernel<4, 1, OBS_F32> : reset_kernel<8, 8, OBS_F32>;
+    else e->reset_fn = small ? reset_kernel<4, 1, OBS_F64> : reset_kernel<8, 8, OBS_F64>;
     e->m_pad = m_pad;
 }
 
@@ -202,6 +214,7 @@ static cudaError_t raise_dyn_smem_limit(const void* fn, size_t bytes) {
 }
 
 static int m_pad_of(const imx_env* e);
+
 // CTA size of the TMA kernel.  128-thread CTAs de-synchronise the load / compute / store phases of neighbouring tiles and
 // measured faster on every shipped config (profiles/r1_other_configs_1gpu.jsonl) except the 4-wide chain at
 // multi-million-env batches, where the 256-thread tile is 2.5% ahead; 512-thread CTAs lose 25%
@@ -209,8 +222,7 @@ static int choose_tma_threads(const imx_env* e) {
     const char* tt = getenv("IMX_TMA_THREADS");
     // 4-wide serial chains in the pipelined regime (working set within ~1.5 x L2, see pipe_pays): 64-thread tiles of 16 envs with
     // 8 resident CTAs per SM measured 3 % ahead of 128-thread tiles (profiles/r2_pipe_sweep.txt); 256-thread tiles from 1 Mi envs
-    const int64_t bytes_per_env = 8 * (int64_t)e->S + 4 * e->R + (int64_t)e->m * (16 + e->O * (e->cfg.obs_f32 ? 4 : 8));
-    const bool small4 = !e->div && m_pad_of(e) == 4 && e->N >= 1024 && bytes_per_env * e->N <= ((int64_t)192 << 20);
+    const bool small4 = !e->div && m_pad_of(e) == 4 && e->N >= 1024 && bytes_per_env(e) * e->N <= ((int64_t)192 << 20);
     // (512 Ki envs of a 4-wide chain, pipelined with the L2 priorities: 256-thread tiles 35.7 us, 128-thread 38.1, 64-thread 38.9)
     const bool big4 = !e->div && m_pad_of(e) == 4 && e->N >= ((int64_t)1 << 19);
     const int dflt = small4 ? 64 : (big4 || (m_pad_of(e) <= 4 && e->N >= ((int64_t)1 << 20))) ? 256 : 128;
@@ -232,7 +244,10 @@ static void compute_tile(const imx_env* e, TileLayout& L, int tile_width, bool w
     int off = 0;
     auto take = [&](int bytes) { const int o = off; off += (bytes + 127) & ~127; return o; };
     L.E = E;
-    L.off_act = take(E * m * 8);
+    // the multi-period kernel's shared-reward scratch ([E][m] float64) lives in the action region: over the consumed float64 actions,
+    // behind float32 ones (which other warps may still be reading when a lane stores its profit)
+    const int act_region = E * m * (act_elem_bytes(e) == 4 ? 12 : 8);
+    L.off_act = take(act_region);
     L.off_inv = take(E * m * 4);
     L.off_bl = take(E * m * 4);
     L.off_ou = take(E * m * 4);
@@ -242,13 +257,13 @@ static void compute_tile(const imx_env* e, TileLayout& L, int tile_width, bool w
     L.off_carry = take(e->has_carry ? E * m * 4 : 0);
     L.off_bt = take(E * e->NB * 4);
     L.off_dem = take(e->R * E * 4);
-    L.off_obs = take(E * m * e->O * (e->cfg.obs_f32 ? 4 : 8));
+    L.off_obs = take(E * m * e->O * obs_elem_bytes(e));
     L.off_rew = take(E * m * 8);
-    L.off_cc = with_cc ? take(E * m * ((m - 1) * (1 + e->O) + e->O) * (e->cfg.obs_f32 ? 4 : 8)) : 0;
+    L.off_cc = with_cc ? take(E * m * ((m - 1) * (1 + e->O) + e->O) * obs_elem_bytes(e)) : 0;
     L.total = off;
     // multi-period launches double-buffer the per-period inputs; the extra regions sit behind the
     // single-period layout so that a plain step launches the same kernel with `total` bytes only
-    L.off_act2 = take(E * m * 8);
+    L.off_act2 = take(act_region);
     L.off_dem2 = take(e->R * E * 4);
     L.total2 = off;
 }
@@ -281,7 +296,8 @@ static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1
     // so the specialised kernels of such a handle read the flag from the argument block
     defs.push_back(e->has_carry ? "IMX_K_noisy=(A.noisy)" : "IMX_K_noisy=0");
     add("need_ho", e->need_ho); add("wd_mult1", e->multi ? 2 : 4); add("wd_mult", e->multi ? 1 : 2); add("TL", TL);
-    add("noisy_demand", (e->div && c.noisy_demand_threshold > 0.0) ? 1 : 0); add("has_info", 0); add("has_obs", has_obs); add("has_tab", TL > 0); add("obs_f32", c.obs_f32 != 0);
+    add("noisy_demand", (e->div && c.noisy_demand_threshold > 0.0) ? 1 : 0); add("has_info", 0); add("has_obs", has_obs); add("has_tab", TL > 0);
+    add("obs_type", obs_type_of(c)); add("act_f32", (c.io_flags & IMX_IO_ACTIONS_F32) ? 1 : 0);
     int ex = 0;
     const double fr = std::frexp(c.b - c.a, &ex);
     add("bma_pow2", (fr == 0.5 && ex > -1000 && ex < 1000) ? 1 : 0);
@@ -500,7 +516,7 @@ static bool stream_is_capturing(cudaStream_t s) {
 // see the comment at the call in select_kernels(); l2_bytes <= 0: the B200's 126 MB (imx_jit_compile_check runs without a device)
 static int decide_l2_hints(const imx_env* e, int l2_bytes) {
     if (l2_bytes <= 0) l2_bytes = 126 << 20;
-    const int64_t per_env = 8 * (int64_t)e->S + 4 * e->R + (int64_t)e->m * (16 + e->O * (e->cfg.obs_f32 ? 4 : 8));
+    const int64_t per_env = bytes_per_env(e);
     const int64_t state_bytes = 4 * (int64_t)e->S * e->N;
     const char* lh = getenv("IMX_L2_HINTS");
     if (lh && !strcmp(lh, "1")) return 1;
@@ -517,7 +533,7 @@ static int select_kernels(imx_env* e) {
     const int m = e->m;
     pick_kernels(e, m_pad_of(e), e->div);
     const int epw = 32 / e->m_pad;
-    const int tile_bytes = (epw * m * e->O * (e->cfg.obs_f32 ? 4 : 8) + 15) & ~15;
+    const int tile_bytes = (epw * m * e->O * obs_elem_bytes(e) + 15) & ~15;
     e->step_smem = (size_t)(STEP_THREADS / 32) * tile_bytes;
     IMX_CUDA(raise_dyn_smem_limit((const void*)e->step_fn, e->step_smem));
     int dev_sms = 0, occ = 0;
@@ -614,6 +630,10 @@ static int derive(imx_env* e) {
     if (!(c.b != c.a)) return fail(-1, "rescale interval needs a != b");
     if (e->multi && !c.time_dependency && c.prev_actions && !c.prev_demand)
         return fail(-5, "Not Implemented");   // MAIM_env.py:135-136, MAIM_div_env.py:164-165
+    if (c.io_flags & ~(IMX_IO_OBS_BF16 | IMX_IO_ACTIONS_F32))
+        return fail(-1, "io_flags 0x%x has unknown bits (known: IMX_IO_OBS_BF16 = 1, IMX_IO_ACTIONS_F32 = 2)", (unsigned)c.io_flags);
+    if ((c.io_flags & IMX_IO_OBS_BF16) && c.obs_f32)
+        return fail(-1, "obs_f32 and IMX_IO_OBS_BF16 both set: choose one observation element type");
 
     e->D = 0;
     e->L = 0;
@@ -747,7 +767,8 @@ static void fill_args(const imx_env* e, StepArgs& A) {
     A.noisy = e->noisy_now;
     A.has_carry = e->has_carry;
     A.need_hd = e->need_hd; A.need_ho = e->need_ho;
-    A.obs_f32 = c.obs_f32 != 0;
+    A.obs_type = obs_type_of(c);
+    A.act_f32 = (c.io_flags & IMX_IO_ACTIONS_F32) ? 1 : 0;
     // watchdog thresholds: MAIM_div 2*dm, dm, dm, dm (:504,526,560,574); IM_div 4*dm, 2*dm, 2*dm, 2*dm (:424,449,483,497)
     A.wd_mult1 = e->multi ? 2 : 4;
     A.wd_mult = e->multi ? 1 : 2;
@@ -762,6 +783,7 @@ static void fill_args(const imx_env* e, StepArgs& A) {
     A.TL = e->TL;
     A.tab = e->d_tab;
     A.tabf = e->d_tab ? reinterpret_cast<const float*>(e->d_tab + (size_t)e->m * 4 * e->TL) : nullptr;   // float32 copy behind the float64 table
+    A.tabh = e->d_tab ? reinterpret_cast<const uint16_t*>(A.tabf + (size_t)e->m * 4 * e->TL) : nullptr; // bfloat16 copy behind that
     A.nodes = e->d_nodes;
     A.inv = (int32_t*)e->field_ptr[IMX_F_INV];
     A.backlog = (int32_t*)e->field_ptr[IMX_F_BACKLOG];
@@ -805,6 +827,20 @@ static std::vector<double> build_tables(const imx_env* e, int* TL_out) {
     }
     *TL_out = (int)TL;
     return tab;
+}
+
+// float32 -> bfloat16 bits, round to nearest even: the rounding of torch's float -> bfloat16 conversion (c10::BFloat16)
+static uint16_t round_bf16(float f) {
+    if (std::isnan(f)) return 0x7FC0;
+    uint32_t u;
+    memcpy(&u, &f, 4);
+    u += 0x7FFFu + ((u >> 16) & 1u);
+    return (uint16_t)(u >> 16);
+}
+extern "C" int imx_round_bf16(const float* in, uint16_t* out, int64_t n) {
+    if ((!in || !out) && n > 0) return fail(-1, "null argument");
+    for (int64_t k = 0; k < n; ++k) out[k] = round_bf16(in[k]);
+    return 0;
 }
 
 static std::vector<double> poisson_cdf(double mu) {
@@ -923,12 +959,16 @@ extern "C" int imx_create(const imx_config* cfg, imx_env** out) {
     {
         std::vector<double> tab = build_tables(e, &e->TL);
         if (e->TL > 0) {
-            // [m][4][TL] float64, then the same entries rounded to float32 (what an obs_f32 kernel stores: np.float32(obs64))
+            // [m][4][TL] float64, then the same entries rounded to float32 (what an obs_f32 kernel stores: np.float32(obs64)), then
+            // those rounded to bfloat16 (what an IMX_IO_OBS_BF16 kernel stores: torch's float64 -> bfloat16, which rounds through float32)
             std::vector<float> tabf(tab.size());
-            for (size_t k = 0; k < tab.size(); ++k) tabf[k] = (float)tab[k];
-            IMX_CREATE_CUDA(cudaMalloc(&e->d_tab, tab.size() * (sizeof(double) + sizeof(float))));
+            std::vector<uint16_t> tabh(tab.size());
+            for (size_t k = 0; k < tab.size(); ++k) { tabf[k] = (float)tab[k]; tabh[k] = round_bf16(tabf[k]); }
+            IMX_CREATE_CUDA(cudaMalloc(&e->d_tab, tab.size() * (sizeof(double) + sizeof(float) + sizeof(uint16_t))));
             IMX_CREATE_CUDA(cudaMemcpy(e->d_tab, tab.data(), tab.size() * sizeof(double), cudaMemcpyHostToDevice));
             IMX_CREATE_CUDA(cudaMemcpy(e->d_tab + tab.size(), tabf.data(), tab.size() * sizeof(float), cudaMemcpyHostToDevice));
+            IMX_CREATE_CUDA(cudaMemcpy(reinterpret_cast<float*>(e->d_tab + tab.size()) + tab.size(), tabh.data(), tab.size() * sizeof(uint16_t),
+                                       cudaMemcpyHostToDevice));
         }
     }
     {   // partial sums of the two-stage statistics: [statistic][slice] (imx_stats.cuh) or [2 x column][STATS_BLOCKS] (imx_eval.cuh)
@@ -1088,11 +1128,10 @@ extern "C" int imx_reset(imx_env* e, const int32_t* demand_dev, const uint8_t* d
 // and the ring's smaller resident tile count costs 5-10 %.
 static bool pipe_pays(const imx_env* e, int n_tiles) {
     (void)n_tiles;
-    const int64_t bytes_per_env = 8 * (int64_t)e->S + 4 * e->R + (int64_t)e->m * (16 + e->O * (e->cfg.obs_f32 ? 4 : 8));
-    if (e->step_et) return bytes_per_env * e->N <= ((int64_t)384 << 20);   // env-per-thread tiles: one-tile kernel from ~0.5 Mi envs (div2: 115 vs 124 us at 1 Mi)
+    if (e->step_et) return bytes_per_env(e) * e->N <= ((int64_t)384 << 20);   // env-per-thread tiles: one-tile kernel from ~0.5 Mi envs (div2: 115 vs 124 us at 1 Mi)
     if (e->div) return true;
     if (e->l2_hints) return true;                          // the priorities live in the pipelined kernel (serial 4-stage at 512 Ki envs: 38.0 vs 41.8 us)
-    return bytes_per_env * e->N <= ((int64_t)192 << 20);
+    return bytes_per_env(e) * e->N <= ((int64_t)192 << 20);
 }
 // CTAs launched per SM by the pipelined kernel (tiles are dealt round-robin over the grid).  Measured per family: 8 for the
 // 64-thread tiles of 4-wide chains, 6 for 8-lane divergent tiles and for the env-per-thread tiles (more CTAs than fit at once:
@@ -1117,9 +1156,16 @@ static int pipe_ctas_for(const imx_env* e, const TileLayout& L) {
 // in shared memory; *done receives how many periods the call really advanced (1 when the fused form is not applicable:
 // tail tiles, diagnostics, the direct path, a layout that does not fit).
 struct CcOut { void* dev; int fill; double lo, hi; };
+// The TMA kernels move a tile's actions, observations (and critic rows) as bulk copies, each of which must be a whole number of
+// 16-byte units; with 4- and 2-byte elements that depends on E * m (* O).  Where it does not hold, the direct kernel serves.
+static bool tile_io_whole16(const imx_env* e, const TileLayout& L, bool cc) {
+    const int64_t cells = (int64_t)L.E * e->m;
+    if ((cells * act_elem_bytes(e)) % 16 != 0 || (cells * e->O * obs_elem_bytes(e)) % 16 != 0) return false;
+    return !cc || (cells * ((e->m - 1) * (1 + e->O) + e->O) * obs_elem_bytes(e)) % 16 == 0;
+}
 constexpr unsigned ET_THREADS_HOST = 128;     // = imx::ET_THREADS of the env-per-thread rollout (device-only constant)
 
-static int launch_step(imx_env* e, const double* actions_dev, double* obs_dev, double* reward_dev,
+static int launch_step(imx_env* e, const void* actions_dev, double* obs_dev, double* reward_dev,
                        const imx_info_out* info, cudaStream_t s, int periods = 1, int* done = nullptr, const CcOut* cc = nullptr,
                        bool* cc_fused = nullptr) {
     if (e->t >= e->T) return fail(-6, "step() past the end of the episode (period %d of %d)", e->t, e->T);
@@ -1128,7 +1174,7 @@ static int launch_step(imx_env* e, const double* actions_dev, double* obs_dev, d
     const size_t cells_all = (size_t)e->N * e->m;
     A.periods = 1;
     A.act_stride = (int64_t)cells_all;
-    A.obs_stride_bytes = (int64_t)(cells_all * e->O * (e->cfg.obs_f32 ? 4 : 8));
+    A.obs_stride_bytes = (int64_t)(cells_all * e->O * obs_elem_bytes(e));
     A.rew_stride = (int64_t)(e->multi ? cells_all : (size_t)e->N);
     A.actions = actions_dev;
     A.obs = obs_dev;
@@ -1146,7 +1192,7 @@ static int launch_step(imx_env* e, const double* actions_dev, double* obs_dev, d
     const imxjit::Kernels* jk = nullptr;
     bool with_cc = false;
     if (cc_fused) *cc_fused = false;
-    if (cc && tma_legal && !A.has_info && obs_dev && aligned16(cc->dev)) {
+    if (cc && tma_legal && !A.has_info && obs_dev && aligned16(cc->dev) && tile_io_whole16(e, e->tile_cc, true)) {
         if (e->jit_cc_state == 0 && !stream_is_capturing(s)) ensure_jit_cc(e);
         const int64_t whole = (e->N / e->tile_cc.E) * e->tile_cc.E;
         if (e->jit_cc_state == 1 && whole == e->N) {       // fused only when every env sits in a whole tile (else: unfused fallback)
@@ -1171,7 +1217,7 @@ static int launch_step(imx_env* e, const double* actions_dev, double* obs_dev, d
     const TileLayout& TL_use = with_cc ? e->tile_cc : use_jit ? e->tile_jit : e->tile;
     const int epw_direct = 32 / e->m_pad;
     int64_t n_tma = 0;
-    if (tma_legal) {
+    if (tma_legal && (with_cc || tile_io_whole16(e, TL_use, false))) {
         n_tma = (e->N / TL_use.E) * TL_use.E;
         while (n_tma > 0 && (n_tma % epw_direct) != 0) n_tma -= TL_use.E;      // the tail kernel starts on a warp-tile boundary
     }
@@ -1240,7 +1286,7 @@ static int launch_step(imx_env* e, const double* actions_dev, double* obs_dev, d
     return 0;
 }
 
-extern "C" int imx_step(imx_env* e, const double* actions_dev, void* obs_dev, double* reward_dev,
+extern "C" int imx_step(imx_env* e, const void* actions_dev, void* obs_dev, double* reward_dev,
                         const imx_info_out* info, void* stream) {
     IMX_NVTX("imx_step");
 
@@ -1251,7 +1297,7 @@ extern "C" int imx_step(imx_env* e, const double* actions_dev, void* obs_dev, do
 
 // step() that also emits the centralised-critic observation rows.  Fused into the step kernel's epilogue wherever the
 // runtime-specialised TMA kernels serve the whole batch; otherwise the plain step followed by the gather kernel.
-extern "C" int imx_step_cc(imx_env* e, const double* actions_dev, void* obs_dev, void* cc_dev, int fill_actions, double clip_lo,
+extern "C" int imx_step_cc(imx_env* e, const void* actions_dev, void* obs_dev, void* cc_dev, int fill_actions, double clip_lo,
                            double clip_hi, double* reward_dev, void* stream) {
     IMX_NVTX("imx_step_cc");
 
@@ -1263,7 +1309,7 @@ extern "C" int imx_step_cc(imx_env* e, const double* actions_dev, void* obs_dev,
     if (!obs) {                                              // the rows are built from the observation tile either way
         if (!e->d_obs_scratch) {
             if (stream_is_capturing(s)) return fail(-1, "imx_step_cc without obs_dev under stream capture: call imx_prepare(IMX_PREPARE_CC) first");
-            IMX_CUDA(cudaMalloc(&e->d_obs_scratch, (size_t)e->N * e->m * e->O * (e->cfg.obs_f32 ? 4 : 8)));
+            IMX_CUDA(cudaMalloc(&e->d_obs_scratch, (size_t)e->N * e->m * e->O * obs_elem_bytes(e)));
         }
         obs = e->d_obs_scratch;
     }
@@ -1271,7 +1317,7 @@ extern "C" int imx_step_cc(imx_env* e, const double* actions_dev, void* obs_dev,
     bool fused = false;
     const int rc = launch_step(e, actions_dev, (double*)obs, reward_dev, nullptr, s, 1, nullptr, &cc, &fused);
     if (rc || fused) return rc;
-    return imx_cc_observe(e, obs, fill_actions ? actions_dev : nullptr, clip_lo, clip_hi, cc_dev, e->cfg.obs_f32 ? 1 : 0, stream);
+    return imx_cc_observe(e, obs, fill_actions ? actions_dev : nullptr, clip_lo, clip_hi, cc_dev, obs_type_of(e->cfg), stream);
 }
 
 static int ensure_host_path(imx_env* e);
@@ -1286,7 +1332,7 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
     if (flags & IMX_PREPARE_HOST) { const int rc = ensure_host_path(e); if (rc) return rc; }
     if ((flags & IMX_PREPARE_CC) && e->multi) {
         ensure_jit_cc(e);
-        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, (size_t)e->N * e->m * e->O * (e->cfg.obs_f32 ? 4 : 8)));
+        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, (size_t)e->N * e->m * e->O * obs_elem_bytes(e)));
     }
     if ((flags & IMX_PREPARE_DFO) && !e->multi && !e->d_dfo_rewards)
         IMX_CUDA(cudaMalloc(&e->d_dfo_rewards, (size_t)e->T * e->N * sizeof(double)));
@@ -1298,7 +1344,7 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
         if (!e->d_ep_profit) IMX_CUDA(cudaMalloc(&e->d_ep_profit, cells * sizeof(double)));
         if (!e->d_ep_ret) IMX_CUDA(cudaMalloc(&e->d_ep_ret, (size_t)e->N * cols * sizeof(double)));
         if (!e->d_ep_stats) IMX_CUDA(cudaMalloc(&e->d_ep_stats, (3 + 2 * (size_t)e->m) * sizeof(double)));
-        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, cells * e->O * (e->cfg.obs_f32 ? 4 : 8)));
+        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, cells * e->O * obs_elem_bytes(e)));
     }
     IMX_CUDA(cudaDeviceSynchronize());
     return 0;
@@ -1307,7 +1353,7 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
 // K consecutive periods on pre-computed actions: one launch that keeps every tile's state in shared memory for all K
 // periods (actions / demand prefetched two periods ahead, observations / rewards streamed out behind the compute)
 // wherever the whole batch goes through the TMA kernel; otherwise K plain launches.  Same results either way.
-extern "C" int imx_step_many(imx_env* e, const double* actions_dev, int K, void* obs_dev, double* reward_dev,
+extern "C" int imx_step_many(imx_env* e, const void* actions_dev, int K, void* obs_dev, double* reward_dev,
                              const imx_info_out* info, void* stream) {
     IMX_NVTX("imx_step_many");
 
@@ -1316,7 +1362,7 @@ extern "C" int imx_step_many(imx_env* e, const double* actions_dev, int K, void*
     if (e->t + K > e->T) return fail(-6, "imx_step_many: %d periods from period %d run past the end of the episode (%d)", K, e->t, e->T);
     IMX_CUDA(cudaSetDevice(e->cfg.device));
     const size_t cells = (size_t)e->N * e->m;
-    const size_t obs_stride = cells * e->O * (e->cfg.obs_f32 ? 4 : 8);
+    const size_t obs_stride = cells * e->O * obs_elem_bytes(e), act_stride = cells * act_elem_bytes(e);
     const size_t rew_stride = e->multi ? cells : (size_t)e->N;
     int j = 0;
     while (j < K) {
@@ -1329,7 +1375,7 @@ extern "C" int imx_step_many(imx_env* e, const double* actions_dev, int K, void*
             at.order_dev = info->order_dev ? info->order_dev + (size_t)j * cells : nullptr;
             at.profit_dev = info->profit_dev ? info->profit_dev + (size_t)j * cells : nullptr;
         }
-        const int rc = launch_step(e, actions_dev + (size_t)j * cells,
+        const int rc = launch_step(e, (const unsigned char*)actions_dev + (size_t)j * act_stride,
                                    obs_dev ? (double*)((unsigned char*)obs_dev + (size_t)j * obs_stride) : nullptr,
                                    reward_dev + (size_t)j * rew_stride, info ? &at : nullptr, (cudaStream_t)stream, K - j, &adv);
         if (rc) return rc;
@@ -1358,7 +1404,7 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
     const bool capturing = stream_is_capturing(s);
     const int64_t N = e->N;
     const int m = e->m;
-    const size_t cols = e->multi ? m : 1, cells = (size_t)N * m, es = e->cfg.obs_f32 ? 4 : 8;
+    const size_t cols = e->multi ? m : 1, cells = (size_t)N * m, es = obs_elem_bytes(e), aes = act_elem_bytes(e);
     if (!capturing) ensure_jit_episode(e, obs_dev != nullptr);
     const imxjit::Kernels* jk = obs_dev ? e->jit_ep : e->jit_ep_noobs;
     EpisodeArgs EA;
@@ -1374,7 +1420,7 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
     // -7 to -12 %, div1 with observations -6 % at 32 768 envs), so the composition serves them
     const bool pays = !e->div || (e->step_et ? obs_dev != nullptr : obs_dev == nullptr);
     const bool fused = pays && jk && jk->step_episode && e->step_path != 1 && e->fuse_periods && N % 4 == 0 && N % E == 0 && E % 2 == 0 &&
-                       smem <= 200 * 1024 && aligned16(actions_dev) && aligned16(obs_dev) && aligned16(reward_dev) && aligned16(return_dev) &&
+                       smem <= 200 * 1024 && tile_io_whole16(e, e->tile_jit, false) && aligned16(actions_dev) && aligned16(obs_dev) && aligned16(reward_dev) && aligned16(return_dev) &&
                        aligned16(eval_acc_dev) && (!demand_dev || (aligned16(demand_dev) && (E * e->R * e->T) % 4 == 0));
     // internal buffers are allocated here (never under capture: imx_prepare(IMX_PREPARE_EPISODE) allocates them up front),
     // before anything is launched
@@ -1455,7 +1501,7 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
             memset(&info, 0, sizeof(info));
             info.profit_dev = e->d_ep_profit;
             void* ob = obs_dev ? (void*)((unsigned char*)obs_dev + (size_t)t * cells * e->O * es) : e->d_obs_scratch;
-            if ((rc = launch_step(e, actions_dev + (size_t)t * cells, (double*)ob, rew + (size_t)t * rstride, &info, s))) return rc;
+            if ((rc = launch_step(e, (const unsigned char*)actions_dev + (size_t)t * cells * aes, (double*)ob, rew + (size_t)t * rstride, &info, s))) return rc;
             if ((rc = imx_eval_accumulate(e, ob, rew + (size_t)t * rstride, e->d_ep_profit, eval_acc_dev, t == 0, stream))) return rc;
         }
     }
@@ -1614,7 +1660,7 @@ extern "C" int imx_eval_accumulate(imx_env* e, const void* obs_dev, const double
     EvalArgs E;
     memset(&E, 0, sizeof(E));
     E.obs = obs_dev; E.reward = reward_dev; E.profit = profit_dev; E.acc = acc_dev; E.nodes = e->d_nodes;
-    E.N = e->N; E.m = e->m; E.O = e->O; E.multi = e->multi ? 1 : 0; E.obs_f32 = e->cfg.obs_f32 ? 1 : 0;
+    E.N = e->N; E.m = e->m; E.O = e->O; E.multi = e->multi ? 1 : 0; E.obs_type = obs_type_of(e->cfg);
     E.rescaled = (e->cfg.kind == IMX_KIND_MAIM_DIV || e->cfg.standardise_state) ? 1 : 0;
     E.reset = reset ? 1 : 0;
     E.a = e->cfg.a; E.bma = e->cfg.b - e->cfg.a;
@@ -1644,7 +1690,7 @@ static int ensure_host_path(imx_env* e) {
     cudaError_t rc = cudaSuccess;
     auto take = [&](void** p, size_t bytes) { if (rc == cudaSuccess && !*p) rc = cudaMalloc(p, bytes); };
     take((void**)&e->d_act_h, cells * sizeof(double));
-    take((void**)&e->d_obs_h, cells * e->O * (e->cfg.obs_f32 ? 4 : 8));
+    take((void**)&e->d_obs_h, cells * e->O * obs_elem_bytes(e));
     take((void**)&e->d_rew_h, cells * sizeof(double));
     take((void**)&e->d_dem_h, (size_t)e->N * e->R * e->T * sizeof(int32_t));
     if (e->has_carry) take((void**)&e->d_mask_h, (size_t)e->N * e->T * e->m);
@@ -1678,7 +1724,7 @@ extern "C" int imx_reset_host(imx_env* e, const int32_t* demand_host, const uint
                    obs_host ? e->d_obs_h : nullptr, s);
     if (rc) return rc;
     if (obs_host)
-        IMX_CUDA(cudaMemcpyAsync(obs_host, e->d_obs_h, (size_t)e->N * e->m * e->O * (e->cfg.obs_f32 ? 4 : 8), cudaMemcpyDeviceToHost, s));
+        IMX_CUDA(cudaMemcpyAsync(obs_host, e->d_obs_h, (size_t)e->N * e->m * e->O * obs_elem_bytes(e), cudaMemcpyDeviceToHost, s));
     IMX_CUDA(cudaStreamSynchronize(s));
     return 0;
 }
@@ -1692,7 +1738,7 @@ static void* pinned_alias(const void* host_ptr) {
     return at.devicePointer;
 }
 
-extern "C" int imx_step_host(imx_env* e, const double* actions_host, void* obs_host, double* reward_host) {
+extern "C" int imx_step_host(imx_env* e, const void* actions_host, void* obs_host, double* reward_host) {
     IMX_NVTX("imx_step_host");
 
     if (!e || !actions_host || !reward_host) return fail(-1, "null argument");
@@ -1703,7 +1749,7 @@ extern "C" int imx_step_host(imx_env* e, const double* actions_host, void* obs_h
     const size_t cells = (size_t)e->N * e->m;
     // Zero-copy fast path: with pinned buffers the kernel's bulk loads / stores address host memory
     // directly over PCIe (UVA), so transfer and compute overlap tile by tile and no staging copy exists.
-    const double* act_d = (const double*)pinned_alias(actions_host);
+    const void* act_d = pinned_alias(actions_host);
     double* obs_d = obs_host ? (double*)pinned_alias(obs_host) : nullptr;
     double* rew_d = (double*)pinned_alias(reward_host);
     const bool zero_copy = e->host_zero_copy && act_d && rew_d && (obs_d || !obs_host);
@@ -1718,10 +1764,10 @@ extern "C" int imx_step_host(imx_env* e, const double* actions_host, void* obs_h
         IMX_CUDA(cudaStreamSynchronize(s));
         return 0;
     }
-    IMX_CUDA(cudaMemcpyAsync(e->d_act_h, actions_host, cells * sizeof(double), cudaMemcpyHostToDevice, s));
+    IMX_CUDA(cudaMemcpyAsync(e->d_act_h, actions_host, cells * act_elem_bytes(e), cudaMemcpyHostToDevice, s));
     rc = launch_step(e, e->d_act_h, obs_host ? e->d_obs_h : nullptr, e->d_rew_h, nullptr, s);
     if (rc) return rc;
-    if (obs_host) IMX_CUDA(cudaMemcpyAsync(obs_host, e->d_obs_h, cells * e->O * (e->cfg.obs_f32 ? 4 : 8), cudaMemcpyDeviceToHost, s));
+    if (obs_host) IMX_CUDA(cudaMemcpyAsync(obs_host, e->d_obs_h, cells * e->O * obs_elem_bytes(e), cudaMemcpyDeviceToHost, s));
     IMX_CUDA(cudaMemcpyAsync(reward_host, e->d_rew_h, (e->multi ? cells : (size_t)e->N) * sizeof(double), cudaMemcpyDeviceToHost, s));
     IMX_CUDA(cudaStreamSynchronize(s));
     return 0;
@@ -1791,10 +1837,11 @@ extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* l
 // --------------------------------------------------------------------------------------
 extern "C" int imx_cc_obs_len(const imx_env* e) { return e ? (e->m - 1) * (1 + e->O) + e->O : fail(-1, "null env"); }
 
-extern "C" int imx_cc_observe(imx_env* e, const void* obs_dev, const double* actions_dev, double clip_lo, double clip_hi,
+extern "C" int imx_cc_observe(imx_env* e, const void* obs_dev, const void* actions_dev, double clip_lo, double clip_hi,
                               void* out_dev, int out_is_f32, void* stream) {
     if (!e || !obs_dev || !out_dev) return fail(-1, "null argument");
     if (!e->multi) return fail(-1, "the centralised-critic observation is defined for the multi-agent kinds");
+    if (out_is_f32 < 0 || out_is_f32 > 2) return fail(-1, "out_is_f32 must be 0 (float64), 1 (float32) or 2 (bfloat16)");
     IMX_CUDA(cudaSetDevice(e->cfg.device));
     const int W = (e->m - 1) * (1 + e->O) + e->O;
     const int64_t total = e->N * e->m * W;
@@ -1803,13 +1850,19 @@ extern "C" int imx_cc_observe(imx_env* e, const void* obs_dev, const double* act
     const int64_t want = (total + 255) / 256;
     const unsigned grid = (unsigned)(want < (int64_t)sms * 16 ? want : (int64_t)sms * 16);
     cudaStream_t s = (cudaStream_t)stream;
-    if (e->cfg.obs_f32) {                        // the env writes float32 observations: read them as such
-        if (out_is_f32) cc_observer_kernel<float, float><<<grid, 256, 0, s>>>((const float*)obs_dev, actions_dev, (float*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
-        else cc_observer_kernel<float, double><<<grid, 256, 0, s>>>((const float*)obs_dev, actions_dev, (double*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
-    } else {
-        if (out_is_f32) cc_observer_kernel<double, float><<<grid, 256, 0, s>>>((const double*)obs_dev, actions_dev, (float*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
-        else cc_observer_kernel<double, double><<<grid, 256, 0, s>>>((const double*)obs_dev, actions_dev, (double*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
-    }
+    const int af = act_elem_bytes(e) == 4 ? 1 : 0;
+    // the observations are read in the element type the env writes, the rows written in the one asked for
+    auto launch = [&](auto in_tag) {
+        using InT = decltype(in_tag);
+        const InT* in = (const InT*)obs_dev;
+        if (out_is_f32 == 2) cc_observer_kernel<InT, Bf16><<<grid, 256, 0, s>>>(in, actions_dev, af, (Bf16*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
+        else if (out_is_f32) cc_observer_kernel<InT, float><<<grid, 256, 0, s>>>(in, actions_dev, af, (float*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
+        else cc_observer_kernel<InT, double><<<grid, 256, 0, s>>>(in, actions_dev, af, (double*)out_dev, e->N, e->m, e->O, clip_lo, clip_hi);
+    };
+    const int ot = obs_type_of(e->cfg);
+    if (ot == OBS_BF16) launch(Bf16{});
+    else if (ot == OBS_F32) launch(0.0f);
+    else launch(0.0);
     IMX_CHECK_LAUNCH("cc_observer_kernel");
     return 0;
 }

@@ -12,8 +12,18 @@
 
 namespace imx {
 
+// Element types: double, float, and Bf16 (bit pattern; widened exactly, narrowed as torch does: float64 -> float32 -> bfloat16).
+struct Bf16 { uint16_t u; };
+__device__ __forceinline__ double widen(double x) { return x; }
+__device__ __forceinline__ double widen(float x) { return (double)x; }
+__device__ __forceinline__ double widen(Bf16 x) { return (double)bf16_to_f32(x.u); }
+template <typename T> __device__ __forceinline__ T narrow(double v);
+template <> __device__ __forceinline__ double narrow<double>(double v) { return v; }
+template <> __device__ __forceinline__ float narrow<float>(double v) { return (float)v; }
+template <> __device__ __forceinline__ Bf16 narrow<Bf16>(double v) { return Bf16{f32_to_bf16((float)v)}; }
+
 template <typename InT, typename OutT>
-__global__ void __launch_bounds__(256) cc_observer_kernel(const InT* __restrict__ obs, const double* __restrict__ actions,
+__global__ void __launch_bounds__(256) cc_observer_kernel(const InT* __restrict__ obs, const void* __restrict__ actions, int act_f32,
                                                           OutT* __restrict__ out, int64_t N, int m, int O, double lo, double hi) {
     const int W = (m - 1) * (1 + O) + O;
     const int64_t total = N * m * W;
@@ -25,16 +35,16 @@ __global__ void __launch_bounds__(256) cc_observer_kernel(const InT* __restrict_
         double v;
         if (w < m - 1) {
             const int j = w < i ? w : w + 1;
-            v = actions ? fmin(fmax(actions[n * m + j], lo), hi) : 0.0;
+            v = actions ? fmin(fmax(load_action(actions, n * m + j, act_f32 != 0), lo), hi) : 0.0;
         } else if (w < (m - 1) * (1 + O)) {
             const int q = w - (m - 1);
             const int slot = q / O, k = q - slot * O;
             const int j = slot < i ? slot : slot + 1;
-            v = (double)obs[(n * m + j) * O + k];
+            v = widen(obs[(n * m + j) * O + k]);
         } else {
-            v = (double)obs[(n * m + i) * O + (w - (m - 1) * (1 + O))];
+            v = widen(obs[(n * m + i) * O + (w - (m - 1) * (1 + O))]);
         }
-        out[idx] = (OutT)v;
+        out[idx] = narrow<OutT>(v);
     }
 }
 

@@ -110,7 +110,8 @@ struct StepArgs {
     int32_t has_carry;         // carry field allocated
     int32_t need_hd, need_ho;  // history state present
     int32_t has_info;          // any imx_info_out pointer set
-    int32_t obs_f32;           // observations are written as float32 (the cast of the float64 value), else float64
+    int32_t obs_type;          // element type of the observations: OBS_F64, OBS_F32 (the float32 cast of the float64 value) or OBS_BF16
+    int32_t act_f32;           // actions are read as float32 (widened to float64 before decoding), else float64
     int32_t wd_mult1, wd_mult;   // watchdog multipliers: LOOP1(A) and the other three
     double a, b, bma;          // bma = b - a
     double inv_bma;            // 1/(b-a) when b-a is a power of two (the division is then an exact scaling), else 0
@@ -120,6 +121,7 @@ struct StepArgs {
     int32_t pad_tl;
     const double* __restrict__ tab;         // [m][4][TL] exact rescale results, see build_tables() in imx_api.cu
     const float* __restrict__ tabf;         // the same table rounded to float32 (obs_f32: the value is stored as loaded, no conversion in the kernel)
+    const uint16_t* __restrict__ tabh;      // the float32 table rounded to bfloat16 (round to nearest even), bit patterns
     const NodeParams* __restrict__ nodes;   // [m]
     // state (SoA, int32)
     int32_t* __restrict__ inv;
@@ -134,7 +136,7 @@ struct StepArgs {
     const int32_t* __restrict__ demand_T;   // [T][R][N]
     const uint8_t* __restrict__ mask_T;     // [T][N][m]
     // I/O
-    const double* __restrict__ actions;     // [N][m]
+    const void* __restrict__ actions;       // [N][m] float64, or float32 when act_f32
     double* __restrict__ obs;               // [N][m][O]
     double* __restrict__ reward;            // [N][m] or [N]
     imx_info_out info;
@@ -142,7 +144,7 @@ struct StepArgs {
     // resident in shared memory; period j reads actions + j * act_stride and writes obs / reward slices j
     int32_t periods;                        // >= 1 (1 = plain step)
     int32_t m_pow2;                         // m is a power of two
-    int64_t act_stride;                     // doubles between consecutive periods' action blocks
+    int64_t act_stride;                     // action elements between consecutive periods' action blocks
     int64_t obs_stride_bytes;               // bytes between consecutive periods' observation blocks
     int64_t rew_stride;                     // doubles between consecutive periods' reward blocks
     // centralised-critic observation emitted by the step itself (imx_step_cc; models/CC_Model.py:165-214): for every agent the
@@ -223,34 +225,69 @@ __device__ __forceinline__ double div_by_m(double s, int m, double inv_m, bool m
     const double rem = __fma_rn(-q0, (double)m, s);
     return __fma_rn(rem, inv_m, q0);
 }
-// float32 observations: the table entry rounded once on the host ((float)tab[v] == np.float32(obs64)) — one 4-byte load and no
-// F2F.F32.F64 in the kernel (conversions run at a fraction of the FP64 rate; 7 per lane made the float32 step of config 2
-// SLOWER than the float64 one although it writes 112 fewer bytes per env)
-__device__ __forceinline__ float scaled_f32(const float* __restrict__ tabrow_f, int TL, int which, int v) {
+// Observation element types (StepArgs.obs_type; the runtime-specialised build injects it as a literal).  bfloat16 elements are
+// what torch's float64 -> bfloat16 conversion gives, which rounds through float32: round-to-nearest-even of the float32 element.
+enum : int { OBS_F64 = 0, OBS_F32 = 1, OBS_BF16 = 2 };
+__host__ __device__ constexpr int obs_elem_bytes(int type) { return type == OBS_BF16 ? 2 : type == OBS_F32 ? 4 : 8; }
+
+// float32 -> bfloat16 bits, round to nearest even (one F2FP; observations are never NaN)
+__device__ __forceinline__ uint16_t f32_to_bf16(float x) {
+    uint16_t r;
+    asm("cvt.rn.bf16.f32 %0, %1;" : "=h"(r) : "f"(x));
+    return r;
+}
+__device__ __forceinline__ float bf16_to_f32(uint16_t u) { return __uint_as_float((uint32_t)u << 16); }
+// the value an observation element of type `type` holds for the float64 value x, widened back to float64
+__device__ __forceinline__ double obs_stored(int type, double x) {
+    if (type == OBS_F32) return (double)(float)x;
+    if (type == OBS_BF16) return (double)bf16_to_f32(f32_to_bf16((float)x));
+    return x;
+}
+// One action element, widened to float64 (exact for float32, so decode_order sees the same value a float64 caller passes)
+__device__ __forceinline__ double load_action(const void* __restrict__ p, int64_t k, bool f32) {
+    return f32 ? (double)reinterpret_cast<const float*>(p)[k] : reinterpret_cast<const double*>(p)[k];
+}
+
+// Reduced-precision observations: the table entry rounded on the host (float32: (float)tab[v] == np.float32(obs64); bfloat16:
+// that float32 rounded to nearest even) — one 4- or 2-byte load and no F2F in the kernel (conversions run at a fraction of the
+// FP64 rate; 7 per lane made the float32 step of config 2 SLOWER than the float64 one although it writes 112 fewer bytes per env)
+template <typename T>
+__device__ __forceinline__ T scaled_lp(const T* __restrict__ tabrow_lp, int TL, int which, int v) {
 #ifdef IMX_DEBUG_BOUNDS
     if ((unsigned)v >= (unsigned)TL) __trap();
 #endif
-    return __ldg(tabrow_f + which * TL + (int)min((unsigned)v, (unsigned)(TL - 1)));
+    return __ldg(tabrow_lp + which * TL + (int)min((unsigned)v, (unsigned)(TL - 1)));
 }
-// One observation element.  `row` addresses the agent's vector in the output element type.
-#define OBS_PUT(row, k, v)                                                           \
-    do {                                                                             \
-        if (KF(obs_f32)) reinterpret_cast<float*>(row)[k] = (float)(v);              \
-        else reinterpret_cast<double*>(row)[k] = (v);                                \
+// Row of the reduced-precision table for node i (null for float64 observations or without tables).
+#define OBS_TABROW_LP(A, i, TL)                                                                                          \
+    (!KHAS(tab) ? (const void*)nullptr                                                                                   \
+     : KF(obs_type) == OBS_F32 ? (const void*)((A).tabf + (size_t)(i) * 4 * (TL))                                        \
+     : KF(obs_type) == OBS_BF16 ? (const void*)((A).tabh + (size_t)(i) * 4 * (TL)) : (const void*)nullptr)
+
+// The single writer of an observation element.  `row` addresses the agent's vector in the output element type.
+#define OBS_PUT(row, k, v)                                                                                               \
+    do {                                                                                                                 \
+        if (KF(obs_type) == OBS_BF16) reinterpret_cast<uint16_t*>(row)[k] = f32_to_bf16((float)(v));                     \
+        else if (KF(obs_type) == OBS_F32) reinterpret_cast<float*>(row)[k] = (float)(v);                                  \
+        else reinterpret_cast<double*>(row)[k] = (v);                                                                    \
     } while (0)
 
-// A rescaled element (scaled() above) and a raw integer element: for float32 rows the float table / the int -> float
-// conversion give the bits of np.float32(float64 value) directly ((float)(double)i == (float)i for every int).
-#define OBS_PUT_SCALED(row, k, CHECKED_, tabrow, tabrow_f, TL, which, v, vmax, a, bma)                                   \
+// A rescaled element (scaled() above) and a raw integer element: for reduced-precision rows the host-rounded table / the
+// int -> float conversion give the bits of the float32 (then bfloat16) rounding of the float64 value directly
+// ((float)(double)i == (float)i for every int).
+#define OBS_PUT_SCALED(row, k, CHECKED_, tabrow, tabrow_lp, TL, which, v, vmax, a, bma)                                  \
     do {                                                                                                                 \
-        if (KF(obs_f32) && KHAS(tab) && (!(CHECKED_) || (unsigned)(v) < (unsigned)(TL)))                                  \
-            reinterpret_cast<float*>(row)[k] = scaled_f32(tabrow_f, TL, which, v);                                        \
-        else OBS_PUT(row, k, scaled<CHECKED_>(KHAS(tab), tabrow, TL, which, v, vmax, a, bma));                            \
+        if (KF(obs_type) != OBS_F64 && KHAS(tab) && (!(CHECKED_) || (unsigned)(v) < (unsigned)(TL))) {                     \
+            if (KF(obs_type) == OBS_BF16)                                                                                \
+                reinterpret_cast<uint16_t*>(row)[k] = scaled_lp(reinterpret_cast<const uint16_t*>(tabrow_lp), TL, which, v); \
+            else reinterpret_cast<float*>(row)[k] = scaled_lp(reinterpret_cast<const float*>(tabrow_lp), TL, which, v);  \
+        } else OBS_PUT(row, k, scaled<CHECKED_>(KHAS(tab), tabrow, TL, which, v, vmax, a, bma));                          \
     } while (0)
-#define OBS_PUT_INT(row, k, v)                                                       \
-    do {                                                                             \
-        if (KF(obs_f32)) reinterpret_cast<float*>(row)[k] = (float)(v);              \
-        else reinterpret_cast<double*>(row)[k] = (double)(v);                        \
+#define OBS_PUT_INT(row, k, v)                                                                                           \
+    do {                                                                                                                 \
+        if (KF(obs_type) == OBS_BF16) reinterpret_cast<uint16_t*>(row)[k] = f32_to_bf16((float)(v));                     \
+        else if (KF(obs_type) == OBS_F32) reinterpret_cast<float*>(row)[k] = (float)(v);                                  \
+        else reinterpret_cast<double*>(row)[k] = (double)(v);                                                            \
     } while (0)
 
 // profit = p*ship - c*order - h*|inv' - target| - bc*backlog'           MAIM_env.py:421-424

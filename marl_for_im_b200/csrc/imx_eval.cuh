@@ -22,13 +22,13 @@ namespace imx {
 constexpr int EVAL_FIXED = 4;
 
 struct EvalArgs {
-    const void* __restrict__ obs;        // [N][m][O] float64 (float32 when obs_f32)
+    const void* __restrict__ obs;        // [N][m][O] in the handle's observation type (OBS_F64 / OBS_F32 / OBS_BF16)
     const double* __restrict__ reward;   // MAIM kinds [N][m], IM kinds [N]
     const double* __restrict__ profit;   // [N][m] or null (stage_profit columns are then left untouched)
     double* __restrict__ acc;            // [N][4 + m]
     const NodeParams* __restrict__ nodes;
     int64_t N;
-    int32_t m, O, multi, obs_f32;
+    int32_t m, O, multi, obs_type;
     int32_t rescaled;                    // observations are standardised: undo with rev_scale (MAIM_env.py:509-519)
     int32_t reset;                       // start a new episode: accumulators begin at 0 instead of acc's contents
     double a, bma;
@@ -44,7 +44,10 @@ __global__ void __launch_bounds__(256) eval_accumulate_kernel(const __grid_const
     if (!E.multi) ep = __dadd_rn(ep, E.reward[n]);                      // inv_management.py:596 "episode_reward += reward"
     for (int i = 0; i < m; ++i) {
         double x0, x1;
-        if (E.obs_f32) {
+        if (E.obs_type == OBS_BF16) {
+            const uint16_t* o = reinterpret_cast<const uint16_t*>(E.obs) + (n * m + i) * O;
+            x0 = (double)bf16_to_f32(o[0]); x1 = (double)bf16_to_f32(o[1]);
+        } else if (E.obs_type == OBS_F32) {
             const float* o = reinterpret_cast<const float*>(E.obs) + (n * m + i) * O;
             x0 = (double)o[0]; x1 = (double)o[1];
         } else {

@@ -23,11 +23,14 @@ struct ResetArgs {
 };
 constexpr int RESET_T_CHUNK = 8;   // periods one thread transposes
 
-template <int DMAX, int PMAX>
-__global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ StepArgs A, const __grid_constant__ ResetArgs Z, int div) {
+// OT: the observation element type as a template constant (one instantiation per type: no type branches on the fill paths)
+template <int DMAX, int PMAX, int OT>
+__global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ StepArgs A_, const __grid_constant__ ResetArgs Z, int div) {
     extern __shared__ __align__(16) double s_tmpl[];                  // [m][O] observation template (8 bytes reserved per element), then int init_inv[m]
+    StepArgs A = A_;                                                  // (the fields read below stay parameter-space loads)
+    A.obs_type = OT;
     const int m = A.m, O = A.O;
-    const int es = A.obs_f32 ? 4 : 8;
+    const int es = obs_elem_bytes(OT);
     int32_t* s_init = reinterpret_cast<int32_t*>(s_tmpl + m * O);
     // everything this kernel writes may still be read by the kernel in front of it (it is launched as a programmatic dependent)
     asm volatile("griddepcontrol.wait;" ::: "memory");
@@ -82,7 +85,6 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
         // every env's initial observation is the same m*O-element template: 16-byte stores where the template
         // length allows it, and the position inside the template advances by (stride mod len) per iteration
         // instead of a 64-bit modulo per element
-        const int es = A.obs_f32 ? 4 : 8;
         const int64_t bytes = A.N * m * O * es;
         const int tmpl_bytes = m * O * es;
         if ((tmpl_bytes & 15) == 0 && (reinterpret_cast<uintptr_t>(A.obs) & 15) == 0) {
@@ -103,7 +105,8 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
             const int step = (int)(stride % len);
             int rem = (int)(gtid % len);
             for (int64_t k = gtid; k < total; k += stride) {
-                if (A.obs_f32) reinterpret_cast<float*>(A.obs)[k] = reinterpret_cast<const float*>(s_tmpl)[rem];
+                if (OT == OBS_BF16) reinterpret_cast<uint16_t*>(A.obs)[k] = reinterpret_cast<const uint16_t*>(s_tmpl)[rem];
+                else if (OT == OBS_F32) reinterpret_cast<float*>(A.obs)[k] = reinterpret_cast<const float*>(s_tmpl)[rem];
                 else A.obs[k] = s_tmpl[rem];
                 rem += step;
                 if (rem >= len) rem -= len;

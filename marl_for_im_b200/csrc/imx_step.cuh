@@ -231,11 +231,11 @@ __device__ __forceinline__ void write_obs_row(void* row, const StepArgs& A, cons
     const double inv_max = (double)np.inv_max, order_max = (double)np.order_max;
     const double dem_max = (double)np.demand_max;
     const double ou_max = KF(multi) ? order_max : inv_max;   // MAIM_env.py:300 vs IM_env.py:265
-    const float* __restrict__ tabrow_f = (KF(obs_f32) && KHAS(tab)) ? A.tabf + (size_t)node_idx * 4 * TL : nullptr;
+    const void* tabrow_lp = OBS_TABROW_LP(A, node_idx, TL);
     if (KF(std_state)) {
-        OBS_PUT_SCALED(row, 0, CHECKED, tabrow, tabrow_f, TL, TAB_INV, inv, inv_max, a, bma);
-        OBS_PUT_SCALED(row, 1, CHECKED, tabrow, tabrow_f, TL, TAB_DEM, backlog, dem_max, a, bma);
-        OBS_PUT_SCALED(row, 2, CHECKED, tabrow, tabrow_f, TL, KF(multi) ? TAB_ORD : TAB_INV, order_u, ou_max, a, bma);
+        OBS_PUT_SCALED(row, 0, CHECKED, tabrow, tabrow_lp, TL, TAB_INV, inv, inv_max, a, bma);
+        OBS_PUT_SCALED(row, 1, CHECKED, tabrow, tabrow_lp, TL, TAB_DEM, backlog, dem_max, a, bma);
+        OBS_PUT_SCALED(row, 2, CHECKED, tabrow, tabrow_lp, TL, KF(multi) ? TAB_ORD : TAB_INV, order_u, ou_max, a, bma);
     } else {
         OBS_PUT_INT(row, 0, inv);
         OBS_PUT_INT(row, 1, backlog);
@@ -256,7 +256,7 @@ __device__ __forceinline__ void write_obs_row(void* row, const StepArgs& A, cons
 #pragma unroll
         for (int j = 0; j < PMAX; ++j)
             if (j < KF(P)) {
-                if (KF(write_hd)) OBS_PUT_SCALED(row, k0 + j, CHECKED, tabrow, tabrow_f, TL, TAB_DEM, hd[j], dem_max, a, bma);
+                if (KF(write_hd)) OBS_PUT_SCALED(row, k0 + j, CHECKED, tabrow, tabrow_lp, TL, TAB_DEM, hd[j], dem_max, a, bma);
                 else OBS_PUT(row, k0 + j, 0.0);             // quirk 2
             }
         k0 += KF(P);
@@ -264,7 +264,7 @@ __device__ __forceinline__ void write_obs_row(void* row, const StepArgs& A, cons
     if (KF(pa)) {
 #pragma unroll
         for (int j = 0; j < PMAX; ++j)
-            if (j < KF(P)) OBS_PUT_SCALED(row, k0 + j, CHECKED, tabrow, tabrow_f, TL, TAB_ORD, ho[j], order_max, a, bma);
+            if (j < KF(P)) OBS_PUT_SCALED(row, k0 + j, CHECKED, tabrow, tabrow_lp, TL, TAB_ORD, ho[j], order_max, a, bma);
         k0 += KF(P);
     }
     if (KF(td)) {
@@ -272,8 +272,8 @@ __device__ __forceinline__ void write_obs_row(void* row, const StepArgs& A, cons
         for (int k = 0; k < DMAX; ++k) {
             if (k < KF(D)) {
                 if (!KF(std_state)) OBS_PUT_INT(row, k0 + k, pipe[k]);                      // IM kinds, raw
-                else if (div && KF(multi)) OBS_PUT_SCALED(row, k0 + k, CHECKED, tabrow, tabrow_f, TL, TAB_PIPE2, min(pipe[k], 2 * np.inv_max), 2.0 * inv_max, a, bma);   // MAIM_div_env.py:408-411
-                else OBS_PUT_SCALED(row, k0 + k, CHECKED, tabrow, tabrow_f, TL, TAB_INV, pipe[k], inv_max, a, bma);
+                else if (div && KF(multi)) OBS_PUT_SCALED(row, k0 + k, CHECKED, tabrow, tabrow_lp, TL, TAB_PIPE2, min(pipe[k], 2 * np.inv_max), 2.0 * inv_max, a, bma);   // MAIM_div_env.py:408-411
+                else OBS_PUT_SCALED(row, k0 + k, CHECKED, tabrow, tabrow_lp, TL, TAB_INV, pipe[k], inv_max, a, bma);
             }
         }
         k0 += KF(D);
@@ -281,17 +281,23 @@ __device__ __forceinline__ void write_obs_row(void* row, const StepArgs& A, cons
     if (KF(share_network)) OBS_PUT(row, k0, rescale((double)node_idx, (double)KF(m), a, bma));       // MAIM_div_env.py:434-435
 }
 
-// Flushes a warp's staged observation tile (`bytes` contiguous bytes, a multiple of 4) to global memory.
+// Flushes a warp's staged observation tile (`bytes` contiguous bytes, a multiple of 2) to global memory: one bulk copy where
+// the size and the global address are whole 16-byte units, else element stores (a bfloat16 tile of m = 5, O = 5 is 200 bytes
+// per 4 envs: its global offset is not 16-byte aligned).
 __device__ __forceinline__ void flush_obs_tile(void* gdst, const void* stile, uint32_t bytes, int lane) {
     const bool bulk_ok = ((bytes & 15u) == 0u) && ((reinterpret_cast<uintptr_t>(gdst) & 15u) == 0u);
     if (bulk_ok) fence_proxy_async_smem();      // every writer orders its stores before the async-proxy read
     __syncwarp();
     if (bulk_ok) {
         if (lane == 0) bulk_store_s2g(gdst, stile, bytes);
-    } else {
+    } else if (((bytes | (uint32_t)reinterpret_cast<uintptr_t>(gdst)) & 3u) == 0u) {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(stile);
         uint32_t* dst = reinterpret_cast<uint32_t*>(gdst);
         for (uint32_t k = lane; k < bytes / 4u; k += 32) dst[k] = src[k];
+    } else {
+        const uint16_t* src = reinterpret_cast<const uint16_t*>(stile);
+        uint16_t* dst = reinterpret_cast<uint16_t*>(gdst);
+        for (uint32_t k = lane; k < bytes / 2u; k += 32) dst[k] = src[k];
     }
 }
 
@@ -319,7 +325,7 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const __grid_constan
     const double om_d = (double)np.order_max;
     const double* __restrict__ tabrow = KHAS(tab) ? A.tab + (size_t)(stage_ok ? i : 0) * 4 * KF(TL) : nullptr;
 
-    const int es = KF(obs_f32) ? 4 : 8;                          // observation element size
+    const int es = obs_elem_bytes(KF(obs_type));                 // observation element size
     const int tile_bytes = (EPW * m * O * es + 15) & ~15;        // keep every warp's tile 16-byte aligned
     unsigned char* wtile = smem_obs + (size_t)warp * tile_bytes;
     bool tile_in_flight = false;
@@ -344,7 +350,7 @@ __global__ void __launch_bounds__(STEP_THREADS) step_kernel(const __grid_constan
 #pragma unroll
         for (int k = 0; k < MAXC; ++k) bt[k] = 0;
         if (ok) {
-            act = A.actions[cell];
+            act = load_action(A.actions, cell, KF(act_f32) != 0);
             inv = A.inv[cell];
             backlog = A.backlog[cell];
             order_u = A.order_u[cell];

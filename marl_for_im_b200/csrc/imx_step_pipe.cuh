@@ -53,7 +53,8 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     constexpr int CT = TMA_THREADS;                  // compute threads; the producer warp sits behind them
     const int tid = threadIdx.x;
     const int m = KF(m), O = KF(O), E = KT(E);
-    const int es = KF(obs_f32) ? 4 : 8;
+    const int es = obs_elem_bytes(KF(obs_type));
+    const int aes = KF(act_f32) ? 4 : 8;
     const int n_my = (PA.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // tiles blockIdx.x, + gridDim.x, ...
 
     pdl_launch_dependents();
@@ -65,10 +66,10 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     __syncthreads();                                 // the only CTA-wide barrier: the roles part ways here
 
     // ---- what every role that issues bulk loads needs (the producer, and lane 0 of each compute warp for the first ring fill) ----
-    const uint32_t b_cell4 = (uint32_t)E * m * 4u, b_cell8 = (uint32_t)E * m * 8u;
+    const uint32_t b_cell4 = (uint32_t)E * m * 4u, b_cell8 = (uint32_t)E * m * 8u, b_act = (uint32_t)E * m * aes;
     const uint32_t b_pipe = (uint32_t)E * KF(L) * 4u, b_hist = b_cell4 * (uint32_t)KF(P);
     const uint32_t b_bt = (uint32_t)E * KF(NB) * 4u, b_dem = (uint32_t)E * 4u;
-    uint32_t b_in = b_cell8 + (uint32_t)KF(R) * b_dem + 3u * b_cell4 + b_pipe;
+    uint32_t b_in = b_act + (uint32_t)KF(R) * b_dem + 3u * b_cell4 + b_pipe;
     if (KF(need_hd)) b_in += b_hist;
     if (KF(need_ho)) b_in += b_hist;
     if (KF(has_carry)) b_in += b_cell4;
@@ -97,7 +98,7 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     // the action tile and demand rows of tile k into L2 while the previous launch drains (see bulk_prefetch_l2)
     auto prefetch_inputs = [&](int k) {
 #if !defined(IMX_NO_ACT_PREFETCH)
-        bulk_prefetch_l2(A.actions + first_env(k) * m, b_cell8);
+        bulk_prefetch_l2(reinterpret_cast<const unsigned char*>(A.actions) + first_env(k) * m * aes, b_act);
         for (int r = 0; r < KF(R); ++r)              // (the demand trace was written at reset() and is long evicted)
             bulk_prefetch_l2(A.demand_T + ((int64_t)A.t * KF(R) + r) * A.N + first_env(k), b_dem);
 #endif
@@ -108,7 +109,7 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
         const int64_t n0 = first_env(k);
         uint64_t* bar = &full[s];
         mbar_expect_tx(bar, b_in);
-        PIPE_LOAD_STREAM(st + KT(off_act), A.actions + n0 * m, b_cell8, bar);
+        PIPE_LOAD_STREAM(st + KT(off_act), reinterpret_cast<const unsigned char*>(A.actions) + n0 * m * aes, b_act, bar);
         for (int r = 0; r < KF(R); ++r)
             PIPE_LOAD_STREAM(st + KT(off_dem) + (size_t)r * b_dem, A.demand_T + ((int64_t)A.t * KF(R) + r) * A.N + n0, b_dem, bar);
         PIPE_LOAD_KEEP(st + KT(off_inv), A.inv + n0 * m, b_cell4, bar);
@@ -175,7 +176,7 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     for (int k = 0; k < n_my; ++k) {
         const int s = k % S;
         unsigned char* st = smem + (size_t)s * KT(total);
-        const TileSmem T = {reinterpret_cast<const double*>(st + KT(off_act)), reinterpret_cast<const int32_t*>(st + KT(off_dem)),
+        const TileSmem T = {st + KT(off_act), reinterpret_cast<const int32_t*>(st + KT(off_dem)),
                             reinterpret_cast<int32_t*>(st + KT(off_inv)), reinterpret_cast<int32_t*>(st + KT(off_bl)),
                             reinterpret_cast<int32_t*>(st + KT(off_ou)), reinterpret_cast<int32_t*>(st + KT(off_pipe)),
                             reinterpret_cast<int32_t*>(st + KT(off_hd)), reinterpret_cast<int32_t*>(st + KT(off_ho)),

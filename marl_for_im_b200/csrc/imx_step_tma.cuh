@@ -2,7 +2,7 @@
 //
 // One CTA = one tile of E = 256 / M_PAD consecutive environments.  Because state and I/O are
 // structure-of-arrays with the env index slowest, every field of a tile is ONE contiguous byte
-// range in HBM:  actions E*m*8,  inv / backlog / order_u E*m*4 each,  pipe E*L*4,  hist E*m*P*4,
+// range in HBM:  actions E*m*8 (float32: E*m*4),  inv / backlog / order_u E*m*4 each,  pipe E*L*4,  hist E*m*P*4,
 // demand E*4 per retailer row,  obs E*m*O*8,  reward E*m*8.
 //   1. one elected thread arms an mbarrier with the tile's byte count and issues one
 //      cp.async.bulk (global -> shared, SASS UBLKCP) per field;
@@ -142,12 +142,15 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // Cure: every lane stores the SAME chunks in a ROTATED order — at store q lane l writes chunk (q + r) mod c with
 // r = (l mod 8) / (8 / g) — which makes the eight lanes of a quarter-warp cover eight different 16-byte bank groups.
 // The rotation is a barrel of selects on registers (static indices only).  Runtime-specialised build only (O is a literal).
-#if defined(IMX_JIT) && ((IMX_K_O * (IMX_K_obs_f32 ? 4 : 8)) % 32 == 0) && ((IMX_K_O * (IMX_K_obs_f32 ? 4 : 8)) <= 256)
+#ifdef IMX_JIT
+#define IMX_K_OBS_ES (IMX_K_obs_type == 2 ? 2 : IMX_K_obs_type == 1 ? 4 : 8)   // = obs_elem_bytes(IMX_K_obs_type), for #if
+#endif
+#if defined(IMX_JIT) && ((IMX_K_O * IMX_K_OBS_ES) % 32 == 0) && ((IMX_K_O * IMX_K_OBS_ES) <= 256)
 #define IMX_OBS_ROTATE 1          // the row is an even number (<= 16) of 16-byte chunks: gcd(c, 8) > 1
 #endif
 #ifdef IMX_OBS_ROTATE
 __host__ __device__ constexpr int obs_gcd8(int c) { return (c % 8 == 0) ? 8 : (c % 4 == 0) ? 4 : (c % 2 == 0) ? 2 : 1; }
-constexpr int OBS_ROW_BYTES = IMX_K_O * (IMX_K_obs_f32 ? 4 : 8);
+constexpr int OBS_ROW_BYTES = IMX_K_O * IMX_K_OBS_ES;
 constexpr int OBS_ROW_CHUNKS = OBS_ROW_BYTES / 16;
 constexpr int OBS_ROT_G = obs_gcd8(OBS_ROW_CHUNKS);
 
@@ -178,10 +181,11 @@ __device__ __forceinline__ void store_row_rotated(unsigned char* dst, const unsi
 
 // Shared-memory views of ONE tile for ONE period (all regions laid out like the global arrays: [E][m] etc.).
 struct TileSmem {
-    const double* act;          // [E][m] actions of this period (consumed first; afterwards scratch for the shared reward)
+    const void* act;            // [E][m] actions of this period, float64 or float32, then (float32 only) a [E][m] float64 scratch
+                                // for the shared reward (see tile_period; float64 actions are overwritten by it once consumed)
     const int32_t* dem;         // [R][E] customer demand of this period
     int32_t *inv, *bl, *ou, *pipe, *hd, *ho, *carry, *bt;   // state, updated in place
-    unsigned char* obs;         // [E][m][O] observation tile (float64 or float32)
+    unsigned char* obs;         // [E][m][O] observation tile (float64, float32 or bfloat16)
     double* rew;                // [E][m] / [E] reward tile
     double* prof;               // [E][m] profits of the period, or null (episode kernel with evaluation accumulators)
     double* ret;                // [E][m] / [E] episode returns, or null (episode kernel): reward added in place, period by period
@@ -236,13 +240,12 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
     const int lane = L.lane, i = L.i, tbase = L.tbase, e_loc = L.e_loc, cell = L.cell;
     const bool ok = L.ok, is_last = L.is_last;
     const int m = KF(m), O = KF(O), E = KT(E);
-    const int es = KF(obs_f32) ? 4 : 8;              // observation element size
+    const int es = obs_elem_bytes(KF(obs_type));     // observation element size
     const int delay_m1 = np.delay - 1;
     const double om_d = (double)np.order_max;
     const double* __restrict__ tabrow = L.tabrow;
     int32_t* my_pipe = S.pipe + e_loc * KF(L) + np.pipe_off;
-    const double* s_act = S.act;
-    (void)lane; (void)E; (void)O; (void)es; (void)s_act;
+    (void)lane; (void)E; (void)O; (void)es;
     // ---- read the tile ----------------------------------------------------------------------
     double act = 0.0;
     int inv = 0, backlog = 0, order_u = 0, carry = 0, cust = 0;
@@ -254,7 +257,7 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
 #pragma unroll
     for (int k = 0; k < MAXC; ++k) bt[k] = 0;
     if (ok) {
-        act = S.act[cell];
+        act = load_action(S.act, cell, KF(act_f32) != 0);
         inv = S.inv[cell];
         backlog = S.bl[cell];
         order_u = S.ou[cell];
@@ -354,10 +357,13 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
             reward_out = div_by_m(tile_seq_sum<M_PAD>(profit, m, tbase), m, A.inv_m, KM_POW2);
         } else {
             // multi-period kernels of wider networks (8-stage 0.90 -> 0.96 of peak) and the rewards-only replay (+7-12 %):
-            // shared reward: the env's m profits meet in ITS row of this period's ACTION tile — already consumed, same
-            // [E][m] float64 shape, refilled only after the CTA barrier below — one 8-byte store per lane, then 16-byte
-            // broadcast loads, instead of 2 m shuffles
-            double* scratch = const_cast<double*>(S.act);
+            // shared reward: the env's m profits meet in ITS row of a [E][m] float64 scratch in this period's ACTION region,
+            // refilled only after the CTA barrier below — one 8-byte store per lane, then 16-byte broadcast loads, instead of
+            // 2 m shuffles.  float64 actions: the scratch IS the action tile (slot `cell` holds only this lane's action, already
+            // read).  float32 actions: slot `cell` would cover the actions of cells 2 cell and 2 cell + 1, which other warps may
+            // not have read yet, so the scratch sits behind the E*m*4 bytes of actions (the region is E*m*12 bytes then)
+            double* scratch = reinterpret_cast<double*>(const_cast<unsigned char*>(static_cast<const unsigned char*>(S.act)) +
+                                                        (KF(act_f32) ? (size_t)E * m * 4 : (size_t)0));
             if (ok) scratch[cell] = profit;
             __syncwarp();
             const double* row = scratch + e_loc * m;
@@ -416,7 +422,14 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
             if (KHAS(obs)) {
                 // build the row in registers (typed like the output elements), then store its chunks in rotated order
                 unsigned long long w[OBS_ROW_BYTES / 8];
-                if (KF(obs_f32)) {
+                if (KF(obs_type) == OBS_BF16) {
+                    uint16_t rowh[IMX_K_O];
+                    write_obs_row<DMAX, PMAX>(rowh, A, np, i, tabrow, inv_new, backlog_new, order_u_new, pipe, hd, ho, DIV);
+#pragma unroll
+                    for (int k = 0; k < OBS_ROW_BYTES / 8; ++k)
+                        w[k] = (unsigned long long)rowh[4 * k] | ((unsigned long long)rowh[4 * k + 1] << 16) |
+                               ((unsigned long long)rowh[4 * k + 2] << 32) | ((unsigned long long)rowh[4 * k + 3] << 48);
+                } else if (KF(obs_type) == OBS_F32) {
                     float rowf[IMX_K_O];
                     write_obs_row<DMAX, PMAX>(rowf, A, np, i, tabrow, inv_new, backlog_new, order_u_new, pipe, hd, ho, DIV);
 #pragma unroll
@@ -453,6 +466,7 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
 // CC_inv_management.py:516-528: opponent actions clipped to [lo, hi]; zeros at sampling time).  Opponents in agent order.
 template <int BYTES> struct CcWord { typedef uint32_t type; };
 template <> struct CcWord<8> { typedef unsigned long long type; };
+template <> struct CcWord<2> { typedef uint16_t type; };
 template <typename ObsT, int MAXC>
 __device__ __forceinline__ void cc_build_row(const StepArgs& A, const TileSmem& S, unsigned char* cc_tile, const LaneCtx<MAXC>& L) {
     if (!L.ok) return;
@@ -460,7 +474,8 @@ __device__ __forceinline__ void cc_build_row(const StepArgs& A, const TileSmem& 
     const int W = (m - 1) * (1 + O) + O;
     const int e0 = L.e_loc * m;
     // a row is copied in units of its element type (4-byte words for float32 rows, which are only 4-byte aligned — W is odd
-    // for m = 2; 8-byte words for float64 rows: 17 STS.64 instead of 34 STS.32 per lane, conflict-free at a stride of 2 W words)
+    // for m = 2; 8-byte words for float64 rows: 17 STS.64 instead of 34 STS.32 per lane, conflict-free at a stride of 2 W words;
+    // 2-byte elements for bfloat16 rows, ObsT = uint16_t, the bit patterns)
     using WordT = typename CcWord<sizeof(ObsT)>::type;
     WordT* row = reinterpret_cast<WordT*>(cc_tile) + (size_t)L.cell * W;
     const WordT* ob = reinterpret_cast<const WordT*>(S.obs);
@@ -471,21 +486,22 @@ __device__ __forceinline__ void cc_build_row(const StepArgs& A, const TileSmem& 
 #pragma unroll
     for (int q = 0; q < m - 1; ++q) {
         const int j = q + (q >= L.i ? 1 : 0);
-        const ObsT v = A.cc_fill ? (ObsT)fmin(fmax(S.act[e0 + j], A.cc_lo), A.cc_hi) : (ObsT)0;
-        if constexpr (sizeof(ObsT) == 4) row[k++] = __float_as_uint((float)v);
-        else row[k++] = (unsigned long long)__double_as_longlong((double)v);
+        const double v = A.cc_fill ? fmin(fmax(load_action(S.act, e0 + j, KF(act_f32) != 0), A.cc_lo), A.cc_hi) : 0.0;
+        if constexpr (sizeof(ObsT) == 2) row[k++] = f32_to_bf16((float)v);
+        else if constexpr (sizeof(ObsT) == 4) row[k++] = __float_as_uint((float)v);
+        else row[k++] = (unsigned long long)__double_as_longlong(v);
     }
     // observation rows: 16-byte shared-memory loads where the rows are 16-byte multiples (one wavefront per quarter-warp instead
     // of the 8-way conflicts of scalar loads at a row stride of 32 or 64 bytes), element-wise stores into the critic row
     auto copy_row = [&](int cell_src) {
         const WordT* src = ob + (size_t)cell_src * O;
-        if (O % VEC == 0) {
+        if (sizeof(ObsT) > 2 && O % VEC == 0) {
 #pragma unroll
             for (int q = 0; q < O / VEC; ++q) {
                 if constexpr (sizeof(ObsT) == 4) {
                     const uint4 v = reinterpret_cast<const uint4*>(src)[q];
                     row[k] = v.x; row[k + 1] = v.y; row[k + 2] = v.z; row[k + 3] = v.w;
-                } else {
+                } else if constexpr (sizeof(ObsT) == 8) {
                     const ulonglong2 v = reinterpret_cast<const ulonglong2*>(src)[q];
                     row[k] = v.x; row[k + 1] = v.y;
                 }
@@ -505,7 +521,8 @@ __device__ __forceinline__ void cc_build(const StepArgs& A, const TileLayout& TL
                                          int nthreads) {
     (void)nthreads;
     __syncwarp();                                    // the env's m observation rows are complete
-    if (KF(obs_f32)) cc_build_row<float, MAXC>(A, S, tile_base + KT(off_cc), L);
+    if (KF(obs_type) == OBS_BF16) cc_build_row<uint16_t, MAXC>(A, S, tile_base + KT(off_cc), L);
+    else if (KF(obs_type) == OBS_F32) cc_build_row<float, MAXC>(A, S, tile_base + KT(off_cc), L);
     else cc_build_row<double, MAXC>(A, S, tile_base + KT(off_cc), L);
 }
 
@@ -529,7 +546,7 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
     constexpr unsigned long long P_BITS[M] = {IMX_L_p_bits}, C_BITS[M] = {IMX_L_c_bits}, H_BITS[M] = {IMX_L_h_bits}, BC_BITS[M] = {IMX_L_bc_bits},
                                  TG_BITS[M] = {IMX_L_target_bits};
     const int E = KT(E), O = KF(O);
-    const int es = KF(obs_f32) ? 4 : 8;
+    const int es = obs_elem_bytes(KF(obs_type));
     const int c0 = e * M;                            // first cell of this thread's env
     int inv[M], bl[M], ou[M], cr[M], pipe[M][DMAX], hd[M][PMAX], ho[M][PMAX], bt[M][MAXC];
     int order[M], demand[M], acq[M], ship[M], incoming[M];
@@ -547,7 +564,7 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
         }
 #pragma unroll
         for (int k = 0; k < MAXC; ++k) bt[j][k] = (DIV && NCHILD[j] > 1 && k < NCHILD[j]) ? S.bt[e * KF(NB) + BT_OFF[j] + k] : 0;
-        order[j] = decode_order(S.act[c0 + j], (double)ORDER_MAX[j], KF(std_actions) != 0, KF(multi) != 0, A.a, A.bma, A.inv_bma, KBMA_POW2);
+        order[j] = decode_order(load_action(S.act, c0 + j, KF(act_f32) != 0), (double)ORDER_MAX[j], KF(std_actions) != 0, KF(multi) != 0, A.a, A.bma, A.inv_bma, KBMA_POW2);
     }
     // ---- demand propagation, acquisition, shipment ------------------------------------------------------------------------
 #pragma unroll
@@ -686,8 +703,8 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
 #endif
 
 // Episode kernel with evaluation accumulators, after each period: thread e repeats eval_accumulate_kernel's float64 operations
-// in its order on the observation elements the step writes (obs[i][0] = inventory, obs[i][1] = backlog: rounded to float32 and
-// widened for float32 observations) and on the period's profits.
+// in its order on the observation elements the step writes (obs[i][0] = inventory, obs[i][1] = backlog: rounded to the
+// observation element type and widened back) and on the period's profits.
 __device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs& EA, unsigned char* smem, int e) {
     const int m = KF(m);
     const int cols = KF(multi) ? m : 1;
@@ -710,7 +727,8 @@ __device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLa
                 x0 = (double)inv[i];
                 x1 = (double)bl[i];
             }
-            if (KF(obs_f32)) { x0 = (double)(float)x0; x1 = (double)(float)x1; }
+            x0 = obs_stored(KF(obs_type), x0);
+            x1 = obs_stored(KF(obs_type), x1);
             if (EA.rescaled) {
                 x0 = rev_scale_dev(x0, inv_max, A.a, A.bma);         // the loops use inv_max for BOTH fields
                 x1 = rev_scale_dev(x1, inv_max, A.a, A.bma);
@@ -759,20 +777,21 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     int32_t* s_ho = reinterpret_cast<int32_t*>(smem + KT(off_ho));
     int32_t* s_carry = reinterpret_cast<int32_t*>(smem + KT(off_carry));
     int32_t* s_bt = reinterpret_cast<int32_t*>(smem + KT(off_bt));
-    const int es = KF(obs_f32) ? 4 : 8;              // observation element size
+    const int es = obs_elem_bytes(KF(obs_type));     // observation element size
+    const int aes = KF(act_f32) ? 4 : 8;             // action element size
 
-    const uint32_t b_cell4 = (uint32_t)E * m * 4u, b_cell8 = (uint32_t)E * m * 8u;
+    const uint32_t b_cell4 = (uint32_t)E * m * 4u, b_cell8 = (uint32_t)E * m * 8u, b_act = (uint32_t)E * m * aes;
     const uint32_t b_pipe = (uint32_t)E * KF(L) * 4u, b_hist = b_cell4 * (uint32_t)KF(P);
     const uint32_t b_bt = (uint32_t)E * KF(NB) * 4u, b_dem = (uint32_t)E * 4u;
     // per-period inputs: actions + demand rows (the episode kernel's demand is resident for the whole launch)
-    const uint32_t b_in = b_cell8 + (EPISODE ? 0u : (uint32_t)KF(R) * b_dem);
+    const uint32_t b_in = b_act + (EPISODE ? 0u : (uint32_t)KF(R) * b_dem);
     const uint32_t b_edem = (uint32_t)E * KF(R) * KF(T) * 4u;     // the tile's [E][R][T] trace (episode kernel)
 
     // per-period inputs of period j (actions block j, demand rows of period t0 + j) into input buffer j & 1
     auto load_inputs = [&](int j) {
-        double* sa = reinterpret_cast<double*>(smem + ((j & 1) ? KT(off_act2) : KT(off_act)));
+        unsigned char* sa = smem + ((j & 1) ? KT(off_act2) : KT(off_act));
         int32_t* sd = reinterpret_cast<int32_t*>(smem + ((j & 1) ? KT(off_dem2) : KT(off_dem)));
-        bulk_load_g2s(sa, A.actions + (int64_t)j * A.act_stride + n0 * m, b_cell8, &bar[j & 1]);
+        bulk_load_g2s(sa, reinterpret_cast<const unsigned char*>(A.actions) + ((int64_t)j * A.act_stride + n0 * m) * aes, b_act, &bar[j & 1]);
         if (!EPISODE)
             for (int r = 0; r < KF(R); ++r)
                 bulk_load_g2s(sd + r * E, A.demand_T + ((int64_t)(A.t + j) * KF(R) + r) * A.N + n0, b_dem, &bar[j & 1]);
@@ -787,7 +806,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     __syncthreads();
     if (tid == 0) {
 #if defined(IMX_JIT) && !defined(IMX_NO_ACT_PREFETCH)
-        bulk_prefetch_l2(A.actions + n0 * m, b_cell8);
+        bulk_prefetch_l2(reinterpret_cast<const unsigned char*>(A.actions) + n0 * m * aes, b_act);
         if (!EPISODE)
             for (int r = 0; r < KF(R); ++r) bulk_prefetch_l2(A.demand_T + ((int64_t)A.t * KF(R) + r) * A.N + n0, b_dem);
 #endif
@@ -848,7 +867,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     for (int j = 0; j < K; ++j) {
     const int t = A.t + j;                           // period being simulated
     const int b = j & 1;
-    const double* s_act = reinterpret_cast<const double*>(smem + (b ? KT(off_act2) : KT(off_act)));
+    const void* s_act = smem + (b ? KT(off_act2) : KT(off_act));
     const int32_t* s_dem = reinterpret_cast<const int32_t*>(smem + (b ? KT(off_dem2) : KT(off_dem)));
     unsigned char* s_obs = smem + KT(off_obs);       // ONE output buffer: period j - 1's bulk stores have long finished
     double* s_rew = reinterpret_cast<double*>(smem + KT(off_rew));   // reading it when period j's dynamics are done (waited below)

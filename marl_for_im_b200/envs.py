@@ -115,8 +115,14 @@ class _ImxEnvBase:
         self.reuse_buffers = bool(take("reuse_buffers", False))
         self.demand_mode = take("demand_mode", "philox" if self.batched else "host")
         obs_dtype = take("obs_dtype", "float64")             # "float32": the cast RLlib applies anyway, half the bytes
-        self.obs_dtype = {"float64": torch.float64, "float32": torch.float32, torch.float64: torch.float64,
-                          torch.float32: torch.float32}[obs_dtype]
+        self.obs_dtype = {"float64": torch.float64, "float32": torch.float32, "bfloat16": torch.bfloat16, torch.float64: torch.float64,
+                          torch.float32: torch.float32, torch.bfloat16: torch.bfloat16}[obs_dtype]
+        # float32 actions: what a reduced-precision policy's output layer emits; results equal float64 actions of the same values
+        self.action_dtype = {"float64": torch.float64, "float32": torch.float32, torch.float64: torch.float64,
+                             torch.float32: torch.float32}[take("action_dtype", "float64")]
+        if not self.batched and (self.obs_dtype == torch.bfloat16 or self.action_dtype == torch.float32):
+            raise ValueError("obs_dtype='bfloat16' and action_dtype='float32' are batched-mode options (construct the env with "
+                             "num_envs=N): the drop-in env mirrors the reference's float64 numpy surface")
         self.mu = self.config.get("mu", 5)
         if self.demand_dist == "poisson":                    # callers pre-draw test sets with env.dist.rvs (inv_management.py:200)
             from scipy.stats import poisson
@@ -165,6 +171,8 @@ class _ImxEnvBase:
         c.uniform_low, c.uniform_high = int(lower_upper[0]), int(lower_upper[1])
         c.device = self.device.index if self.device.index is not None else (torch.cuda.current_device() if torch.cuda.is_available() else 0)
         c.obs_f32 = int(self.obs_dtype == torch.float32)
+        c.io_flags = (_lib.IO_OBS_BF16 if self.obs_dtype == torch.bfloat16 else 0) | \
+                     (_lib.IO_ACTIONS_F32 if self.action_dtype == torch.float32 else 0)
         c.a, c.b = float(self.a), float(self.b)
         c.mu = float(self.config.get("mu", 5))
         c.noisy_delay_threshold = float(self.noisy_delay_threshold)
@@ -434,6 +442,8 @@ class _ImxEnvBase:
         return torch.empty(shape, dtype=torch.float64, device=self.device)
 
     def _actions_to_device(self, action):
+        """[N, m] contiguous CUDA tensor in the handle's action dtype.  With action_dtype='float32' a float64 input is rounded
+        to float32 first (round to nearest even), so the env decodes the float32 value, not the float64 one."""
         N, m = self.num_envs, self.num_nodes
         if isinstance(action, dict):
             vals = [action[name] for name in self._agent_names]
@@ -444,17 +454,17 @@ class _ImxEnvBase:
         else:
             act = action
         if isinstance(act, torch.Tensor):
-            act = act.to(device=self.device, dtype=torch.float64).reshape(N, m)
+            act = act.to(device=self.device, dtype=self.action_dtype).reshape(N, m)
             return act if act.is_contiguous() else act.contiguous()
         arr = np.ascontiguousarray(np.asarray(act, dtype=np.float64).reshape(N, m))   # np.squeeze semantics of IM_env.py:299
-        return torch.as_tensor(arr, device=self.device)
+        return torch.as_tensor(arr, device=self.device).to(self.action_dtype)
 
     def step_packed(self, action):
-        """Lean batched step for device-side loops (an RL loop with a GPU policy): ``action`` a contiguous float64
-        ``[N, m]`` CUDA tensor (anything else is converted like ``step`` does), returns the packed tensors
+        """Lean batched step for device-side loops (an RL loop with a GPU policy): ``action`` a contiguous ``[N, m]`` CUDA
+        tensor of the env's ``action_dtype`` (anything else is converted like ``step`` does), returns the packed tensors
         ``(obs [N, m, O], reward [N, m] / [N], done)`` — no per-agent dicts, no diagnostics.  With
         ``reuse_buffers=True`` the same two output tensors are overwritten every call and nothing is allocated."""
-        if isinstance(action, torch.Tensor) and action.dtype == torch.float64 and action.is_cuda and action.is_contiguous() \
+        if isinstance(action, torch.Tensor) and action.dtype == self.action_dtype and action.is_cuda and action.is_contiguous() \
                 and action.numel() == self.num_envs * self.num_nodes:
             act = action
         else:
@@ -616,7 +626,7 @@ class _ImxEnvBase:
             raise _lib.ImxError("step_many is a batched-mode call (construct the env with num_envs=N)")
         N, m, O = self.num_envs, self.num_nodes, self.obs_len
         act = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions, dtype=np.float64))
-        act = act.to(device=self.device, dtype=torch.float64).reshape(-1, N, m).contiguous()
+        act = act.to(device=self.device, dtype=self.action_dtype).reshape(-1, N, m).contiguous()
         K = act.shape[0]
         if want_obs and obs_out is None:
             obs_out = torch.empty((K, N, m, O), dtype=self.obs_dtype, device=self.device)
@@ -657,7 +667,7 @@ class _ImxEnvBase:
             raise _lib.ImxError("replay_episode is a batched-mode call (construct the env with num_envs=N)")
         N, m, O, T = self.num_envs, self.num_nodes, self.obs_len, self.num_periods
         act = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions, dtype=np.float64))
-        act = act.to(device=self.device, dtype=torch.float64)
+        act = act.to(device=self.device, dtype=self.action_dtype)
         if act.numel() != T * N * m:
             raise ValueError(f"actions must hold a whole episode: [T={T}, N={N}, m={m}]")
         act = act.reshape(T, N, m).contiguous()

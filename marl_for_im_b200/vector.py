@@ -21,6 +21,12 @@ import numpy as np
 import torch
 
 
+def _host(t):
+    """numpy copy of a device tensor; bfloat16 (which numpy lacks) as its exact float32 widening."""
+    t = t.cpu()
+    return (t.float() if t.dtype == torch.bfloat16 else t).numpy()
+
+
 class _LockStepBatch:
     def __init__(self, env):
         if not env.batched:
@@ -36,7 +42,7 @@ class _LockStepBatch:
         self.env.reset()
         obs = self.env.last_obs           # the packed [N, m, O] tensor the per-agent views point into
         self._obs_dev = obs
-        self._obs_host = obs.cpu().numpy()
+        self._obs_host = _host(obs)
         self._reset_pending = False
         return obs
 
@@ -68,7 +74,7 @@ class BatchedVectorEnv(_LockStepBatch):
 
     def vector_step(self, actions):
         obs, rew, done = self.step_tensors(torch.as_tensor(np.asarray(actions, dtype=np.float64), device=self.env.device))
-        o, r = obs.cpu().numpy(), rew.cpu().numpy()
+        o, r = _host(obs), rew.cpu().numpy()
         N = self.num_envs
         return [o[n] for n in range(N)], [np.float64(r[n]) for n in range(N)], [done] * N, [{} for _ in range(N)]
 
@@ -104,7 +110,7 @@ class BatchedMultiAgentEnv(_LockStepBatch):
             return {}, {}, {}, {}, {}
         obs_d, rew_d, done = self._pending
         self._pending = None
-        o = obs_d.cpu().numpy()
+        o = _host(obs_d)
         r = rew_d.cpu().numpy() if rew_d is not None else None
         obs, rewards, dones, infos = {}, {}, {}, {}
         for n in range(self.num_envs):

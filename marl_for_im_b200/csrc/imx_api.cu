@@ -80,6 +80,12 @@ extern "C" int64_t imx_launch_count(void) { return g_launches.load(); }
 // --------------------------------------------------------------------------------------
 typedef void (*reset_fn_t)(const StepArgs, const ResetArgs, int);
 
+// The runtime-specialised modules a handle may load, numbered as imx_jit_compile_check's `variant`: the step kernels (step,
+// step_many, rollout, pipelined); the same without the observation output (step / step_many with obs = NULL: scoring a stored
+// plan needs rewards only — the observation build and 60 % of the bytes fold away); the step with the centralised-critic rows
+// (imx_step_cc); the one-launch episode kernel (imx_replay_episode) with and without observations.
+enum JitVariant { JIT_STEP, JIT_NOOBS, JIT_CC, JIT_EPISODE, JIT_EPISODE_NOOBS, JIT_VARIANTS };
+
 struct imx_env {
     imx_config cfg;
     bool div, multi;
@@ -121,14 +127,13 @@ struct imx_env {
     tma_fn_t tma_fn = nullptr;
     tma_fn_t tma_many_fn = nullptr;      // the same kernel instantiated with the multi-period loop (imx_step_many)
     TileLayout tile = {};                // ahead-of-time kernels: tile width = m rounded up to a power of two
-    TileLayout tile_jit = {};            // runtime-specialised kernels: tile width = m (dense lane packing)
+    TileLayout tile_jit = {};            // runtime-specialised kernels: the same width, or one env per thread (step_et)
     int step_path = 0;                   // 0 auto, 1 direct only, 2 TMA wherever legal (IMX_STEP_PATH)
     int host_zero_copy = 1;              // imx_step_host addresses pinned host buffers directly (IMX_HOST_ZERO_COPY=0: staged copies)
-    int step_dense = 0;                  // experimental: m-wide tiles in the specialised step kernel (IMX_STEP_DENSE=1)
     int tma_threads = 256;               // CTA size of the TMA kernel (IMX_TMA_THREADS: 64, 128 or 256)
     int use_pdl = 1;                     // chain step launches with programmatic dependent launch (IMX_PDL=0 disables)
     int fuse_periods = 1;                // imx_step_many advances all its periods in one launch (IMX_FUSE_PERIODS=0: K plain launches)
-    int l2_hints = 0;                    // L2 eviction priorities on the pipelined kernel's bulk copies (IMX_L2_HINTS; default: see select_kernels)
+    int l2_hints = 0;                    // L2 eviction priorities on the pipelined kernel's bulk copies (IMX_L2_HINTS; default: see decide_l2_hints)
     int step_et = 0;                     // the specialised STEP kernels use the env-per-thread period (IMX_STEP_ET; default: divergent networks, m <= 8)
     int rollout_et = 0;                  // the specialised ROLLOUT kernel is the env-per-thread one (imx_rollout_et.cuh; IMX_ROLLOUT_ET, default m <= 8)
     int jit_threads = 128;               // CTA size (compute threads) of the specialised TMA kernels: tma_threads, or the env-per-thread group size
@@ -137,17 +142,10 @@ struct imx_env {
     int pipe_ctas = 0;                   // resident CTAs per SM of the pipelined kernel (IMX_PIPE_CTAS; 0 = derived)
     int sm_count = 148;
     int jit_policy = 0;                  // 0 auto (large batches), 1 always, -1 never (IMX_JIT)
-    int jit_state = 0;                   // 0 not tried, 1 specialised kernels loaded, -1 unavailable
-    const imxjit::Kernels* jit = nullptr;
-    const imxjit::Kernels* jit_noobs = nullptr;   // specialised without the observation output
-    int jit_noobs_state = 0;
-    const imxjit::Kernels* jit_cc = nullptr;      // specialised with the centralised-critic rows emitted by the step (imx_step_cc)
-    int jit_cc_state = 0;
+    const imxjit::Kernels* jit[JIT_VARIANTS] = {};   // the loaded module of each JitVariant ...
+    int jit_state[JIT_VARIANTS] = {};    // ... and its state: 0 not tried, 1 loaded, -1 unavailable
     TileLayout tile_cc = {};             // tile_jit + the [E][m][W] critic-row region
     void* d_obs_scratch = nullptr;       // [N][m][O] observations of the unfused imx_step_cc / imx_replay_episode when the caller passes none
-    const imxjit::Kernels* jit_ep = nullptr;        // the one-launch episode kernel (imx_replay_episode) with observations ...
-    const imxjit::Kernels* jit_ep_noobs = nullptr;  // ... and without
-    int jit_ep_state = 0, jit_ep_noobs_state = 0;
     double* d_ep_rewards = nullptr;      // [T][N](m) rewards of the unfused imx_replay_episode when the caller passes none
     double* d_ep_profit = nullptr;       // [N][m] one period's profits (unfused imx_replay_episode with evaluation accumulators)
     double* d_ep_ret = nullptr;          // [N](m) returns of imx_replay_episode when only the statistics are wanted
@@ -178,7 +176,12 @@ IMX_DECL_PICK(2, 0) IMX_DECL_PICK(4, 0) IMX_DECL_PICK(8, 0) IMX_DECL_PICK(16, 0)
 IMX_DECL_PICK(4, 1) IMX_DECL_PICK(8, 1) IMX_DECL_PICK(16, 1) IMX_DECL_PICK(32, 1)
 #undef IMX_DECL_PICK
 
-static int m_pad_of(const imx_env* e);
+static int m_pad_of(const imx_env* e) {
+    const int m = e->m;
+    if (e->div) return m <= 4 ? 4 : m <= 8 ? 8 : m <= 16 ? 16 : 32;
+    return m <= 2 ? 2 : m <= 4 ? 4 : m <= 8 ? 8 : m <= 16 ? 16 : 32;
+}
+
 static void pick_kernels(imx_env* e, int m_pad, bool div) {
     const bool small = (e->D <= 4 && e->P <= 1);
     const bool few = e->maxc <= 2;
@@ -213,8 +216,6 @@ static cudaError_t raise_dyn_smem_limit(const void* fn, size_t bytes) {
     return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
-static int m_pad_of(const imx_env* e);
-
 // CTA size of the TMA kernel.  128-thread CTAs de-synchronise the load / compute / store phases of neighbouring tiles and
 // measured faster on every shipped config (profiles/r1_other_configs_1gpu.jsonl) except the 4-wide chain at
 // multi-million-env batches, where the 256-thread tile is 2.5% ahead; 512-thread CTAs lose 25%
@@ -228,12 +229,6 @@ static int choose_tma_threads(const imx_env* e) {
     const int dflt = small4 ? 64 : (big4 || (m_pad_of(e) <= 4 && e->N >= ((int64_t)1 << 20))) ? 256 : 128;
     const int v = tt ? atoi(tt) : dflt;
     return ((v == 64 || v == 128 || v == 256 || v == 512) && v >= 2 * m_pad_of(e)) ? v : 256;
-}
-
-static int m_pad_of(const imx_env* e) {
-    const int m = e->m;
-    if (e->div) return m <= 4 ? 4 : m <= 8 ? 8 : m <= 16 ? 16 : 32;
-    return m <= 2 ? 2 : m <= 4 ? 4 : m <= 8 ? 8 : m <= 16 ? 16 : 32;
 }
 
 // shared-memory tile layout of the TMA kernel (regions 128-byte aligned); pure host arithmetic
@@ -268,7 +263,87 @@ static void compute_tile(const imx_env* e, TileLayout& L, int tile_width, bool w
     L.total2 = off;
 }
 
-// -D options and template instantiations of the runtime-specialised build (imx_jit.cuh)
+// L2 eviction priorities (observation stream evict_first, state + rewards evict_last): they pay exactly where a launch
+// streams more than about half of L2 while the state itself would still fit — the write-once stream then no longer
+// pushes the state out between two periods (config 2 at 262 144 envs 20.7 -> 16.6 us = 1.15 of the HBM copy peak, div2
+// 33.4 -> 27.1 us, 8-stage 49.2 -> 43.0 us); below that everything is L2-resident anyway (-1 %), above it the state does
+// not fit and the priorities only disturb the replacement (-2 .. -4 %).  profiles/r2_l2_hints_ab.txt
+// l2_bytes <= 0: the B200's 126 MB (imx_jit_compile_check runs without a device)
+static int decide_l2_hints(const imx_env* e, int l2_bytes) {
+    if (l2_bytes <= 0) l2_bytes = 126 << 20;
+    const int64_t per_env = bytes_per_env(e);
+    const int64_t state_bytes = 4 * (int64_t)e->S * e->N;
+    const char* lh = getenv("IMX_L2_HINTS");
+    if (lh && !strcmp(lh, "1")) return 1;
+    if (lh && !strcmp(lh, "2")) return 2;                  // outputs only (measurement switch)
+    if (lh && !strcmp(lh, "0")) return 0;
+    // below the window: outputs only (2) — the step itself is unchanged (everything is L2-resident), but the step rewards are
+    // still in L2 when imx_episode_stats reads them back after 30 periods of observation traffic (config 2 episode 205.2 -> 202.1 us,
+    // 32 768 envs 143.2 -> 140.3 us; profiles/r2_l2_hints_small_ab.txt)
+    if (per_env * e->N <= (int64_t)l2_bytes / 2) return 2;
+    return state_bytes <= (int64_t)l2_bytes * 5 / 8 ? 1 : 0;
+}
+
+// The handle's kernel plan: every choice that needs no device beyond its SM count and L2 size, and every tuning switch
+// (IMX_*).  Pure host arithmetic after derive(): select_kernels() calls it with the device's values, and
+// imx_jit_compile_check() with the B200's, so that the check builds the specialisations a handle loads.
+static void plan_handle(imx_env* e, int sm_count, int l2_bytes) {
+    e->sm_count = sm_count;
+    e->tma_threads = choose_tma_threads(e);
+    // env-per-thread rollout (imx_rollout_et.cuh): networks up to 8 nodes, lead times up to 4 (registers); IMX_ROLLOUT_ET=0 disables
+    const char* re = getenv("IMX_ROLLOUT_ET");
+    e->rollout_et = (re && !strcmp(re, "0")) ? 0 : (e->m <= 8 && e->D <= 4);
+    // env-per-thread STEP kernels: divergent networks up to 8 nodes (their lane-mapped kernels are issue-bound); IMX_STEP_ET=0/1
+    const char* se = getenv("IMX_STEP_ET");
+    const bool et_ok = e->m <= 8 && e->D <= 4 && e->P <= 2;
+    // default: divergent networks whose node count is not a power of two (the lane mapping pads them: div2 runs 19 of 32 lanes);
+    // div2 262 144 envs 34.9 -> 33.6 us, 1 Mi envs 129 -> 115 us; no gain on the 4-node div1 (profiles/r2_step_et_sweep.txt)
+    const bool non_pow2 = (e->m & (e->m - 1)) != 0;
+    e->step_et = (se && !strcmp(se, "0")) ? 0 : (se && !strcmp(se, "1")) ? et_ok : (et_ok && e->div && non_pow2);
+    const char* st = getenv("IMX_STEP_ET_THREADS");
+    const int et_threads = (st && (atoi(st) == 32 || atoi(st) == 64 || atoi(st) == 128)) ? atoi(st) : 32;
+    e->jit_threads = e->step_et ? et_threads : e->tma_threads;
+    // the specialised STEP kernel keeps the power-of-two tile: a dense m-wide tile makes the per-field byte
+    // ranges (e.g. 40 envs x 6 nodes x 4 B = 960 B) straddle 128-byte lines, measured slower at 262144 envs;
+    // the issue-bound ROLLOUT kernel is specialised with tile width = m (dense lane packing, +21% on div2)
+    compute_tile(e, e->tile, m_pad_of(e));
+    compute_tile(e, e->tile_jit, m_pad_of(e), false, e->step_et ? e->jit_threads : 0);
+    compute_tile(e, e->tile_cc, m_pad_of(e), true);
+    const char* pth = getenv("IMX_STEP_PATH");
+    e->step_path = (pth && !strcmp(pth, "direct")) ? 1 : (pth && !strcmp(pth, "tma")) ? 2 : 0;
+    const char* zc = getenv("IMX_HOST_ZERO_COPY");
+    e->host_zero_copy = (zc && !strcmp(zc, "0")) ? 0 : 1;
+    const char* pd = getenv("IMX_PDL");
+    e->use_pdl = (pd && !strcmp(pd, "0")) ? 0 : 1;
+    const char* fu = getenv("IMX_FUSE_PERIODS");
+    e->fuse_periods = (fu && !strcmp(fu, "0")) ? 0 : 1;
+    const char* jp = getenv("IMX_JIT");
+    e->jit_policy = (jp && !strcmp(jp, "1")) ? 1 : (jp && !strcmp(jp, "0")) ? -1 : 0;
+    const char* pm = getenv("IMX_PIPE");
+    e->pipe_mode = (pm && !strcmp(pm, "1")) ? 1 : (pm && !strcmp(pm, "0")) ? -1 : 0;
+    const char* ps = getenv("IMX_PIPE_STAGES");
+    e->pipe_stages = ps ? atoi(ps) : 0;                    // 0: the measured default of pipe_stages_for()
+    if (e->pipe_stages < 2 || e->pipe_stages > 8) e->pipe_stages = 0;
+    const char* pc = getenv("IMX_PIPE_CTAS");
+    e->pipe_ctas = pc ? atoi(pc) : 0;
+    e->l2_hints = decide_l2_hints(e, l2_bytes);
+}
+
+// Shared-memory layout of the episode kernel: tile_jit's multi-period layout, then the episode regions of EpisodeArgs that the
+// call needs (the returns and the accumulators adjacent: the kernel zeroes [off_ret, off_prof) in one loop) — a launch reserves
+// no bytes it does not use, since resident CTAs per SM bound this latency-bound loop.  Returns the total bytes.
+static int64_t episode_layout(const imx_env* e, EpisodeArgs& EA, bool ret = true, bool eval = true) {
+    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1;
+    int64_t off = e->tile_jit.total2;
+    auto take = [&](int64_t bytes) { const int64_t o = off; off += (bytes + 127) & ~(int64_t)127; return (int32_t)(o < (1 << 30) ? o : 0); };
+    EA.off_edem = take(E * e->R * e->T * 4);
+    EA.off_ret = take(ret ? E * cols * 8 : 0);
+    EA.off_eval = take(eval ? E * (EVAL_FIXED + e->m) * 8 : 0);
+    EA.off_prof = take(eval ? E * e->m * 8 : 0);
+    EA.total = (int32_t)(off < (1 << 30) ? off : 0);
+    return off;
+}
+
 // Ring depth of the pipelined kernel for a given tile layout.  Measured shapes (profiles/r2_pipe_sweep.txt, r2_step_et_sweep.txt):
 // four stages for the lane-mapped tiles, two for the env-per-thread tiles (their 32-env tiles are 2-3 x larger: a deeper ring
 // costs resident CTAs); the critic-row variant shortens its ring until four CTAs fit on an SM.
@@ -279,8 +354,11 @@ static int pipe_stages_for(const imx_env* e, const TileLayout& L) {
     return s;
 }
 
-// episode != 0: the module holds the one-launch episode kernel only (imx_replay_episode)
-static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1, int has_cc = 0, int episode = 0) {
+// -D options, template instantiations and dynamic shared memory of one JitVariant's module (imx_jit.cuh).  The episode
+// variants hold the one-launch episode kernel only; the critic rows ride on the single-period kernels only.
+static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[imxjit::N_KERNELS]) {
+    const int has_obs = (variant != JIT_NOOBS && variant != JIT_EPISODE_NOOBS) ? 1 : 0, has_cc = variant == JIT_CC ? 1 : 0;
+    const int TL = e->TL;
     std::vector<std::string>& defs = sp.defines;
     const imx_config& c = e->cfg;
     const bool always_std = (c.kind == IMX_KIND_MAIM_DIV);
@@ -340,7 +418,7 @@ static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1
     defs.push_back("IMX_HOST_SIZEOF_TILELAYOUT=" + std::to_string(sizeof(TileLayout)));
     defs.push_back("IMX_HOST_SIZEOF_ROLLOUTARGS=" + std::to_string(sizeof(RolloutArgs)));
     defs.push_back("IMX_HOST_SIZEOF_EPISODEARGS=" + std::to_string(sizeof(EpisodeArgs)));
-    const int mp = e->step_dense ? e->m : m_pad_of(e);     // step kernel: power-of-two tile width (see select_kernels)
+    const int mp = m_pad_of(e);                            // step kernel: power-of-two tile width (see plan_handle)
     const int pmax = (e->need_hd || e->need_ho) ? e->P : 1;
     const int maxc = e->maxc > 1 ? e->maxc : 1;
     const std::string dv = e->div ? "true" : "false";
@@ -407,104 +485,51 @@ static void jit_spec(const imx_env* e, int TL, imxjit::Spec& sp, int has_obs = 1
         sp.name[2] = "imx::rollout_kernel<" + std::to_string(e->m) + ", " + std::to_string(e->D) + ", " + std::to_string(e->div ? maxc : 1) +
                      ", " + dv + ">";
     sp.name[3] = "";
-    if (has_cc) { sp.name[1] = ""; sp.name[2] = ""; }      // the critic rows ride on the single-period kernels only
-    if (e->pipe_mode >= 0 && (int64_t)pipe_stages_for(e, L) * L.total <= 200 * 1024) {
+    if (has_cc) { sp.name[1] = ""; sp.name[2] = ""; }
+    const int64_t pipe_smem = (int64_t)pipe_stages_for(e, L) * L.total;
+    if (e->pipe_mode >= 0 && pipe_smem <= 200 * 1024) {
         defs.push_back("IMX_PIPE_STAGES=" + std::to_string(pipe_stages_for(e, L)));
         const char* pr = getenv("IMX_PIPE_MAXNREG");
         if (pr && atoi(pr) > 0) defs.push_back("IMX_PIPE_MAXNREG=" + std::to_string(atoi(pr)));
         sp.name[3] = "imx::step_kernel_pipe" + targs;
     }
     sp.name[4] = "";
-    if (episode) {
+    if (variant >= JIT_EPISODE) {
         for (int k = 0; k < 4; ++k) sp.name[k] = "";
         sp.name[4] = "imx::step_kernel_tma_episode" + targs;
     }
-}
-
-static void jit_smem(const imx_env* e, int smem[imxjit::N_KERNELS]) {
-    smem[0] = e->tile_jit.total;
-    smem[1] = e->tile_jit.total2 <= 200 * 1024 ? e->tile_jit.total2 : e->tile_jit.total;
-    smem[2] = 0;
-    smem[3] = pipe_stages_for(e, e->tile_jit) * e->tile_jit.total;
-    smem[4] = 0;
-}
-
-// Loads the specialised kernels for this handle (large batches, or IMX_JIT=1).  Called from imx_create() /
-// imx_prepare(); a later call only happens for handles whose policy changed, and never under stream capture.
-static void ensure_jit(imx_env* e) {
-    if (e->jit_state != 0) return;
-    e->jit_state = -1;
-    if (e->jit_policy < 0 || !e->tma_fn) return;
-    if (e->jit_policy == 0 && e->N < 1024) return;        // below ~1k envs a step is launch latency either way; the compile (1-2 s) is not worth it
-    if (e->tile_jit.total > 200 * 1024) return;
-    imxjit::Spec sp;
-    jit_spec(e, e->TL, sp);
-    int smem[imxjit::N_KERNELS];
-    jit_smem(e, smem);
-    e->jit = imxjit::get(sp, smem, e->cfg.device);
-    if (e->jit) e->jit_state = 1;
-}
-
-// The same kernels specialised WITHOUT an observation output (step / step_many with obs = NULL: scoring a stored plan
-// needs rewards only — the observation build and 60 % of the bytes fold away).  Compiled by imx_prepare(IMX_PREPARE_NOOBS)
-// or on first use outside stream capture.
-static void ensure_jit_noobs(imx_env* e) {
-    if (e->jit_noobs_state != 0) return;
-    e->jit_noobs_state = -1;
-    ensure_jit(e);
-    if (e->jit_state != 1) return;
-    imxjit::Spec sp;
-    jit_spec(e, e->TL, sp, 0);
-    int smem[imxjit::N_KERNELS];
-    jit_smem(e, smem);
-    e->jit_noobs = imxjit::get(sp, smem, e->cfg.device);
-    if (e->jit_noobs) e->jit_noobs_state = 1;
-}
-
-// ... and WITH the centralised-critic rows (imx_step_cc).  Compiled by imx_prepare(IMX_PREPARE_CC) or on first use outside capture.
-static void ensure_jit_cc(imx_env* e) {
-    if (e->jit_cc_state != 0) return;
-    e->jit_cc_state = -1;
-    ensure_jit(e);
-    if (e->jit_state != 1 || !e->multi || e->tile_cc.total > 200 * 1024) return;
-    imxjit::Spec sp;
-    jit_spec(e, e->TL, sp, 1, 1);
-    int smem[imxjit::N_KERNELS] = {e->tile_cc.total, 0, 0, pipe_stages_for(e, e->tile_cc) * e->tile_cc.total};
-    if (smem[3] > 200 * 1024) smem[3] = 0;
-    e->jit_cc = imxjit::get(sp, smem, e->cfg.device);
-    if (e->jit_cc) e->jit_cc_state = 1;
-}
-
-// Shared-memory layout of the episode kernel: tile_jit's multi-period layout, then the episode regions of EpisodeArgs that the
-// call needs (the returns and the accumulators adjacent: the kernel zeroes [off_ret, off_prof) in one loop) — a launch reserves
-// no bytes it does not use, since resident CTAs per SM bound this latency-bound loop.  Returns the total bytes.
-static int64_t episode_layout(const imx_env* e, EpisodeArgs& EA, bool ret = true, bool eval = true) {
-    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1;
-    int64_t off = e->tile_jit.total2;
-    auto take = [&](int64_t bytes) { const int64_t o = off; off += (bytes + 127) & ~(int64_t)127; return (int32_t)(o < (1 << 30) ? o : 0); };
-    EA.off_edem = take(E * e->R * e->T * 4);
-    EA.off_ret = take(ret ? E * cols * 8 : 0);
-    EA.off_eval = take(eval ? E * (EVAL_FIXED + e->m) * 8 : 0);
-    EA.off_prof = take(eval ? E * e->m * 8 : 0);
-    EA.total = (int32_t)(off < (1 << 30) ? off : 0);
-    return off;
-}
-
-// The episode kernel, with (obs) or without observations.  Compiled by imx_prepare(IMX_PREPARE_EPISODE) or on first use
-// outside stream capture; unavailable where the specialised kernels are (small batches) or the layout exceeds 200 KB.
-static void ensure_jit_episode(imx_env* e, bool obs) {
-    int& st = obs ? e->jit_ep_state : e->jit_ep_noobs_state;
-    if (st != 0) return;
-    st = -1;
-    ensure_jit(e);
+    // (only the kernels the module holds take their size)
     EpisodeArgs EA;
-    if (e->jit_state != 1 || episode_layout(e, EA) > 200 * 1024) return;
+    episode_layout(e, EA);
+    smem[0] = L.total;
+    smem[1] = L.total2 <= 200 * 1024 ? L.total2 : L.total;
+    smem[2] = 0;
+    smem[3] = (int)pipe_smem;
+    smem[4] = EA.total;
+}
+
+// Builds and loads one JitVariant of the specialised kernels, once per handle: a failed build is remembered and not retried.
+// The step module is built by imx_create() for large batches (or IMX_JIT=1); the others by imx_prepare() or on first use
+// outside stream capture (module loads are not capturable).
+static void ensure_jit(imx_env* e, int variant) {
+    if (e->jit_state[variant] != 0) return;
+    e->jit_state[variant] = -1;
+    if (variant == JIT_STEP) {
+        if (e->jit_policy < 0 || !e->tma_fn) return;
+        if (e->jit_policy == 0 && e->N < 1024) return;    // below ~1k envs a step is launch latency either way; the compile (1-2 s) is not worth it
+        if (e->tile_jit.total > 200 * 1024) return;
+    } else {
+        ensure_jit(e, JIT_STEP);                           // the other variants serve only where the step module does
+        if (e->jit_state[JIT_STEP] != 1) return;
+        if (variant == JIT_CC && (!e->multi || e->tile_cc.total > 200 * 1024)) return;
+        EpisodeArgs EA;
+        if (variant >= JIT_EPISODE && episode_layout(e, EA) > 200 * 1024) return;
+    }
     imxjit::Spec sp;
-    jit_spec(e, e->TL, sp, obs ? 1 : 0, 0, 1);
-    const int smem[imxjit::N_KERNELS] = {0, 0, 0, 0, EA.total};
-    const imxjit::Kernels* k = imxjit::get(sp, smem, e->cfg.device);
-    (obs ? e->jit_ep : e->jit_ep_noobs) = k;
-    if (k) st = 1;
+    int smem[imxjit::N_KERNELS];
+    jit_spec(e, variant, sp, smem);
+    e->jit[variant] = imxjit::get(sp, smem, e->cfg.device);
+    if (e->jit[variant]) e->jit_state[variant] = 1;
 }
 
 static bool stream_is_capturing(cudaStream_t s) {
@@ -513,60 +538,29 @@ static bool stream_is_capturing(cudaStream_t s) {
     return st != cudaStreamCaptureStatusNone;
 }
 
-// see the comment at the call in select_kernels(); l2_bytes <= 0: the B200's 126 MB (imx_jit_compile_check runs without a device)
-static int decide_l2_hints(const imx_env* e, int l2_bytes) {
-    if (l2_bytes <= 0) l2_bytes = 126 << 20;
-    const int64_t per_env = bytes_per_env(e);
-    const int64_t state_bytes = 4 * (int64_t)e->S * e->N;
-    const char* lh = getenv("IMX_L2_HINTS");
-    if (lh && !strcmp(lh, "1")) return 1;
-    if (lh && !strcmp(lh, "2")) return 2;                  // outputs only (measurement switch)
-    if (lh && !strcmp(lh, "0")) return 0;
-    // below the window: outputs only (2) — the step itself is unchanged (everything is L2-resident), but the step rewards are
-    // still in L2 when imx_episode_stats reads them back after 30 periods of observation traffic (config 2 episode 205.2 -> 202.1 us,
-    // 32 768 envs 143.2 -> 140.3 us; profiles/r2_l2_hints_small_ab.txt)
-    if (per_env * e->N <= (int64_t)l2_bytes / 2) return 2;
-    return state_bytes <= (int64_t)l2_bytes * 5 / 8 ? 1 : 0;
+// The module of `variant` for a launch on stream s, built first if it was never tried and s is not capturing; NULL: the
+// ahead-of-time kernels serve.
+static const imxjit::Kernels* jit_module(imx_env* e, int variant, cudaStream_t s) {
+    if (e->jit_state[variant] == 0 && !stream_is_capturing(s)) ensure_jit(e, variant);
+    return e->jit[variant];
 }
 
 static int select_kernels(imx_env* e) {
-    const int m = e->m;
     pick_kernels(e, m_pad_of(e), e->div);
     const int epw = 32 / e->m_pad;
-    const int tile_bytes = (epw * m * e->O * obs_elem_bytes(e) + 15) & ~15;
+    const int tile_bytes = (epw * e->m * e->O * obs_elem_bytes(e) + 15) & ~15;
     e->step_smem = (size_t)(STEP_THREADS / 32) * tile_bytes;
     IMX_CUDA(raise_dyn_smem_limit((const void*)e->step_fn, e->step_smem));
-    int dev_sms = 0, occ = 0;
+    int dev_sms = 0, occ = 0, l2_bytes = 0;
     IMX_CUDA(cudaDeviceGetAttribute(&dev_sms, cudaDevAttrMultiProcessorCount, e->cfg.device));
     IMX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (const void*)e->step_fn, STEP_THREADS, e->step_smem));
     if (occ < 1) return fail(-4, "step kernel does not fit on an SM (smem %zu B)", e->step_smem);
     e->step_grid_cap = dev_sms * occ;
-    {
-        e->tma_threads = choose_tma_threads(e);
-        const char* dn = getenv("IMX_STEP_DENSE");
-        e->step_dense = (dn && !strcmp(dn, "1")) ? 1 : 0;
-    }
-    compute_tile(e, e->tile, m_pad_of(e));
-    // the specialised STEP kernel keeps the power-of-two tile: a dense m-wide tile makes the per-field byte
-    // ranges (e.g. 40 envs x 6 nodes x 4 B = 960 B) straddle 128-byte lines, measured slower at 262144 envs;
-    // the issue-bound ROLLOUT kernel is specialised with tile width = m (dense lane packing, +21% on div2)
-    {
-        // env-per-thread rollout (imx_rollout_et.cuh): networks up to 8 nodes, lead times up to 4 (registers); IMX_ROLLOUT_ET=0 disables
-        const char* re = getenv("IMX_ROLLOUT_ET");
-        e->rollout_et = (re && !strcmp(re, "0")) ? 0 : (e->m <= 8 && e->D <= 4);
-        // env-per-thread STEP kernels: divergent networks up to 8 nodes (their lane-mapped kernels are issue-bound); IMX_STEP_ET=0/1
-        const char* se = getenv("IMX_STEP_ET");
-        const bool et_ok = e->m <= 8 && e->D <= 4 && e->P <= 2;
-        // default: divergent networks whose node count is not a power of two (the lane mapping pads them: div2 runs 19 of 32 lanes);
-        // div2 262 144 envs 34.9 -> 33.6 us, 1 Mi envs 129 -> 115 us; no gain on the 4-node div1 (profiles/r2_step_et_sweep.txt)
-        const bool non_pow2 = (e->m & (e->m - 1)) != 0;
-        e->step_et = (se && !strcmp(se, "0")) ? 0 : (se && !strcmp(se, "1")) ? et_ok : (et_ok && e->div && non_pow2);
-        const char* st = getenv("IMX_STEP_ET_THREADS");
-        const int et_threads = (st && (atoi(st) == 32 || atoi(st) == 64 || atoi(st) == 128)) ? atoi(st) : 32;
-        e->jit_threads = e->step_et ? et_threads : e->tma_threads;
-    }
-    compute_tile(e, e->tile_jit, e->step_dense ? e->m : m_pad_of(e), false, e->step_et ? e->jit_threads : 0);
-    compute_tile(e, e->tile_cc, e->step_dense ? e->m : m_pad_of(e), true);
+    IMX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (const void*)e->rollout_fn, ROLLOUT_THREADS, 0));
+    if (occ < 1) return fail(-4, "rollout kernel does not fit on an SM");
+    e->rollout_grid_cap = dev_sms * occ;
+    cudaDeviceGetAttribute(&l2_bytes, cudaDevAttrL2CacheSize, e->cfg.device);
+    plan_handle(e, dev_sms, l2_bytes);
     if (e->tile.total <= 200 * 1024) {
         IMX_CUDA(raise_dyn_smem_limit((const void*)e->tma_fn, (size_t)e->tile.total));
         if (e->tile.total2 <= 200 * 1024)
@@ -574,37 +568,6 @@ static int select_kernels(imx_env* e) {
     }
     else
         e->tma_fn = nullptr;
-    {
-        const char* pth = getenv("IMX_STEP_PATH");
-        e->step_path = (pth && !strcmp(pth, "direct")) ? 1 : (pth && !strcmp(pth, "tma")) ? 2 : 0;
-        const char* zc = getenv("IMX_HOST_ZERO_COPY");
-        e->host_zero_copy = (zc && !strcmp(zc, "0")) ? 0 : 1;
-        const char* pd = getenv("IMX_PDL");
-        e->use_pdl = (pd && !strcmp(pd, "0")) ? 0 : 1;
-        const char* fu = getenv("IMX_FUSE_PERIODS");
-        e->fuse_periods = (fu && !strcmp(fu, "0")) ? 0 : 1;
-        const char* jp = getenv("IMX_JIT");
-        e->jit_policy = (jp && !strcmp(jp, "1")) ? 1 : (jp && !strcmp(jp, "0")) ? -1 : 0;
-        const char* pm = getenv("IMX_PIPE");
-        e->pipe_mode = (pm && !strcmp(pm, "1")) ? 1 : (pm && !strcmp(pm, "0")) ? -1 : 0;
-        const char* ps = getenv("IMX_PIPE_STAGES");
-        e->pipe_stages = ps ? atoi(ps) : 0;                 // 0: the measured default of pipe_stages_for()
-        if (e->pipe_stages < 2 || e->pipe_stages > 8) e->pipe_stages = 0;
-        const char* pc = getenv("IMX_PIPE_CTAS");
-        e->pipe_ctas = pc ? atoi(pc) : 0;
-        e->sm_count = dev_sms;
-        // L2 eviction priorities (observation stream evict_first, state + rewards evict_last): they pay exactly where a launch
-        // streams more than about half of L2 while the state itself would still fit — the write-once stream then no longer
-        // pushes the state out between two periods (config 2 at 262 144 envs 20.7 -> 16.6 us = 1.15 of the HBM copy peak, div2
-        // 33.4 -> 27.1 us, 8-stage 49.2 -> 43.0 us); below that everything is L2-resident anyway (-1 %), above it the state does
-        // not fit and the priorities only disturb the replacement (-2 .. -4 %).  profiles/r2_l2_hints_ab.txt
-        int l2_bytes = 0;
-        cudaDeviceGetAttribute(&l2_bytes, cudaDevAttrL2CacheSize, e->cfg.device);
-        e->l2_hints = decide_l2_hints(e, l2_bytes);
-    }
-    IMX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (const void*)e->rollout_fn, ROLLOUT_THREADS, 0));
-    if (occ < 1) return fail(-4, "rollout kernel does not fit on an SM");
-    e->rollout_grid_cap = dev_sms * occ;
     return 0;
 }
 
@@ -987,7 +950,7 @@ extern "C" int imx_create(const imx_config* cfg, imx_env** out) {
         IMX_CREATE_CUDA(cudaDeviceSynchronize());
     }
 #undef IMX_CREATE_CUDA
-    ensure_jit(e);            // compile / load the specialised kernels now: no later call compiles on the step path
+    ensure_jit(e, JIT_STEP);  // compile / load the specialised kernels now: no later call compiles on the step path
     *out = e;
     return 0;
 }
@@ -1046,6 +1009,39 @@ extern "C" int imx_set_period(imx_env* e, int t) {
 // --------------------------------------------------------------------------------------
 // reset / step
 // --------------------------------------------------------------------------------------
+// launches `kern` as a programmatic dependent of the kernel in front of it on the stream (the kernel itself starts with
+// griddepcontrol.wait): its launch latency overlaps the predecessor's tail
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_dependent(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl, Args... args) {
+    cudaLaunchConfig_t lc;
+    memset(&lc, 0, sizeof(lc));
+    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = smem; lc.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    lc.attrs = at;
+    lc.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&lc, kern, KArgs(args)...);
+}
+
+// the same for a runtime-specialised kernel (driver API); counts the launch
+static CUresult launch_dependent_jit(CUfunction f, unsigned grid, unsigned block, unsigned smem, cudaStream_t s, bool pdl, void** params) {
+    CUlaunchConfig lc;
+    memset(&lc, 0, sizeof(lc));
+    lc.gridDimX = grid; lc.gridDimY = 1; lc.gridDimZ = 1;
+    lc.blockDimX = block; lc.blockDimY = 1; lc.blockDimZ = 1;
+    lc.sharedMemBytes = smem;
+    lc.hStream = (CUstream)s;
+    CUlaunchAttribute at[1];
+    at[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
+    at[0].value.programmaticStreamSerializationAllowed = 1;
+    lc.attrs = at;
+    lc.numAttrs = pdl ? 1 : 0;
+    const CUresult cr = imxjit::g_api.LaunchKernelEx(&lc, f, params, nullptr);
+    if (cr == CUDA_SUCCESS) g_launches.fetch_add(1, std::memory_order_relaxed);
+    return cr;
+}
+
 // launches the reset fill kernel (state zero + inv init + optional t = 0 observation)
 static void launch_reset_kernel(imx_env* e, double* obs_dev, cudaStream_t s, const int32_t* demand_in) {
     StepArgs A;
@@ -1059,22 +1055,11 @@ static void launch_reset_kernel(imx_env* e, double* obs_dev, cudaStream_t s, con
     Z.demand_T = e->d_demand_T;
     Z.R = e->R; Z.T = e->T;
     const int64_t work = (obs_dev ? e->N * e->m * e->O : 0) > Z.zero_words / 4 ? e->N * e->m * e->O : Z.zero_words / 4;
-    int sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->cfg.device);
     int64_t blocks = (work + 255) / 256;
-    if (blocks > (int64_t)sms * 8) blocks = (int64_t)sms * 8;
+    if (blocks > (int64_t)e->sm_count * 8) blocks = (int64_t)e->sm_count * 8;
     if (blocks < 1) blocks = 1;
     const size_t smem = (size_t)e->m * e->O * sizeof(double) + (size_t)e->m * sizeof(int32_t);   // template sized for float64
-    // a programmatic dependent of whatever is in front of it on the stream (the kernel starts with griddepcontrol.wait)
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = dim3((unsigned)blocks); lc.blockDim = dim3(256); lc.dynamicSmemBytes = smem; lc.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = at;
-    lc.numAttrs = e->use_pdl ? 1 : 0;
-    cudaLaunchKernelEx(&lc, e->reset_fn, A, Z, e->div ? 1 : 0);
+    launch_dependent(e->reset_fn, dim3((unsigned)blocks), dim3(256), smem, s, e->use_pdl, A, Z, e->div ? 1 : 0);
 }
 
 static DemandGen make_gen(const imx_env* e, uint64_t episode) {
@@ -1126,8 +1111,7 @@ extern "C" int imx_reset(imx_env* e, const int32_t* demand_dev, const uint8_t* d
 // (one-wave regime: -3 % .. -20 % per launch; even with one tile per CTA its compute warps retire early, which lets the
 // next dependent launch in sooner); for larger serial batches the one-tile-per-CTA kernel already runs at the HBM copy peak
 // and the ring's smaller resident tile count costs 5-10 %.
-static bool pipe_pays(const imx_env* e, int n_tiles) {
-    (void)n_tiles;
+static bool pipe_pays(const imx_env* e) {
     if (e->step_et) return bytes_per_env(e) * e->N <= ((int64_t)384 << 20);   // env-per-thread tiles: one-tile kernel from ~0.5 Mi envs (div2: 115 vs 124 us at 1 Mi)
     if (e->div) return true;
     if (e->l2_hints) return true;                          // the priorities live in the pipelined kernel (serial 4-stage at 512 Ki envs: 38.0 vs 41.8 us)
@@ -1193,10 +1177,10 @@ static int launch_step(imx_env* e, const void* actions_dev, double* obs_dev, dou
     bool with_cc = false;
     if (cc_fused) *cc_fused = false;
     if (cc && tma_legal && !A.has_info && obs_dev && aligned16(cc->dev) && tile_io_whole16(e, e->tile_cc, true)) {
-        if (e->jit_cc_state == 0 && !stream_is_capturing(s)) ensure_jit_cc(e);
+        const imxjit::Kernels* k = jit_module(e, JIT_CC, s);
         const int64_t whole = (e->N / e->tile_cc.E) * e->tile_cc.E;
-        if (e->jit_cc_state == 1 && whole == e->N) {       // fused only when every env sits in a whole tile (else: unfused fallback)
-            jk = e->jit_cc;
+        if (k && whole == e->N) {                          // fused only when every env sits in a whole tile (else: unfused fallback)
+            jk = k;
             use_jit = with_cc = true;
             A.cc = cc->dev; A.cc_fill = cc->fill; A.cc_lo = cc->lo; A.cc_hi = cc->hi;
             A.cc_W = (e->m - 1) * (1 + e->O) + e->O;
@@ -1205,13 +1189,8 @@ static int launch_step(imx_env* e, const void* actions_dev, double* obs_dev, dou
     }
     if (!with_cc && tma_legal && !A.has_info) {
         // the specialised kernels were loaded by imx_create() / imx_prepare(); the obs-less variant may still be
-        // compiled here on first use, but never while the stream is being captured (module loads are not capturable)
-        if (obs_dev) { if (e->jit_state == 1) jk = e->jit; }
-        else {
-            if (e->jit_noobs_state == 0 && !stream_is_capturing(s)) ensure_jit_noobs(e);
-            if (e->jit_noobs_state == 1) jk = e->jit_noobs;
-            else if (e->jit_state == 1 && e->jit_noobs_state == 0) jk = nullptr;   // capture in progress: ahead-of-time kernel
-        }
+        // compiled here on first use, but never while the stream is being captured (then the ahead-of-time kernel serves)
+        jk = jit_module(e, obs_dev ? JIT_STEP : JIT_NOOBS, s);
         use_jit = jk != nullptr;
     }
     const TileLayout& TL_use = with_cc ? e->tile_cc : use_jit ? e->tile_jit : e->tile;
@@ -1232,43 +1211,22 @@ static int launch_step(imx_env* e, const void* actions_dev, double* obs_dev, dou
             PipeArgs PA;
             PA.n_tiles = (int32_t)(n_tma / TL_use.E);
             PA.stages = pipe_stages_for(e, TL_use);
-            const bool pipe = !fused && jk->step_pipe && e->pipe_mode >= 0 && (e->pipe_mode == 1 || pipe_pays(e, PA.n_tiles));
+            const bool pipe = !fused && jk->step_pipe && e->pipe_mode >= 0 && (e->pipe_mode == 1 || pipe_pays(e));
             void* params[] = {(void*)&A, (void*)&TL_use, (void*)&PA};
-            CUlaunchConfig lc;
-            memset(&lc, 0, sizeof(lc));
-            lc.gridDimX = (unsigned)(n_tma / TL_use.E); lc.gridDimY = 1; lc.gridDimZ = 1;
-            const unsigned jthreads = (unsigned)((with_cc && e->step_et) ? e->tma_threads : e->jit_threads);
-            lc.blockDimX = jthreads; lc.blockDimY = 1; lc.blockDimZ = 1;
-            lc.sharedMemBytes = tma_smem;
+            unsigned grid = (unsigned)(n_tma / TL_use.E), block = (unsigned)((with_cc && e->step_et) ? e->tma_threads : e->jit_threads);
+            unsigned smem = tma_smem;
             if (pipe) {
                 const int64_t resident = (int64_t)e->sm_count * pipe_ctas_for(e, TL_use);
-                lc.gridDimX = (unsigned)(PA.n_tiles < resident ? PA.n_tiles : resident);
-                lc.blockDimX = jthreads + 32;
-                lc.sharedMemBytes = (unsigned)(PA.stages * TL_use.total);
+                grid = (unsigned)(PA.n_tiles < resident ? PA.n_tiles : resident);
+                block += 32;
+                smem = (unsigned)(PA.stages * TL_use.total);
             }
-            lc.hStream = (CUstream)s;
-            CUlaunchAttribute at[1];
-            at[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
-            at[0].value.programmaticStreamSerializationAllowed = 1;
-            lc.attrs = at;
-            lc.numAttrs = e->use_pdl ? 1 : 0;
-            const CUresult cr = imxjit::g_api.LaunchKernelEx(&lc, pipe ? jk->step_pipe : fused ? jk->step_many : jk->step, params, nullptr);
+            const CUresult cr = launch_dependent_jit(pipe ? jk->step_pipe : fused ? jk->step_many : jk->step, grid, block, smem, s, e->use_pdl, params);
             if (cr != CUDA_SUCCESS) return fail(-3, "launch of the specialised step kernel failed (CUresult %d)", (int)cr);
-            g_launches.fetch_add(1, std::memory_order_relaxed);
             e->last_variant = pipe ? 3 : 2;
         } else {
-            cudaLaunchConfig_t lc;
-            memset(&lc, 0, sizeof(lc));
-            lc.gridDim = dim3((unsigned)(n_tma / TL_use.E));
-            lc.blockDim = dim3((unsigned)e->tma_threads);
-            lc.dynamicSmemBytes = (size_t)tma_smem;
-            lc.stream = s;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-            at[0].val.programmaticStreamSerializationAllowed = 1;
-            lc.attrs = at;
-            lc.numAttrs = e->use_pdl ? 1 : 0;
-            IMX_CUDA(cudaLaunchKernelEx(&lc, fused ? e->tma_many_fn : e->tma_fn, A, e->tile));
+            IMX_CUDA(launch_dependent(fused ? e->tma_many_fn : e->tma_fn, dim3((unsigned)(n_tma / TL_use.E)), dim3((unsigned)e->tma_threads),
+                                      (size_t)tma_smem, s, e->use_pdl, A, e->tile));
             IMX_CHECK_LAUNCH("step_kernel_tma");
             e->last_variant = 1;
         }
@@ -1327,18 +1285,18 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
     IMX_CUDA(cudaSetDevice(e->cfg.device));
     // (0 keeps meaning the five flags it always meant: IMX_PREPARE_EPISODE compiles two more modules and is asked for explicitly)
     if (flags == 0) flags = IMX_PREPARE_STEP | IMX_PREPARE_NOOBS | IMX_PREPARE_HOST | IMX_PREPARE_DFO | IMX_PREPARE_CC;
-    if (flags & IMX_PREPARE_STEP) ensure_jit(e);
-    if (flags & IMX_PREPARE_NOOBS) ensure_jit_noobs(e);
+    if (flags & IMX_PREPARE_STEP) ensure_jit(e, JIT_STEP);
+    if (flags & IMX_PREPARE_NOOBS) ensure_jit(e, JIT_NOOBS);
     if (flags & IMX_PREPARE_HOST) { const int rc = ensure_host_path(e); if (rc) return rc; }
     if ((flags & IMX_PREPARE_CC) && e->multi) {
-        ensure_jit_cc(e);
+        ensure_jit(e, JIT_CC);
         if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, (size_t)e->N * e->m * e->O * obs_elem_bytes(e)));
     }
     if ((flags & IMX_PREPARE_DFO) && !e->multi && !e->d_dfo_rewards)
         IMX_CUDA(cudaMalloc(&e->d_dfo_rewards, (size_t)e->T * e->N * sizeof(double)));
     if (flags & IMX_PREPARE_EPISODE) {                     // both episode modules + every scratch buffer of the unfused form
-        ensure_jit_episode(e, true);
-        ensure_jit_episode(e, false);
+        ensure_jit(e, JIT_EPISODE);
+        ensure_jit(e, JIT_EPISODE_NOOBS);
         const size_t cols = e->multi ? e->m : 1, cells = (size_t)e->N * e->m;
         if (!e->d_ep_rewards) IMX_CUDA(cudaMalloc(&e->d_ep_rewards, (size_t)e->T * e->N * cols * sizeof(double)));
         if (!e->d_ep_profit) IMX_CUDA(cudaMalloc(&e->d_ep_profit, cells * sizeof(double)));
@@ -1405,8 +1363,7 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
     const int64_t N = e->N;
     const int m = e->m;
     const size_t cols = e->multi ? m : 1, cells = (size_t)N * m, es = obs_elem_bytes(e), aes = act_elem_bytes(e);
-    if (!capturing) ensure_jit_episode(e, obs_dev != nullptr);
-    const imxjit::Kernels* jk = obs_dev ? e->jit_ep : e->jit_ep_noobs;
+    const imxjit::Kernels* jk = jit_module(e, obs_dev ? JIT_EPISODE : JIT_EPISODE_NOOBS, s);
     EpisodeArgs EA;
     memset(&EA, 0, sizeof(EA));
     const int64_t smem = episode_layout(e, EA, return_dev || stats_dev, eval_acc_dev != nullptr);
@@ -1456,20 +1413,8 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
         EA.delay_thr = e->cfg.noisy_delay_threshold;
         EA.rescaled = (e->cfg.kind == IMX_KIND_MAIM_DIV || e->cfg.standardise_state) ? 1 : 0;
         void* params[] = {(void*)&A, (void*)&e->tile_jit, (void*)&EA};
-        CUlaunchConfig lc;
-        memset(&lc, 0, sizeof(lc));
-        lc.gridDimX = (unsigned)(N / E); lc.gridDimY = 1; lc.gridDimZ = 1;
-        lc.blockDimX = (unsigned)e->jit_threads; lc.blockDimY = 1; lc.blockDimZ = 1;
-        lc.sharedMemBytes = (unsigned)smem;
-        lc.hStream = (CUstream)s;
-        CUlaunchAttribute at[1];
-        at[0].id = CU_LAUNCH_ATTRIBUTE_PROGRAMMATIC_STREAM_SERIALIZATION;
-        at[0].value.programmaticStreamSerializationAllowed = 1;
-        lc.attrs = at;
-        lc.numAttrs = e->use_pdl ? 1 : 0;
-        const CUresult cr = imxjit::g_api.LaunchKernelEx(&lc, jk->step_episode, params, nullptr);
+        const CUresult cr = launch_dependent_jit(jk->step_episode, (unsigned)(N / E), (unsigned)e->jit_threads, (unsigned)smem, s, e->use_pdl, params);
         if (cr != CUDA_SUCCESS) return fail(-3, "launch of the episode kernel failed (CUresult %d)", (int)cr);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
         e->last_variant = 4;
         e->t = e->T;
         e->episode = episode;
@@ -1550,7 +1495,8 @@ extern "C" int imx_rollout_basestock(imx_env* e, const double* z_dev, int z_stri
     const int64_t warp_tiles = (e->N + epw - 1) / epw;
     const int64_t blocks_needed = (warp_tiles + (ROLLOUT_THREADS / 32) - 1) / (ROLLOUT_THREADS / 32);
     const unsigned grid = (unsigned)(blocks_needed < e->rollout_grid_cap ? blocks_needed : e->rollout_grid_cap);
-    if (e->jit_state == 1 && e->jit->rollout && e->rollout_et) {
+    const imxjit::Kernels* jk = e->jit[JIT_STEP];
+    if (jk && jk->rollout && e->rollout_et) {
         EtNodeConsts C;
         memset(&C, 0, sizeof(C));
         for (int i = 0; i < e->m; ++i) {
@@ -1560,12 +1506,12 @@ extern "C" int imx_rollout_basestock(imx_env* e, const double* z_dev, int z_stri
         const int64_t blocks = (e->N + ET_THREADS_HOST - 1) / ET_THREADS_HOST;
         const int64_t cap = (int64_t)e->sm_count * 16;
         Rg.coop_demand = 0;
-        const CUresult cr = imxjit::g_api.LaunchKernel(e->jit->rollout, (unsigned)(blocks < cap ? blocks : cap), 1, 1, ET_THREADS_HOST, 1, 1, 0, (CUstream)s,
+        const CUresult cr = imxjit::g_api.LaunchKernel(jk->rollout, (unsigned)(blocks < cap ? blocks : cap), 1, 1, ET_THREADS_HOST, 1, 1, 0, (CUstream)s,
                                                        params, nullptr);
         if (cr != CUDA_SUCCESS) return fail(-3, "launch of the env-per-thread rollout kernel failed (CUresult %d)", (int)cr);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         e->last_variant = 2;
-    } else if (e->jit_state == 1 && e->jit->rollout) {
+    } else if (jk && jk->rollout) {
         void* params[] = {(void*)&A, (void*)&Rg};
         const int epw_j = 32 / e->m;                         // dense packing in the specialised build
         const int64_t wt_j = (e->N + epw_j - 1) / epw_j;
@@ -1575,7 +1521,7 @@ extern "C" int imx_rollout_basestock(imx_env* e, const double* z_dev, int z_stri
         const size_t draw_j = (size_t)(ROLLOUT_THREADS / 32) * epw_j * e->R * ((e->T + 1) & ~1) * sizeof(int32_t);
         if (coop && draw_j > 40 * 1024) Rg.coop_demand = 0;
         const size_t roll_smem_j = Rg.coop_demand ? draw_j : 0;
-        const CUresult cr = imxjit::g_api.LaunchKernel(e->jit->rollout, g2, 1, 1, ROLLOUT_THREADS, 1, 1, (unsigned)roll_smem_j, (CUstream)s, params, nullptr);
+        const CUresult cr = imxjit::g_api.LaunchKernel(jk->rollout, g2, 1, 1, ROLLOUT_THREADS, 1, 1, (unsigned)roll_smem_j, (CUstream)s, params, nullptr);
         if (cr != CUDA_SUCCESS) return fail(-3, "launch of the specialised rollout kernel failed (CUresult %d)", (int)cr);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         e->last_variant = 2;
@@ -1592,21 +1538,6 @@ extern "C" int imx_rollout_basestock(imx_env* e, const double* z_dev, int z_stri
     return 0;
 }
 
-// launches `kern` as a programmatic dependent of the kernel in front of it on the stream (the kernel itself starts with
-// griddepcontrol.wait): its launch latency overlaps the predecessor's tail
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_dependent(void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t s, bool pdl, Args... args) {
-    cudaLaunchConfig_t lc;
-    memset(&lc, 0, sizeof(lc));
-    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = 0; lc.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = at;
-    lc.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&lc, kern, KArgs(args)...);
-}
-
 // stage 1 (one block per slice of envs; FUSED adds the step rewards first) + stage 2 of the return statistics
 static int launch_return_stats(imx_env* e, const double* src, int periods, bool fused, double* ret_out, double* stats_dev, int accumulate,
                                cudaStream_t s) {
@@ -1619,13 +1550,13 @@ static int launch_return_stats(imx_env* e, const double* src, int periods, bool 
     // one row of "step rewards" whose sum nobody asked for IS the returns: the plain kernel keeps four loads per thread in flight
     if (fused && periods == 1 && !ret_out) fused = false;
     if (fused)
-        IMX_CUDA(launch_dependent(stats_slice_kernel<true>, dim3((unsigned)nslices), dim3(STATS_THREADS), s, pdl, src, ret_out, e->d_stats_partial,
+        IMX_CUDA(launch_dependent(stats_slice_kernel<true>, dim3((unsigned)nslices), dim3(STATS_THREADS), 0, s, pdl, src, ret_out, e->d_stats_partial,
                                   e->N, cols, per_agent, periods, epb, nslices));
     else
-        IMX_CUDA(launch_dependent(stats_slice_kernel<false>, dim3((unsigned)nslices), dim3(STATS_THREADS), s, pdl, src, (double*)nullptr,
+        IMX_CUDA(launch_dependent(stats_slice_kernel<false>, dim3((unsigned)nslices), dim3(STATS_THREADS), 0, s, pdl, src, (double*)nullptr,
                                   e->d_stats_partial, e->N, cols, per_agent, 1, epb, nslices));
     g_launches.fetch_add(1, std::memory_order_relaxed);
-    IMX_CUDA(launch_dependent(stats_final_kernel, dim3((unsigned)nstat), dim3(STATS_THREADS), s, pdl, (const double*)e->d_stats_partial, stats_dev,
+    IMX_CUDA(launch_dependent(stats_final_kernel, dim3((unsigned)nstat), dim3(STATS_THREADS), 0, s, pdl, (const double*)e->d_stats_partial, stats_dev,
                               e->N, nslices, accumulate));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return 0;
@@ -1797,29 +1728,14 @@ extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* l
     tmp.cfg = *cfg;
     const int rc = derive(&tmp);
     if (rc) return rc;
-    tmp.tma_threads = choose_tma_threads(&tmp);
-    {
-        const char* re = getenv("IMX_ROLLOUT_ET");
-        tmp.rollout_et = (re && !strcmp(re, "0")) ? 0 : (tmp.m <= 8 && tmp.D <= 4);
-        const char* se = getenv("IMX_STEP_ET");
-        const bool et_ok = tmp.m <= 8 && tmp.D <= 4 && tmp.P <= 2;
-        const bool non_pow2 = (tmp.m & (tmp.m - 1)) != 0;
-        tmp.step_et = (se && !strcmp(se, "0")) ? 0 : (se && !strcmp(se, "1")) ? et_ok : (et_ok && tmp.div && non_pow2);
-        const char* st = getenv("IMX_STEP_ET_THREADS");
-        const int et_threads = (st && (atoi(st) == 32 || atoi(st) == 64 || atoi(st) == 128)) ? atoi(st) : 32;
-        tmp.jit_threads = tmp.step_et ? et_threads : tmp.tma_threads;
-        tmp.l2_hints = decide_l2_hints(&tmp, 0);
-    }
-    compute_tile(&tmp, tmp.tile, m_pad_of(&tmp));
-    compute_tile(&tmp, tmp.tile_jit, m_pad_of(&tmp), false, tmp.step_et ? tmp.jit_threads : 0);
-    compute_tile(&tmp, tmp.tile_cc, m_pad_of(&tmp), true);
-    int TL = 0;
-    build_tables(&tmp, &TL);
-    imxjit::Spec sp;
-    if (variant == 2 && !tmp.multi) return fail(-1, "the critic rows exist for the multi-agent kinds only");
+    plan_handle(&tmp, 148, 0);
+    build_tables(&tmp, &tmp.TL);
+    if (variant == JIT_CC && !tmp.multi) return fail(-1, "the critic rows exist for the multi-agent kinds only");
     EpisodeArgs EA;
-    if (variant >= 3 && episode_layout(&tmp, EA) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
-    jit_spec(&tmp, TL, sp, (variant == 1 || variant == 4) ? 0 : 1, variant == 2 ? 1 : 0, variant >= 3 ? 1 : 0);
+    if (variant >= JIT_EPISODE && episode_layout(&tmp, EA) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
+    imxjit::Spec sp;
+    int smem[imxjit::N_KERNELS];
+    jit_spec(&tmp, variant, sp, smem);
     std::string lg;
     std::vector<char> cubin;
     const size_t n = imxjit::compile_only(sp, lg, &cubin);

@@ -44,7 +44,9 @@
 extern "C" {
 #endif
 
-#define IMX_ABI_VERSION 3     /* 3 (later, source-compatible): imx_config.reserved0 became io_flags (bfloat16 observations, float32
+#define IMX_ABI_VERSION 3     /* 3 (later, source-compatible): imx_records_out, imx_replay_episode_records, IMX_PREPARE_RECORDS and
+                                 imx_jit_compile_check variants 5 / 6 (the episode kernel with per-period records).
+                                 3 (later, source-compatible): imx_config.reserved0 became io_flags (bfloat16 observations, float32
                                  actions); action pointers are const void* (imx_replay_episode's keeps its spelling); imx_round_bf16.
                                  3: obs pointers are void* (float64, or float32 with cfg.obs_f32) everywhere; imx_rollout_basestock gained
                                  delay_mask_dev / noisy and takes pmf [N][R][T]; imx_prepare; imx_step_cc.
@@ -122,6 +124,20 @@ typedef struct imx_info_out {
     double*  profit_dev;       /* [N][m] */
 } imx_info_out;
 
+/* Per-period records of one episode: the reference's history arrays (MAIM_env.py:222-230, DSHLP_4.py:918-923).
+ * Any pointer may be NULL (not recorded).  Row t of a [T][N][m] block is period t; the state blocks have T + 1 rows,
+ * row 0 = the reset state, row t + 1 = the state after period t (the reference's inv[t + 1, :]). */
+typedef struct imx_records_out {
+    int32_t* inv_dev;          /* [T+1][N][m] */
+    int32_t* backlog_dev;      /* [T+1][N][m] */
+    int32_t* order_u_dev;      /* [T+1][N][m] */
+    int32_t* demand_dev;       /* [T][N][m]   what imx_info_out.demand_dev reports for period t */
+    int32_t* ship_dev;         /* [T][N][m] */
+    int32_t* acquisition_dev;  /* [T][N][m] */
+    int32_t* order_dev;        /* [T][N][m]   'actual order' (order_r) */
+    double*  profit_dev;       /* [T][N][m] */
+} imx_records_out;
+
 /* State fields for imx_state_field(): the persistent per-env state is exactly these int32
  * arrays (SURVEY.md appendix A.2); everything else in the reference's [T+1, m] arrays is history. */
 enum imx_field {
@@ -156,11 +172,12 @@ int imx_destroy(imx_env* env);
  *          obs_dev = NULL specialisation), IMX_PREPARE_HOST (staging buffers + stream of the *_host calls),
  *          IMX_PREPARE_DFO (scratch of the dfo objective), IMX_PREPARE_CC (imx_step_cc's specialisation and scratch),
  *          IMX_PREPARE_EPISODE (imx_replay_episode's two episode kernels, with and without observations, and the scratch
- *          buffers of its unfused form: [T][N](m) rewards, [N][m][O] observations, [N][m] profits, [N](m) returns);
- *          0 = the first five (STEP | NOOBS | HOST | DFO | CC; not EPISODE, so existing callers compile nothing more).
+ *          buffers of its unfused form: [T][N](m) rewards, [N][m][O] observations, [N][m] profits, [N](m) returns),
+ *          IMX_PREPARE_RECORDS (imx_replay_episode_records' two episode kernels with records and the same scratch buffers);
+ *          0 = the first five (STEP | NOOBS | HOST | DFO | CC; not EPISODE or RECORDS, so existing callers compile nothing more).
  *          Synchronous; may take seconds (NVRTC). */
 enum imx_prepare_flags { IMX_PREPARE_STEP = 1, IMX_PREPARE_NOOBS = 2, IMX_PREPARE_HOST = 4, IMX_PREPARE_DFO = 8, IMX_PREPARE_CC = 16,
-                         IMX_PREPARE_EPISODE = 32 };
+                         IMX_PREPARE_EPISODE = 32, IMX_PREPARE_RECORDS = 64 };
 int imx_prepare(imx_env* env, int flags);
 
 /* Derived sizes: O (observation length per agent), S (int32 state words per env), R, L, NB. */
@@ -229,6 +246,23 @@ int imx_step_many(imx_env* env, const void* actions_dev, int K, void* obs_dev, d
 int imx_replay_episode(imx_env* env, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
                        const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
                        double* stats_dev, int accumulate, double* eval_acc_dev, void* stream);
+
+/* imx_replay_episode that also records every period: the reference's history arrays (env.inv / backlog / order_u,
+ * MAIM_env.py:222-230) and the LP replay loop's array_demand / array_ship / array_acquisition / array_profit
+ * (DSHLP_4.py:918-923), bit for bit what a reset + T imx_step calls with imx_info_out and a copy of the state fields
+ * after the reset and after every step would give.  records may be NULL (= imx_replay_episode, which is this call with
+ * records = NULL); every other argument and output as in imx_replay_episode.
+ * Wherever the runtime-specialised kernels serve the whole batch with one tile per CTA (imx_replay_episode's conditions, on
+ * divergent networks with and without observations alike, plus 16-byte aligned record pointers and whole 16-byte units per
+ * tile, E * m * 4 bytes) this is one launch: the episode kernel with records writes them with bulk stores next to the
+ * observations and rewards (imx_kernel_variant() = 4).  Elsewhere the library runs the composition:
+ * imx_reset, then per period imx_step with imx_info_out pointing into row t and cudaMemcpyAsync device-to-device copies of
+ * the three state fields into their rows — the same bytes.  Under stream capture call imx_prepare(IMX_PREPARE_RECORDS)
+ * first; without it a call with records under capture returns an error. */
+int imx_replay_episode_records(imx_env* env, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
+                               const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
+                               double* stats_dev, int accumulate, double* eval_acc_dev, const imx_records_out* records,
+                               void* stream);
 
 /* dfo_func's loop  —  base_restock_policy.py:24-45 with base_stock_policy :4-21 fused in: a whole
  * K = T period episode per env in ONE kernel, state on chip.
@@ -322,7 +356,8 @@ const char* imx_jit_log(void);
 /* Compiles the specialised kernels for `cfg` with NVRTC for sm_100a WITHOUT a GPU (build check; also warms the on-disk
  * cubin cache).  variant: 0 = the step / step_many / rollout / pipelined kernels, 1 = the same without observations
  * (obs_dev = NULL), 2 = with the centralised-critic rows (imx_step_cc), 3 = imx_replay_episode's episode kernel,
- * 4 = the same without observations.
+ * 4 = the same without observations, 5 = the episode kernel with records (imx_replay_episode_records), 6 = the same
+ * without observations.
  * Returns the cubin size in bytes, or a negative error; `log` receives the compiler log. */
 int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap);
 

@@ -13,6 +13,7 @@ ABI_VERSION = 3          # IMX_ABI_VERSION of include/imx_b200.h this binding mi
 KIND = {"IM": 0, "MAIM": 1, "IM_div": 2, "MAIM_div": 3}
 DIST = {"replay": 0, "custom": 0, "poisson": 1, "uniform": 2}
 PREPARE_EPISODE = 32    # IMX_PREPARE_EPISODE: imx_replay_episode's kernels and scratch (imx_prepare)
+PREPARE_RECORDS = 64    # IMX_PREPARE_RECORDS: imx_replay_episode_records' kernels and scratch (imx_prepare)
 IO_OBS_BF16, IO_ACTIONS_F32 = 1, 2   # imx_config.io_flags: bfloat16 observations, float32 actions
 F_INV, F_BACKLOG, F_ORDER_U, F_PIPE, F_HIST_D, F_HIST_O, F_CARRY, F_BACKLOG_TO, F_ERROR, F_DEMAND, F_DELAY_MASK = range(11)
 
@@ -42,6 +43,11 @@ class ImxInfoOut(C.Structure):
                 ("order_dev", C.c_void_p), ("profit_dev", C.c_void_p)]
 
 
+class ImxRecordsOut(C.Structure):
+    _fields_ = [("inv_dev", C.c_void_p), ("backlog_dev", C.c_void_p), ("order_u_dev", C.c_void_p), ("demand_dev", C.c_void_p),
+                ("ship_dev", C.c_void_p), ("acquisition_dev", C.c_void_p), ("order_dev", C.c_void_p), ("profit_dev", C.c_void_p)]
+
+
 # every symbol include/imx_b200.h declares: (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -65,6 +71,8 @@ SYMBOLS = {
     "imx_step": (C.c_int, [_P, _P, _P, _P, C.POINTER(ImxInfoOut), _P]),
     "imx_step_many": (C.c_int, [_P, _P, C.c_int, _P, _P, C.POINTER(ImxInfoOut), _P]),
     "imx_replay_episode": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, C.c_int, _P, _P]),
+    "imx_replay_episode_records": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, C.c_int, _P,
+                                             C.POINTER(ImxRecordsOut), _P]),
     "imx_rollout_basestock": (C.c_int, [_P, _P, C.c_int, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, C.c_int, _P]),
     "imx_prepare": (C.c_int, [_P, C.c_int]),
     "imx_step_cc": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_double, C.c_double, _P, _P]),

@@ -83,8 +83,11 @@ typedef void (*reset_fn_t)(const StepArgs, const ResetArgs, int);
 // The runtime-specialised modules a handle may load, numbered as imx_jit_compile_check's `variant`: the step kernels (step,
 // step_many, rollout, pipelined); the same without the observation output (step / step_many with obs = NULL: scoring a stored
 // plan needs rewards only — the observation build and 60 % of the bytes fold away); the step with the centralised-critic rows
-// (imx_step_cc); the one-launch episode kernel (imx_replay_episode) with and without observations.
-enum JitVariant { JIT_STEP, JIT_NOOBS, JIT_CC, JIT_EPISODE, JIT_EPISODE_NOOBS, JIT_VARIANTS };
+// (imx_step_cc); the one-launch episode kernel (imx_replay_episode) with and without observations; the same with per-period
+// records (imx_replay_episode_records), with and without observations.
+enum JitVariant { JIT_STEP, JIT_NOOBS, JIT_CC, JIT_EPISODE, JIT_EPISODE_NOOBS, JIT_EPISODE_REC, JIT_EPISODE_REC_NOOBS, JIT_VARIANTS };
+static bool jit_has_obs(int variant) { return variant != JIT_NOOBS && variant != JIT_EPISODE_NOOBS && variant != JIT_EPISODE_REC_NOOBS; }
+static bool jit_has_rec(int variant) { return variant == JIT_EPISODE_REC || variant == JIT_EPISODE_REC_NOOBS; }
 
 struct imx_env {
     imx_config cfg;
@@ -133,6 +136,8 @@ struct imx_env {
     int tma_threads = 256;               // CTA size of the TMA kernel (IMX_TMA_THREADS: 64, 128 or 256)
     int use_pdl = 1;                     // chain step launches with programmatic dependent launch (IMX_PDL=0 disables)
     int fuse_periods = 1;                // imx_step_many advances all its periods in one launch (IMX_FUSE_PERIODS=0: K plain launches)
+    int episode_fuse = 0;                // imx_replay_episode(_records) on divergent networks: 0 the measured rule, 1 the episode kernel
+                                         // wherever it is legal, -1 never (IMX_EPISODE_FUSE; a measurement switch)
     int l2_hints = 0;                    // L2 eviction priorities on the pipelined kernel's bulk copies (IMX_L2_HINTS; default: see decide_l2_hints)
     int step_et = 0;                     // the specialised STEP kernels use the env-per-thread period (IMX_STEP_ET; default: divergent networks, m <= 8)
     int rollout_et = 0;                  // the specialised ROLLOUT kernel is the env-per-thread one (imx_rollout_et.cuh; IMX_ROLLOUT_ET, default m <= 8)
@@ -317,6 +322,8 @@ static void plan_handle(imx_env* e, int sm_count, int l2_bytes) {
     e->use_pdl = (pd && !strcmp(pd, "0")) ? 0 : 1;
     const char* fu = getenv("IMX_FUSE_PERIODS");
     e->fuse_periods = (fu && !strcmp(fu, "0")) ? 0 : 1;
+    const char* ef = getenv("IMX_EPISODE_FUSE");
+    e->episode_fuse = (ef && !strcmp(ef, "1")) ? 1 : (ef && !strcmp(ef, "0")) ? -1 : 0;
     const char* jp = getenv("IMX_JIT");
     e->jit_policy = (jp && !strcmp(jp, "1")) ? 1 : (jp && !strcmp(jp, "0")) ? -1 : 0;
     const char* pm = getenv("IMX_PIPE");
@@ -331,17 +338,30 @@ static void plan_handle(imx_env* e, int sm_count, int l2_bytes) {
 
 // Shared-memory layout of the episode kernel: tile_jit's multi-period layout, then the episode regions of EpisodeArgs that the
 // call needs (the returns and the accumulators adjacent: the kernel zeroes [off_ret, off_prof) in one loop) — a launch reserves
-// no bytes it does not use, since resident CTAs per SM bound this latency-bound loop.  Returns the total bytes.
-static int64_t episode_layout(const imx_env* e, EpisodeArgs& EA, bool ret = true, bool eval = true) {
-    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1;
+// no bytes it does not use, since resident CTAs per SM bound this latency-bound loop.  rec: the records the call asks for
+// (each of the four int32 diagnostics tiles only when its output is set; the profit tile when eval or profit_dev; the
+// state records need no tile), or NULL; all_rec: reserve every record tile (the module's upper bound).  Returns the total bytes.
+static int64_t episode_layout(const imx_env* e, EpisodeArgs& EA, bool ret = true, bool eval = true, const imx_records_out* rec = nullptr,
+                              bool all_rec = false) {
+    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1, cell4 = E * e->m * 4;
     int64_t off = e->tile_jit.total2;
     auto take = [&](int64_t bytes) { const int64_t o = off; off += (bytes + 127) & ~(int64_t)127; return (int32_t)(o < (1 << 30) ? o : 0); };
+    auto want = [&](const void* p) { return all_rec || (rec && p); };
     EA.off_edem = take(E * e->R * e->T * 4);
     EA.off_ret = take(ret ? E * cols * 8 : 0);
     EA.off_eval = take(eval ? E * (EVAL_FIXED + e->m) * 8 : 0);
-    EA.off_prof = take(eval ? E * e->m * 8 : 0);
+    EA.off_prof = take((eval || want(rec ? rec->profit_dev : nullptr)) ? E * e->m * 8 : 0);
+    EA.off_rdem = take(want(rec ? rec->demand_dev : nullptr) ? cell4 : 0);
+    EA.off_rship = take(want(rec ? rec->ship_dev : nullptr) ? cell4 : 0);
+    EA.off_racq = take(want(rec ? rec->acquisition_dev : nullptr) ? cell4 : 0);
+    EA.off_rord = take(want(rec ? rec->order_dev : nullptr) ? cell4 : 0);
     EA.total = (int32_t)(off < (1 << 30) ? off : 0);
     return off;
+}
+// The largest layout a module of `variant` launches with (its shared-memory attribute, and the 200 KB rule of its build).
+static int64_t episode_layout_max(const imx_env* e, int variant) {
+    EpisodeArgs EA;
+    return episode_layout(e, EA, true, true, nullptr, jit_has_rec(variant));
 }
 
 // Ring depth of the pipelined kernel for a given tile layout.  Measured shapes (profiles/r2_pipe_sweep.txt, r2_step_et_sweep.txt):
@@ -357,7 +377,7 @@ static int pipe_stages_for(const imx_env* e, const TileLayout& L) {
 // -D options, template instantiations and dynamic shared memory of one JitVariant's module (imx_jit.cuh).  The episode
 // variants hold the one-launch episode kernel only; the critic rows ride on the single-period kernels only.
 static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[imxjit::N_KERNELS]) {
-    const int has_obs = (variant != JIT_NOOBS && variant != JIT_EPISODE_NOOBS) ? 1 : 0, has_cc = variant == JIT_CC ? 1 : 0;
+    const int has_obs = jit_has_obs(variant) ? 1 : 0, has_cc = variant == JIT_CC ? 1 : 0;
     const int TL = e->TL;
     std::vector<std::string>& defs = sp.defines;
     const imx_config& c = e->cfg;
@@ -382,6 +402,7 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
     add("m_pow2", ((e->m & (e->m - 1)) == 0) ? 1 : 0);
     const TileLayout& L = has_cc ? e->tile_cc : e->tile_jit;
     add("has_cc", has_cc);
+    if (jit_has_rec(variant)) add("has_rec", 1);          // (absent from the other variants: their specifications stay as they were)
     auto addt = [&](const char* k, long long v) { defs.push_back(std::string("IMX_KT_") + k + "=" + std::to_string(v)); };
     addt("E", L.E); addt("off_act", L.off_act); addt("off_inv", L.off_inv); addt("off_bl", L.off_bl); addt("off_ou", L.off_ou);
     addt("off_pipe", L.off_pipe); addt("off_hd", L.off_hd); addt("off_ho", L.off_ho); addt("off_carry", L.off_carry);
@@ -499,13 +520,12 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
         sp.name[4] = "imx::step_kernel_tma_episode" + targs;
     }
     // (only the kernels the module holds take their size)
-    EpisodeArgs EA;
-    episode_layout(e, EA);
     smem[0] = L.total;
     smem[1] = L.total2 <= 200 * 1024 ? L.total2 : L.total;
     smem[2] = 0;
     smem[3] = (int)pipe_smem;
-    smem[4] = EA.total;
+    const int64_t ep_smem = episode_layout_max(e, variant);
+    smem[4] = (int)(ep_smem < (1 << 30) ? ep_smem : 0);
 }
 
 // Builds and loads one JitVariant of the specialised kernels, once per handle: a failed build is remembered and not retried.
@@ -522,8 +542,7 @@ static void ensure_jit(imx_env* e, int variant) {
         ensure_jit(e, JIT_STEP);                           // the other variants serve only where the step module does
         if (e->jit_state[JIT_STEP] != 1) return;
         if (variant == JIT_CC && (!e->multi || e->tile_cc.total > 200 * 1024)) return;
-        EpisodeArgs EA;
-        if (variant >= JIT_EPISODE && episode_layout(e, EA) > 200 * 1024) return;
+        if (variant >= JIT_EPISODE && episode_layout_max(e, variant) > 200 * 1024) return;
     }
     imxjit::Spec sp;
     int smem[imxjit::N_KERNELS];
@@ -1294,9 +1313,15 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
     }
     if ((flags & IMX_PREPARE_DFO) && !e->multi && !e->d_dfo_rewards)
         IMX_CUDA(cudaMalloc(&e->d_dfo_rewards, (size_t)e->T * e->N * sizeof(double)));
-    if (flags & IMX_PREPARE_EPISODE) {                     // both episode modules + every scratch buffer of the unfused form
+    if (flags & IMX_PREPARE_EPISODE) {                     // both episode modules
         ensure_jit(e, JIT_EPISODE);
         ensure_jit(e, JIT_EPISODE_NOOBS);
+    }
+    if (flags & IMX_PREPARE_RECORDS) {                     // both episode modules with records
+        ensure_jit(e, JIT_EPISODE_REC);
+        ensure_jit(e, JIT_EPISODE_REC_NOOBS);
+    }
+    if (flags & (IMX_PREPARE_EPISODE | IMX_PREPARE_RECORDS)) {   // + every scratch buffer of the unfused form
         const size_t cols = e->multi ? e->m : 1, cells = (size_t)e->N * e->m;
         if (!e->d_ep_rewards) IMX_CUDA(cudaMalloc(&e->d_ep_rewards, (size_t)e->T * e->N * cols * sizeof(double)));
         if (!e->d_ep_profit) IMX_CUDA(cudaMalloc(&e->d_ep_profit, cells * sizeof(double)));
@@ -1345,12 +1370,20 @@ extern "C" int imx_step_many(imx_env* e, const void* actions_dev, int K, void* o
 static int launch_return_stats(imx_env* e, const double* src, int periods, bool fused, double* ret_out, double* stats_dev, int accumulate,
                                cudaStream_t s);
 
-// A whole stored-plan episode: reset + T steps + returns / statistics / evaluation accumulators.  One launch of the episode
-// kernel (plus the two statistics launches over the returns) wherever the runtime-specialised build serves the whole batch
-// with one tile per CTA; otherwise the composition of the existing calls, with the same results.
+// A whole stored-plan episode: reset + T steps + returns / statistics / evaluation accumulators (+ per-period records).  One
+// launch of the episode kernel (plus the two statistics launches over the returns) wherever the runtime-specialised build
+// serves the whole batch with one tile per CTA; otherwise the composition of the existing calls, with the same results.
 extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
                                   const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
                                   double* stats_dev, int accumulate, double* eval_acc_dev, void* stream) {
+    return imx_replay_episode_records(e, demand_dev, delay_mask_dev, noisy, episode, actions_dev, obs_dev, reward_dev, return_dev,
+                                      stats_dev, accumulate, eval_acc_dev, nullptr, stream);
+}
+
+extern "C" int imx_replay_episode_records(imx_env* e, const int32_t* demand_dev, const uint8_t* delay_mask_dev, int noisy, uint64_t episode,
+                                          const double* actions_dev, void* obs_dev, double* reward_dev, double* return_dev,
+                                          double* stats_dev, int accumulate, double* eval_acc_dev, const imx_records_out* records,
+                                          void* stream) {
     IMX_NVTX("imx_replay_episode");
 
     if (!e || !actions_dev) return fail(-1, "null argument");
@@ -1363,20 +1396,34 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
     const int64_t N = e->N;
     const int m = e->m;
     const size_t cols = e->multi ? m : 1, cells = (size_t)N * m, es = obs_elem_bytes(e), aes = act_elem_bytes(e);
-    const imxjit::Kernels* jk = jit_module(e, obs_dev ? JIT_EPISODE : JIT_EPISODE_NOOBS, s);
+    const imx_records_out* rec = (records && (records->inv_dev || records->backlog_dev || records->order_u_dev || records->demand_dev ||
+                                              records->ship_dev || records->acquisition_dev || records->order_dev || records->profit_dev))
+                                     ? records : nullptr;
+    const int variant = rec ? (obs_dev ? JIT_EPISODE_REC : JIT_EPISODE_REC_NOOBS) : (obs_dev ? JIT_EPISODE : JIT_EPISODE_NOOBS);
+    // a records call under capture never silently takes the T-launch composition because its module was not loaded yet
+    if (rec && capturing && e->jit_state[variant] == 0)
+        return fail(-1, "imx_replay_episode_records under stream capture: call imx_prepare(IMX_PREPARE_RECORDS) first");
+    const imxjit::Kernels* jk = jit_module(e, variant, s);
     EpisodeArgs EA;
     memset(&EA, 0, sizeof(EA));
-    const int64_t smem = episode_layout(e, EA, return_dev || stats_dev, eval_acc_dev != nullptr);
+    const int64_t smem = episode_layout(e, EA, return_dev || stats_dev, eval_acc_dev != nullptr, rec);
     const int64_t E = e->tile_jit.E;
     const auto aligned16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
+    // records: every pointer 16-byte aligned and a tile's [E][m] int32 block a whole number of 16-byte units
+    const bool rec_legal = !rec || ((E * m * 4) % 16 == 0 && aligned16(rec->inv_dev) && aligned16(rec->backlog_dev) &&
+                                    aligned16(rec->order_u_dev) && aligned16(rec->demand_dev) && aligned16(rec->ship_dev) &&
+                                    aligned16(rec->acquisition_dev) && aligned16(rec->order_dev) && aligned16(rec->profit_dev));
     // the legality of imx_step_many's fused form (whole tiles, N % 4, 16-byte aligned buffers, a layout that fits), and the
     // replayed trace's per-tile block [E][R][T] must be a whole number of 16-byte units
     // divergent networks (measured, profiles/r3_replay_episode.jsonl): the episode kernel is ahead where the period body is the
     // env-per-thread one and observations are written (div2 +3 %), and where it is lane-mapped without observations (div1 +1 to
     // +6 %); in the other two cases its larger resident layout costs more than the bookkeeping it saves (div2 without observations
-    // -7 to -12 %, div1 with observations -6 % at 32 768 envs), so the composition serves them
-    const bool pays = !e->div || (e->step_et ? obs_dev != nullptr : obs_dev == nullptr);
-    const bool fused = pays && jk && jk->step_episode && e->step_path != 1 && e->fuse_periods && N % 4 == 0 && N % E == 0 && E % 2 == 0 &&
+    // -7 to -12 %, div1 with observations -6 % at 32 768 envs), so the composition serves them.  With records the composition
+    // is T launches of an ahead-of-time step kernel plus 3 T state copies, and the episode kernel measured 3.0-3.9 x ahead of it in
+    // those two cases (profiles/r3_replay_records.jsonl), so a call with records takes the episode kernel wherever it is legal
+    const bool pays = e->episode_fuse != 0 ? e->episode_fuse > 0
+                                           : (rec || !e->div || (e->step_et ? obs_dev != nullptr : obs_dev == nullptr));
+    const bool fused = pays && rec_legal && jk && jk->step_episode && e->step_path != 1 && e->fuse_periods && N % 4 == 0 && N % E == 0 && E % 2 == 0 &&
                        smem <= 200 * 1024 && tile_io_whole16(e, e->tile_jit, false) && aligned16(actions_dev) && aligned16(obs_dev) && aligned16(reward_dev) && aligned16(return_dev) &&
                        aligned16(eval_acc_dev) && (!demand_dev || (aligned16(demand_dev) && (E * e->R * e->T) % 4 == 0));
     // internal buffers are allocated here (never under capture: imx_prepare(IMX_PREPARE_EPISODE) allocates them up front),
@@ -1412,6 +1459,7 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
         EA.gen = make_gen(e, episode);
         EA.delay_thr = e->cfg.noisy_delay_threshold;
         EA.rescaled = (e->cfg.kind == IMX_KIND_MAIM_DIV || e->cfg.standardise_state) ? 1 : 0;
+        if (rec) EA.rec = *rec;
         void* params[] = {(void*)&A, (void*)&e->tile_jit, (void*)&EA};
         const CUresult cr = launch_dependent_jit(jk->step_episode, (unsigned)(N / E), (unsigned)e->jit_threads, (unsigned)smem, s, e->use_pdl, params);
         if (cr != CUDA_SUCCESS) return fail(-3, "launch of the episode kernel failed (CUresult %d)", (int)cr);
@@ -1421,13 +1469,13 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
         e->noisy_now = A.noisy;
         return stats_dev ? launch_return_stats(e, ret, 1, false, nullptr, stats_dev, accumulate, s) : 0;
     }
-    // the composition: imx_reset + imx_step_many (per-period steps with the profit diagnostics when the accumulators are
-    // wanted) + imx_episode_stats
+    // the composition: imx_reset + imx_step_many (per-period steps with the diagnostics when the accumulators or the records are
+    // wanted, the state fields copied into their record rows after the reset and after every step) + imx_episode_stats
     double* rew = reward_dev;
     if (!rew && (rc = scratch((void**)&e->d_ep_rewards, (size_t)e->T * N * cols * sizeof(double)))) return rc;
     if (!rew) rew = e->d_ep_rewards;
     if (eval_acc_dev) {
-        if ((rc = scratch((void**)&e->d_ep_profit, cells * sizeof(double)))) return rc;
+        if (!(rec && rec->profit_dev) && (rc = scratch((void**)&e->d_ep_profit, cells * sizeof(double)))) return rc;
         if (!obs_dev && (rc = scratch(&e->d_obs_scratch, cells * e->O * es))) return rc;
     }
     double* st = stats_dev;
@@ -1438,16 +1486,34 @@ extern "C" int imx_replay_episode(imx_env* e, const int32_t* demand_dev, const u
     }
     if ((rc = imx_reset(e, demand_dev, delay_mask_dev, noisy, episode, nullptr, stream))) return rc;
     const size_t rstride = (size_t)N * cols;
-    if (!eval_acc_dev) {
+    // state records: row `row` of each requested [T+1][N][m] block <- the handle's state field (same stream, device to device)
+    auto copy_state = [&](int row) -> int {
+        int32_t* dst[3] = {rec->inv_dev, rec->backlog_dev, rec->order_u_dev};
+        const int field[3] = {IMX_F_INV, IMX_F_BACKLOG, IMX_F_ORDER_U};
+        for (int k = 0; k < 3; ++k)
+            if (dst[k]) IMX_CUDA(cudaMemcpyAsync(dst[k] + (size_t)row * cells, e->field_ptr[field[k]], cells * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+        return 0;
+    };
+    if (!eval_acc_dev && !rec) {
         if ((rc = imx_step_many(e, actions_dev, e->T, obs_dev, rew, nullptr, stream))) return rc;
     } else {
+        if (rec && (rc = copy_state(0))) return rc;
         for (int t = 0; t < e->T; ++t) {
+            const size_t row = (size_t)t * cells;
             imx_info_out info;
             memset(&info, 0, sizeof(info));
-            info.profit_dev = e->d_ep_profit;
-            void* ob = obs_dev ? (void*)((unsigned char*)obs_dev + (size_t)t * cells * e->O * es) : e->d_obs_scratch;
+            if (rec) {
+                info.demand_dev = rec->demand_dev ? rec->demand_dev + row : nullptr;
+                info.ship_dev = rec->ship_dev ? rec->ship_dev + row : nullptr;
+                info.acquisition_dev = rec->acquisition_dev ? rec->acquisition_dev + row : nullptr;
+                info.order_dev = rec->order_dev ? rec->order_dev + row : nullptr;
+                info.profit_dev = rec->profit_dev ? rec->profit_dev + row : nullptr;
+            }
+            if (eval_acc_dev && !info.profit_dev) info.profit_dev = e->d_ep_profit;
+            void* ob = obs_dev ? (void*)((unsigned char*)obs_dev + (size_t)t * cells * e->O * es) : eval_acc_dev ? e->d_obs_scratch : nullptr;
             if ((rc = launch_step(e, (const unsigned char*)actions_dev + (size_t)t * cells * aes, (double*)ob, rew + (size_t)t * rstride, &info, s))) return rc;
-            if ((rc = imx_eval_accumulate(e, ob, rew + (size_t)t * rstride, e->d_ep_profit, eval_acc_dev, t == 0, stream))) return rc;
+            if (eval_acc_dev && (rc = imx_eval_accumulate(e, ob, rew + (size_t)t * rstride, info.profit_dev, eval_acc_dev, t == 0, stream))) return rc;
+            if (rec && (rc = copy_state(t + 1))) return rc;
         }
     }
     if (st) return imx_episode_stats(e, rew, e->T, return_dev, st, accumulate, stream);
@@ -1722,8 +1788,9 @@ extern "C" const char* imx_jit_log(void) { return imxjit::g_last_log.c_str(); }
 
 extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap) {
     if (!cfg) return fail(-1, "null argument");
-    if (variant < 0 || variant > 4)
-        return fail(-1, "variant must be 0 (step), 1 (no observations), 2 (critic rows), 3 (episode) or 4 (episode without observations)");
+    if (variant < 0 || variant >= JIT_VARIANTS)
+        return fail(-1, "variant must be 0 (step), 1 (no observations), 2 (critic rows), 3 (episode), 4 (episode without observations), "
+                        "5 (episode with records) or 6 (episode with records, without observations)");
     imx_env tmp;
     tmp.cfg = *cfg;
     const int rc = derive(&tmp);
@@ -1731,8 +1798,7 @@ extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* l
     plan_handle(&tmp, 148, 0);
     build_tables(&tmp, &tmp.TL);
     if (variant == JIT_CC && !tmp.multi) return fail(-1, "the critic rows exist for the multi-agent kinds only");
-    EpisodeArgs EA;
-    if (variant >= JIT_EPISODE && episode_layout(&tmp, EA) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
+    if (variant >= JIT_EPISODE && episode_layout_max(&tmp, variant) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
     imxjit::Spec sp;
     int smem[imxjit::N_KERNELS];
     jit_spec(&tmp, variant, sp, smem);

@@ -39,6 +39,14 @@ struct TileLayout {
     int32_t off_cc;            // centralised-critic rows [E][m][W] (layouts built for imx_step_cc only; inside `total`)
 };
 
+// Per-period records of the episode kernel (imx_replay_episode_records): a compile-time flag of the specialised build, so the
+// episode modules without records (IMX_K_has_rec undefined) contain none of this code.
+#if defined(IMX_JIT) && defined(IMX_K_has_rec) && IMX_K_has_rec
+#define IMX_REC 1
+#else
+#define IMX_REC 0
+#endif
+
 // One whole stored-plan episode per launch (imx_replay_episode, step_kernel_tma_episode): what the kernel needs beyond the
 // multi-period StepArgs.  The episode regions of shared memory sit behind TileLayout.total2 (the per-period demand rows of
 // that layout are unused: the episode's whole trace is resident instead).
@@ -52,9 +60,13 @@ struct EpisodeArgs {
     int32_t off_edem;                     // [E][R][T] int32 demand of the tile's envs
     int32_t off_ret;                      // [E][m] / [E] float64 returns
     int32_t off_eval;                     // [E][4 + m] float64 accumulators
-    int32_t off_prof;                     // [E][m] float64 profits of the current period (eval only)
+    int32_t off_prof;                     // [E][m] float64 profits of the current period (eval or records.profit_dev)
     int32_t total;                        // dynamic shared memory bytes
     int32_t rescaled;                     // the state is standardised: the accumulators undo the scaling (rev_scale)
+    // records (modules with IMX_K_has_rec only): [E][m] int32 tiles of the period's demand / ship / acquisition / order, each
+    // reserved only when its output is asked for; the state rows are stored straight from the state tiles
+    int32_t off_rdem, off_rship, off_racq, off_rord;
+    imx_records_out rec;                  // [T+1][N][m] state rows, [T][N][m] per-period rows; NULL fields are not recorded
 };
 
 // Noisy-delay outcome of (local env n, node i, period t) in an episode launch: the replayed mask, or the draw
@@ -189,6 +201,7 @@ struct TileSmem {
     double* rew;                // [E][m] / [E] reward tile
     double* prof;               // [E][m] profits of the period, or null (episode kernel with evaluation accumulators)
     double* ret;                // [E][m] / [E] episode returns, or null (episode kernel): reward added in place, period by period
+    int32_t *rdem, *rship, *racq, *rord;   // [E][m] record tiles of the period's demand / ship / acquisition / order, or null
 };
 
 // Per-thread constants of the lanes = stages mapping.
@@ -413,6 +426,12 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
         if (KF(multi)) S.rew[cell] = reward_out;
         else if (i == 0) S.rew[e_loc] = reward_out;
         if (EP && S.prof) S.prof[cell] = profit;
+        if (EP && IMX_REC) {                         // records: the period's diagnostics into their tiles (stored by the caller)
+            if (S.rdem) S.rdem[cell] = demand;
+            if (S.rship) S.rship[cell] = ship;
+            if (S.racq) S.racq[cell] = acq;
+            if (S.rord) S.rord[cell] = order;
+        }
         if (EP && S.ret) {                           // stats_slice_kernel<true>'s order: from 0, period by period
             if (KF(multi)) S.ret[cell] = __dadd_rn(S.ret[cell], reward_out);
             else if (i == 0) S.ret[e_loc] = __dadd_rn(S.ret[e_loc], reward_out);
@@ -684,6 +703,12 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
         }
         if (KF(multi)) S.rew[c0 + j] = reward[j];
         if (EP && S.prof) S.prof[c0 + j] = profit[j];
+        if (EP && IMX_REC) {                         // records, as in tile_period
+            if (S.rdem) S.rdem[c0 + j] = demand[j];
+            if (S.rship) S.rship[c0 + j] = ship[j];
+            if (S.racq) S.racq[c0 + j] = acq[j];
+            if (S.rord) S.rord[c0 + j] = order[j];
+        }
         if (KHAS(obs)) {
             NodeParams np;                           // the integer maxima write_obs_row scales with (compile-time values)
             np.inv_max = INV_MAX[j]; np.order_max = ORDER_MAX[j]; np.demand_max = DEMAND_MAX[j];
@@ -768,6 +793,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     const bool ok = i < m && sub < EPW;               // full tiles only: every env slot is live
     const int64_t n0 = (int64_t)blockIdx.x * E;      // first env of the tile
     const int K = MANY ? A.periods : 1;              // periods this launch advances
+    constexpr bool REC = EPISODE && IMX_REC;         // the episode kernel streams out per-period records
 
     int32_t* s_inv = reinterpret_cast<int32_t*>(smem + KT(off_inv));
     int32_t* s_bl = reinterpret_cast<int32_t*>(smem + KT(off_bl));
@@ -861,7 +887,15 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
                 if (2 * p + 1 < KF(T)) s_d[er * KF(T) + 2 * p + 1] = d1;
             }
         }
+        if (REC) fence_proxy_async_smem();          // the reset state is row 0 of the state records
         __syncthreads();
+        if (REC && tid == 0) {
+            const imx_records_out& R = EA->rec;
+            if (R.inv_dev) bulk_store_only(R.inv_dev + n0 * m, s_inv, b_cell4);
+            if (R.backlog_dev) bulk_store_only(R.backlog_dev + n0 * m, s_bl, b_cell4);
+            if (R.order_u_dev) bulk_store_only(R.order_u_dev + n0 * m, s_ou, b_cell4);
+            bulk_commit();
+        }
     }
 
     for (int j = 0; j < K; ++j) {
@@ -877,11 +911,19 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
 
     mbar_wait(&bar[b], (uint32_t)((j >> 1) & 1));
 
+    auto rec_tile = [&](const void* out, int32_t off) { return (REC && out) ? reinterpret_cast<int32_t*>(smem + off) : nullptr; };
     const TileSmem S = {s_act, EPISODE ? reinterpret_cast<const int32_t*>(smem + EA->off_edem) : s_dem, s_inv, s_bl, s_ou, s_pipe, s_hd,
-                        s_ho, s_carry, s_bt, s_obs, s_rew, (EPISODE && EA->eval) ? reinterpret_cast<double*>(smem + EA->off_prof) : nullptr,
-                        (EPISODE && EA->ret) ? reinterpret_cast<double*>(smem + EA->off_ret) : nullptr};
+                        s_ho, s_carry, s_bt, s_obs, s_rew,
+                        (EPISODE && (EA->eval || (REC && EA->rec.profit_dev))) ? reinterpret_cast<double*>(smem + EA->off_prof) : nullptr,
+                        (EPISODE && EA->ret) ? reinterpret_cast<double*>(smem + EA->off_ret) : nullptr,
+                        REC ? rec_tile(EA->rec.demand_dev, EA->off_rdem) : nullptr, REC ? rec_tile(EA->rec.ship_dev, EA->off_rship) : nullptr,
+                        REC ? rec_tile(EA->rec.acquisition_dev, EA->off_racq) : nullptr, REC ? rec_tile(EA->rec.order_dev, EA->off_rord) : nullptr};
+    // The state tiles are rewritten in place, and with records they are also the source of bulk stores (row 0 from the
+    // prologue, row t + 1 after period t), as are the record and profit tiles.  tile_period / tile_period_et write all of them
+    // only after this hook, whose bulk_wait_read_all drains every earlier bulk read of the tile: keep it that way.  Period 0
+    // waits too when records are on (the prologue's row-0 stores read the state tiles).
     auto before_store = [&]() {
-        if (MANY && j > 0) {                         // the previous period's stores must be done reading the output buffer
+        if (MANY && (j > 0 || REC)) {                // the previous period's stores must be done reading the output buffer
             if (tid == 0) bulk_wait_read_all();
             __syncthreads();
         }
@@ -909,6 +951,18 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
             if (KF(need_ho)) bulk_store_only(A.hist_o + n0 * m * KF(P), s_ho, b_hist);
             if (KF(has_carry)) bulk_store_only(A.carry + n0 * m, s_carry, b_cell4);
             if (DIV && KF(NB) > 0) bulk_store_only(A.bt + n0 * KF(NB), s_bt, b_bt);
+        }
+        if (REC) {                     // records of period t: the diagnostics to row t, the state after it to row t + 1
+            const imx_records_out& R = EA->rec;
+            const int64_t row = ((int64_t)j * A.N + n0) * m, row1 = row + A.N * m;
+            if (R.demand_dev) bulk_store_only(R.demand_dev + row, smem + EA->off_rdem, b_cell4);
+            if (R.ship_dev) bulk_store_only(R.ship_dev + row, smem + EA->off_rship, b_cell4);
+            if (R.acquisition_dev) bulk_store_only(R.acquisition_dev + row, smem + EA->off_racq, b_cell4);
+            if (R.order_dev) bulk_store_only(R.order_dev + row, smem + EA->off_rord, b_cell4);
+            if (R.profit_dev) bulk_store_only(R.profit_dev + row, smem + EA->off_prof, b_cell8);
+            if (R.inv_dev) bulk_store_only(R.inv_dev + row1, s_inv, b_cell4);
+            if (R.backlog_dev) bulk_store_only(R.backlog_dev + row1, s_bl, b_cell4);
+            if (R.order_u_dev) bulk_store_only(R.order_u_dev + row1, s_ou, b_cell4);
         }
         bulk_commit();
         if (j + 2 < K) {               // input buffer b is free again: fetch the inputs of period j + 2

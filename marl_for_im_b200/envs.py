@@ -651,8 +651,14 @@ class _ImxEnvBase:
             return obs_out, reward_out, self._shape_done(done), info
         return obs_out, reward_out, (self._shape_done(done))
 
+    # replay_episode(records=...): name -> (C field of imx_records_out, state block with T + 1 rows, dtype)
+    RECORD_FIELDS = {"inv": ("inv_dev", True, torch.int32), "backlog": ("backlog_dev", True, torch.int32),
+                     "order_u": ("order_u_dev", True, torch.int32), "demand": ("demand_dev", False, torch.int32),
+                     "ship": ("ship_dev", False, torch.int32), "acquisition": ("acquisition_dev", False, torch.int32),
+                     "order_r": ("order_dev", False, torch.int32), "profit": ("profit_dev", False, torch.float64)}
+
     def replay_episode(self, actions, customer_demand=None, delay_mask=None, noisy_delay=None, want_obs=False, want_rewards=False,
-                       returns=True, stats=None, accumulate=False, eval_acc=False):
+                       returns=True, stats=None, accumulate=False, eval_acc=False, records=False):
         """A whole episode on a stored plan ``actions [T, N, m]``: ``reset(customer_demand)`` + T ``step()`` calls + the episode's
         returns, statistics and evaluation-loop accumulators (the LP scripts' replay loop, DSHLP_4.py:896-928) in one call —
         one kernel launch where the batch allows it, without materialising per-period rewards or observations unless asked.
@@ -660,12 +666,27 @@ class _ImxEnvBase:
         customer_demand: [N, R, T] / [N, T] / one trace, or None (Philox, the stream ``reset()`` draws from).  Noisy delays follow
         the env's sticky ``noisy_delay`` flag unless ``noisy_delay`` is given; ``delay_mask`` replays them ([N, T, m] / [T, m]).
         stats: None (not wanted), True (a new vector) or a float64 tensor ``[3 (+ 2m)]`` to write, or with ``accumulate=True``
-        to add into.  Returns ``dict(returns, stats, obs [T, N, m, O], rewards [T, N(, m)], eval [N, 4 + m])`` with None for
+        to add into.  Returns ``dict(returns, stats, obs [T, N, m, O], rewards [T, N(, m)], eval [N, 4 + m], records)`` with None for
         what was not asked; ``eval`` is what ``eval_accumulate`` builds over the episode (``eval_stats`` / ``eval_summary``
-        take it as is).  Leaves the env at period T with the final state."""
+        take it as is).  Leaves the env at period T with the final state.
+
+        records: False, True (every field) or an iterable of names — the reference's history arrays of every env, under the
+        reference's attribute names: ``inv, backlog, order_u`` [T + 1, N, m] int32 (row 0 = the reset state, row t + 1 = the
+        state after period t), ``demand, ship, acquisition, order_r`` [T, N, m] int32 and ``profit`` [T, N, m] float64 (the
+        LP replay loop's per-period records, DSHLP_4.py:918-923).  They come back as ``records``, a dict with None for the
+        fields not asked for (None when records=False)."""
         if not self.batched:
             raise _lib.ImxError("replay_episode is a batched-mode call (construct the env with num_envs=N)")
         N, m, O, T = self.num_envs, self.num_nodes, self.obs_len, self.num_periods
+        if records is True:
+            wanted = set(self.RECORD_FIELDS)
+        elif records is False or records is None:
+            wanted = None
+        else:
+            wanted = set([records] if isinstance(records, str) else records)
+            unknown = wanted - set(self.RECORD_FIELDS)
+            if unknown:
+                raise ValueError(f"unknown record fields {sorted(unknown)}; known: {list(self.RECORD_FIELDS)}")
         act = actions if isinstance(actions, torch.Tensor) else torch.as_tensor(np.asarray(actions, dtype=np.float64))
         act = act.to(device=self.device, dtype=self.action_dtype)
         if act.numel() != T * N * m:
@@ -691,17 +712,24 @@ class _ImxEnvBase:
         if stats is not None and (stats.dtype != torch.float64 or not stats.is_contiguous() or stats.numel() != 3 + (2 * m if self.MULTI else 0)):
             raise ValueError("stats must be a contiguous float64 tensor of 3 (+ 2m for the multi-agent kinds) entries")
         ev = torch.empty((N, 4 + m), **f64) if eval_acc else None
+        recs, rec_struct = None, None
+        if wanted is not None:
+            recs = {k: (torch.empty((T + 1 if state else T, N, m), dtype=dt, device=self.device) if k in wanted else None)
+                    for k, (_, state, dt) in self.RECORD_FIELDS.items()}
+            rec_struct = _lib.ImxRecordsOut(**{f: (recs[k].data_ptr() if recs[k] is not None else None)
+                                               for k, (f, _, _) in self.RECORD_FIELDS.items()})
         self._episode += 1
         p = lambda x: C.c_void_p(x.data_ptr()) if x is not None else None   # noqa: E731
-        _lib.check(self._lib.imx_replay_episode(self._handle, p(demand_dev), p(mask_dev), int(want_noisy), self._episode, p(act),
-                                                p(obs), p(rew), p(ret), p(stats), int(bool(accumulate)), p(ev), self._stream()))
+        _lib.check(self._lib.imx_replay_episode_records(self._handle, p(demand_dev), p(mask_dev), int(want_noisy), self._episode, p(act),
+                                                        p(obs), p(rew), p(ret), p(stats), int(bool(accumulate)), p(ev),
+                                                        C.byref(rec_struct) if rec_struct is not None else None, self._stream()))
         self._keepalive = (act, demand_dev, mask_dev)
         if obs is not None:
             self.last_obs = obs[T - 1]
             self.state = self._shape_obs(obs[T - 1])
         if rew is not None:
             self.last_reward = rew[T - 1]
-        return {"returns": ret, "stats": stats, "obs": obs, "rewards": rew, "eval": ev}
+        return {"returns": ret, "stats": stats, "obs": obs, "rewards": rew, "eval": ev, "records": recs}
 
     # ------------------------------------------------------------------ drop-in mode histories
     def _alloc_histories(self):

@@ -4,8 +4,9 @@ episode, so no Python runs between the launches (a plain Python loop is host-bou
 kernel, see benchmarks/bench_python_loop.py).
 
 The "policy" here is a stand-in (a per-agent linear map of the observation squashed to [-1, 1]); swap in any module
-whose forward is graph-capturable.  Prints one JSON line.  Measured on a B200 at 65 536 envs: 22 us per period, of which
-the env step is 5 us — the four small torch kernels of the stand-in policy are the rest.
+whose forward is graph-capturable.  The returns are added up by the step launch itself (env.step_eval).  Prints one JSON
+line.  Measured on a B200 (1000 W power limit, 1965 MHz max SM clock) at 65 536 envs: 20.1 us per period, of which the env
+step with the returns measured 6.5 us with float64 observations (profiles/r3_step_eval.jsonl) — the four small torch kernels of the stand-in policy are the rest.
 
     python examples/rl_loop_cuda_graph.py [--envs 65536] [--episodes 20]
 """
@@ -18,7 +19,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 import torch  # noqa: E402
 
-from marl_for_im_b200 import presets  # noqa: E402
+from marl_for_im_b200 import _lib, presets  # noqa: E402
 from marl_for_im_b200.envs import MultiAgentInvManagement  # noqa: E402
 
 
@@ -34,15 +35,15 @@ def main():
     torch.manual_seed(0)
     w = torch.randn((m, O), device=dev) * 0.3                       # one weight vector per agent
     actions = torch.empty((N, m), dtype=torch.float64, device=dev)   # the graph's action buffer
-    returns = torch.zeros((N, m), dtype=torch.float64, device=dev)
+    returns = torch.zeros((N, m), dtype=torch.float64, device=dev)   # step_eval restarts it at period 0
+    _lib.check(env._lib.imx_prepare(env._handle, _lib.PREPARE_EVAL))  # its kernels are loaded before the capture
 
     env.reset()
     obs = env.last_obs                                               # the reused [N, m, O] float32 output buffer
 
     def period():
         actions.copy_(torch.tanh(torch.einsum("nmo,mo->nm", obs, w)))   # policy forward -> actions (float32 -> float64 buffer)
-        env.step_packed(actions)                                     # one launch; writes the reused obs / reward buffers
-        returns.add_(env.last_reward)
+        env.step_eval(actions, returns=returns, want_rewards=False)  # one launch: the reused obs buffer + the returns
 
     # warm up on a side stream (module loads, allocator), then capture.  An imx_step launch carries its period index
     # (it selects the demand row), so the periods are captured in order, all T of them in one graph.
@@ -54,13 +55,12 @@ def main():
     torch.cuda.current_stream().wait_stream(s)
     env.reset()
     g = torch.cuda.CUDAGraph()
-    with torch.cuda.graph(g):                                        # the whole episode: T x (policy, step, return accumulation)
+    with torch.cuda.graph(g):                                        # the whole episode: T x (policy, step with return accumulation)
         for t in range(T):
             period()
 
     def episode_exact():
         env.reset()                                                  # fresh Philox demand drawn on the device
-        returns.zero_()
         g.replay()
         env._lib.imx_set_period(env._handle, T)                      # host-side period counter (a replay does not advance it)
 
@@ -73,7 +73,7 @@ def main():
     e1.record()
     torch.cuda.synchronize()
     dt = e0.elapsed_time(e1) * 1e-3 / args.episodes
-    print(json.dumps({"case": "T x (policy forward + env.step + return accumulation) captured as one CUDA graph, float32 observations",
+    print(json.dumps({"case": "T x (policy forward + env.step_eval with the returns) captured as one CUDA graph, float32 observations",
                       "envs": N, "ms_per_episode": dt * 1e3, "us_per_period": dt / T * 1e6,
                       "agent_steps_per_sec": N * m * T / dt, "mean_return": float(returns.sum(-1).mean().item())}))
 

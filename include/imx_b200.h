@@ -44,7 +44,9 @@
 extern "C" {
 #endif
 
-#define IMX_ABI_VERSION 3     /* 3 (later, source-compatible): imx_records_out, imx_replay_episode_records, IMX_PREPARE_RECORDS and
+#define IMX_ABI_VERSION 3     /* 3 (later, source-compatible): imx_step_eval, IMX_PREPARE_EVAL and imx_jit_compile_check variants 8 / 9
+                                 (the step kernels with returns, evaluation accumulators and diagnostics; 7 is not assigned).
+                                 3 (later, source-compatible): imx_records_out, imx_replay_episode_records, IMX_PREPARE_RECORDS and
                                  imx_jit_compile_check variants 5 / 6 (the episode kernel with per-period records).
                                  3 (later, source-compatible): imx_config.reserved0 became io_flags (bfloat16 observations, float32
                                  actions); action pointers are const void* (imx_replay_episode's keeps its spelling); imx_round_bf16.
@@ -173,11 +175,13 @@ int imx_destroy(imx_env* env);
  *          IMX_PREPARE_DFO (scratch of the dfo objective), IMX_PREPARE_CC (imx_step_cc's specialisation and scratch),
  *          IMX_PREPARE_EPISODE (imx_replay_episode's two episode kernels, with and without observations, and the scratch
  *          buffers of its unfused form: [T][N](m) rewards, [N][m][O] observations, [N][m] profits, [N](m) returns),
- *          IMX_PREPARE_RECORDS (imx_replay_episode_records' two episode kernels with records and the same scratch buffers);
- *          0 = the first five (STEP | NOOBS | HOST | DFO | CC; not EPISODE or RECORDS, so existing callers compile nothing more).
+ *          IMX_PREPARE_RECORDS (imx_replay_episode_records' two episode kernels with records and the same scratch buffers),
+ *          IMX_PREPARE_EVAL (imx_step_eval's two modules, with and without observations, and the scratch buffers of its
+ *          composition: [N](m) rewards, [N][m][O] observations, [N][m] profits);
+ *          0 = the first five (STEP | NOOBS | HOST | DFO | CC; not EPISODE, RECORDS or EVAL, so existing callers compile nothing more).
  *          Synchronous; may take seconds (NVRTC). */
 enum imx_prepare_flags { IMX_PREPARE_STEP = 1, IMX_PREPARE_NOOBS = 2, IMX_PREPARE_HOST = 4, IMX_PREPARE_DFO = 8, IMX_PREPARE_CC = 16,
-                         IMX_PREPARE_EPISODE = 32, IMX_PREPARE_RECORDS = 64 };
+                         IMX_PREPARE_EPISODE = 32, IMX_PREPARE_RECORDS = 64, IMX_PREPARE_EVAL = 128 };
 int imx_prepare(imx_env* env, int flags);
 
 /* Derived sizes: O (observation length per agent), S (int32 state words per env), R, L, NB. */
@@ -264,6 +268,27 @@ int imx_replay_episode_records(imx_env* env, const int32_t* demand_dev, const ui
                                double* stats_dev, int accumulate, double* eval_acc_dev, const imx_records_out* records,
                                void* stream);
 
+/* step(action) with the bookkeeping of a closed-loop evaluation period: the evaluation loops that drive the env with a policy
+ * reading each period's observation (MA_inv_management.py:517-587, inv_management.py:567-606, CC_inv_management.py:494-558), where
+ * every period is one launch anyway.  With t = imx_period(env) before the call, bit-identical to
+ *   imx_step(env, actions, obs', reward', info', s);    obs' / reward': the caller's buffers or library scratch; info': the caller's
+ *                                                       fields, plus the profits in scratch when eval_acc_dev is given and
+ *                                                       info->profit_dev is not
+ *   return[c] = (t == 0 ? 0.0 : return[c]) + reward'[c] for every cell, [N][m] (MAIM kinds) / [N] (IM kinds)  (so a reward of -0.0
+ *                                                       starts the return at +0.0, as in imx_episode_stats)
+ *   imx_eval_accumulate(env, obs', reward', profit', eval_acc_dev, t == 0, s);
+ * Period 0 starts the episode's returns and accumulators; after T calls on a stored plan's actions return_dev and eval_acc_dev
+ * hold what imx_replay_episode writes for that plan.  obs_dev, reward_dev, info (and any of its fields), return_dev and
+ * eval_acc_dev may each be NULL; actions_dev may not.  Errors as imx_step (-6 past the end of the episode).
+ * Where the runtime-specialised kernels serve the whole batch in whole tiles (imx_step's rules for them, 16-byte aligned buffers,
+ * E * m * 4 bytes per diagnostics tile a whole number of 16-byte units) this is ONE launch: the returns and accumulator tiles
+ * move with the state tiles, the diagnostics tiles are stored next to the observations, and imx_kernel_variant() returns 2
+ * (one tile per CTA) or 3 (pipelined).  Elsewhere the library runs the composition itself, and imx_kernel_variant() reports the
+ * kernel that served its imx_step (0 or 1 whenever the diagnostics or the accumulators are asked for).  Under stream capture call
+ * imx_prepare(IMX_PREPARE_EVAL) first; without it a call under capture returns an error and launches nothing. */
+int imx_step_eval(imx_env* env, const void* actions_dev, void* obs_dev, double* reward_dev, const imx_info_out* info,
+                  double* return_dev, double* eval_acc_dev, void* stream);
+
 /* dfo_func's loop  —  base_restock_policy.py:24-45 with base_stock_policy :4-21 fused in: a whole
  * K = T period episode per env in ONE kernel, state on chip.
  *   z_dev          base-stock levels, [m] (z_stride = 0) or [N][m] (z_stride = m)
@@ -349,7 +374,8 @@ int imx_poisson_cdf(const imx_env* env, double* out, int cap);
 
 /* Which kernel served the last step()/rollout of this handle: 0 ahead-of-time direct kernel,
  * 1 ahead-of-time TMA-staged kernel, 2 runtime-specialised (NVRTC, same sources, flags as literals),
- * 3 runtime-specialised persistent pipeline (imx_step_pipe.cuh), 4 the one-launch episode kernel (imx_replay_episode). */
+ * 3 runtime-specialised persistent pipeline (imx_step_pipe.cuh), 4 the one-launch episode kernel (imx_replay_episode).
+ * imx_step_eval reports 2 / 3 for its specialised kernels, and its step's kernel on the composition. */
 int imx_kernel_variant(const imx_env* env);
 /* Last message of the runtime-specialisation layer (why it is unavailable, or a compile log). */
 const char* imx_jit_log(void);
@@ -357,7 +383,8 @@ const char* imx_jit_log(void);
  * cubin cache).  variant: 0 = the step / step_many / rollout / pipelined kernels, 1 = the same without observations
  * (obs_dev = NULL), 2 = with the centralised-critic rows (imx_step_cc), 3 = imx_replay_episode's episode kernel,
  * 4 = the same without observations, 5 = the episode kernel with records (imx_replay_episode_records), 6 = the same
- * without observations.
+ * without observations, 8 = the step and pipelined kernels with returns, accumulators and diagnostics (imx_step_eval), 9 = the
+ * same without observations (7 is not assigned and is refused).
  * Returns the cubin size in bytes, or a negative error; `log` receives the compiler log. */
 int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap);
 

@@ -14,6 +14,7 @@ KIND = {"IM": 0, "MAIM": 1, "IM_div": 2, "MAIM_div": 3}
 DIST = {"replay": 0, "custom": 0, "poisson": 1, "uniform": 2}
 PREPARE_EPISODE = 32    # IMX_PREPARE_EPISODE: imx_replay_episode's kernels and scratch (imx_prepare)
 PREPARE_RECORDS = 64    # IMX_PREPARE_RECORDS: imx_replay_episode_records' kernels and scratch (imx_prepare)
+PREPARE_EVAL = 128      # IMX_PREPARE_EVAL: imx_step_eval's kernels and scratch (imx_prepare)
 IO_OBS_BF16, IO_ACTIONS_F32 = 1, 2   # imx_config.io_flags: bfloat16 observations, float32 actions
 F_INV, F_BACKLOG, F_ORDER_U, F_PIPE, F_HIST_D, F_HIST_O, F_CARRY, F_BACKLOG_TO, F_ERROR, F_DEMAND, F_DELAY_MASK = range(11)
 
@@ -70,6 +71,7 @@ SYMBOLS = {
     "imx_reset": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P]),
     "imx_step": (C.c_int, [_P, _P, _P, _P, C.POINTER(ImxInfoOut), _P]),
     "imx_step_many": (C.c_int, [_P, _P, C.c_int, _P, _P, C.POINTER(ImxInfoOut), _P]),
+    "imx_step_eval": (C.c_int, [_P, _P, _P, _P, C.POINTER(ImxInfoOut), _P, _P, _P]),
     "imx_replay_episode": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, C.c_int, _P, _P]),
     "imx_replay_episode_records": (C.c_int, [_P, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, C.c_int, _P,
                                              C.POINTER(ImxRecordsOut), _P]),

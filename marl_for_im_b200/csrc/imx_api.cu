@@ -84,10 +84,17 @@ typedef void (*reset_fn_t)(const StepArgs, const ResetArgs, int);
 // step_many, rollout, pipelined); the same without the observation output (step / step_many with obs = NULL: scoring a stored
 // plan needs rewards only — the observation build and 60 % of the bytes fold away); the step with the centralised-critic rows
 // (imx_step_cc); the one-launch episode kernel (imx_replay_episode) with and without observations; the same with per-period
-// records (imx_replay_episode_records), with and without observations.
-enum JitVariant { JIT_STEP, JIT_NOOBS, JIT_CC, JIT_EPISODE, JIT_EPISODE_NOOBS, JIT_EPISODE_REC, JIT_EPISODE_REC_NOOBS, JIT_VARIANTS };
-static bool jit_has_obs(int variant) { return variant != JIT_NOOBS && variant != JIT_EPISODE_NOOBS && variant != JIT_EPISODE_REC_NOOBS; }
+// records (imx_replay_episode_records), with and without observations; the step and pipelined kernels with the period's
+// returns, accumulators and diagnostics (imx_step_eval), with and without observations.  Number 7 is not assigned: callers of
+// imx_jit_compile_check have always had it refused, and it stays refused.
+enum JitVariant { JIT_STEP, JIT_NOOBS, JIT_CC, JIT_EPISODE, JIT_EPISODE_NOOBS, JIT_EPISODE_REC, JIT_EPISODE_REC_NOOBS, JIT_UNASSIGNED_7,
+                  JIT_STEP_EVAL, JIT_STEP_EVAL_NOOBS, JIT_VARIANTS };
+static bool jit_has_obs(int variant) {
+    return variant != JIT_NOOBS && variant != JIT_EPISODE_NOOBS && variant != JIT_EPISODE_REC_NOOBS && variant != JIT_STEP_EVAL_NOOBS;
+}
 static bool jit_has_rec(int variant) { return variant == JIT_EPISODE_REC || variant == JIT_EPISODE_REC_NOOBS; }
+static bool jit_is_episode(int variant) { return variant >= JIT_EPISODE && variant <= JIT_EPISODE_REC_NOOBS; }
+static bool jit_has_eval(int variant) { return variant == JIT_STEP_EVAL || variant == JIT_STEP_EVAL_NOOBS; }
 
 struct imx_env {
     imx_config cfg;
@@ -155,6 +162,7 @@ struct imx_env {
     double* d_ep_profit = nullptr;       // [N][m] one period's profits (unfused imx_replay_episode with evaluation accumulators)
     double* d_ep_ret = nullptr;          // [N](m) returns of imx_replay_episode when only the statistics are wanted
     double* d_ep_stats = nullptr;        // [3 + 2m] statistics of the unfused imx_replay_episode when only the returns are wanted
+                                         // (imx_step_eval's composition: d_ep_ret holds one period's rewards, d_ep_profit its profits)
     int last_variant = 0;                // 0 AOT direct, 1 AOT TMA, 2 runtime-specialised TMA, 3 pipelined, 4 one-launch episode
     reset_fn_t reset_fn = nullptr;
     rollout_fn_t rollout_fn = nullptr;
@@ -364,6 +372,30 @@ static int64_t episode_layout_max(const imx_env* e, int variant) {
     return episode_layout(e, EA, true, true, nullptr, jit_has_rec(variant));
 }
 
+// Shared-memory layout of one tile of imx_step_eval's kernels: tile_jit's single-period layout, then the regions of StepEvalArgs
+// the call needs (none it does not use: resident CTAs and the ring depth follow from the stage size).  all: every region (the
+// module's upper bound).  Returns the total bytes.
+static int64_t step_eval_layout(const imx_env* e, StepEvalArgs& EV, bool all) {
+    const int64_t E = e->tile_jit.E, cols = e->multi ? e->m : 1, cell4 = E * e->m * 4;
+    int64_t off = e->tile_jit.total;
+    auto take = [&](bool want, int64_t bytes) { const int64_t o = off; if (want) off += (bytes + 127) & ~(int64_t)127; return (int32_t)(o < (1 << 30) ? o : 0); };
+    const imx_info_out& I = EV.info;
+    EV.off_ret = take(all || EV.ret, E * cols * 8);
+    EV.off_eval = take(all || EV.eval, E * (EVAL_FIXED + e->m) * 8);
+    EV.off_prof = take(all || EV.eval || I.profit_dev, E * e->m * 8);
+    EV.off_idem = take(all || I.demand_dev, cell4);
+    EV.off_iship = take(all || I.ship_dev, cell4);
+    EV.off_iacq = take(all || I.acquisition_dev, cell4);
+    EV.off_iord = take(all || I.order_dev, cell4);
+    EV.total = (int32_t)(off < (1 << 30) ? off : 0);
+    return off;
+}
+static int64_t step_eval_layout_max(const imx_env* e) {
+    StepEvalArgs EV;
+    memset(&EV, 0, sizeof(EV));
+    return step_eval_layout(e, EV, true);
+}
+
 // Ring depth of the pipelined kernel for a given tile layout.  Measured shapes (profiles/r2_pipe_sweep.txt, r2_step_et_sweep.txt):
 // four stages for the lane-mapped tiles, two for the env-per-thread tiles (their 32-env tiles are 2-3 x larger: a deeper ring
 // costs resident CTAs); the critic-row variant shortens its ring until four CTAs fit on an SM.
@@ -400,9 +432,13 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
     const double fr = std::frexp(c.b - c.a, &ex);
     add("bma_pow2", (fr == 0.5 && ex > -1000 && ex < 1000) ? 1 : 0);
     add("m_pow2", ((e->m & (e->m - 1)) == 0) ? 1 : 0);
-    const TileLayout& L = has_cc ? e->tile_cc : e->tile_jit;
+    // imx_step_eval's modules: the stage of the pipelined kernel is the tile with every bookkeeping region (its ring depth follows)
+    TileLayout L_eval = e->tile_jit;
+    L_eval.total = (int32_t)step_eval_layout_max(e);
+    const TileLayout& L = has_cc ? e->tile_cc : jit_has_eval(variant) ? L_eval : e->tile_jit;
     add("has_cc", has_cc);
     if (jit_has_rec(variant)) add("has_rec", 1);          // (absent from the other variants: their specifications stay as they were)
+    if (jit_has_eval(variant)) add("has_eval", 1);
     auto addt = [&](const char* k, long long v) { defs.push_back(std::string("IMX_KT_") + k + "=" + std::to_string(v)); };
     addt("E", L.E); addt("off_act", L.off_act); addt("off_inv", L.off_inv); addt("off_bl", L.off_bl); addt("off_ou", L.off_ou);
     addt("off_pipe", L.off_pipe); addt("off_hd", L.off_hd); addt("off_ho", L.off_ho); addt("off_carry", L.off_carry);
@@ -439,6 +475,7 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
     defs.push_back("IMX_HOST_SIZEOF_TILELAYOUT=" + std::to_string(sizeof(TileLayout)));
     defs.push_back("IMX_HOST_SIZEOF_ROLLOUTARGS=" + std::to_string(sizeof(RolloutArgs)));
     defs.push_back("IMX_HOST_SIZEOF_EPISODEARGS=" + std::to_string(sizeof(EpisodeArgs)));
+    if (jit_has_eval(variant)) defs.push_back("IMX_HOST_SIZEOF_STEPEVALARGS=" + std::to_string(sizeof(StepEvalArgs)));
     const int mp = m_pad_of(e);                            // step kernel: power-of-two tile width (see plan_handle)
     const int pmax = (e->need_hd || e->need_ho) ? e->P : 1;
     const int maxc = e->maxc > 1 ? e->maxc : 1;
@@ -506,7 +543,7 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
         sp.name[2] = "imx::rollout_kernel<" + std::to_string(e->m) + ", " + std::to_string(e->D) + ", " + std::to_string(e->div ? maxc : 1) +
                      ", " + dv + ">";
     sp.name[3] = "";
-    if (has_cc) { sp.name[1] = ""; sp.name[2] = ""; }
+    if (has_cc || jit_has_eval(variant)) { sp.name[1] = ""; sp.name[2] = ""; }
     const int64_t pipe_smem = (int64_t)pipe_stages_for(e, L) * L.total;
     if (e->pipe_mode >= 0 && pipe_smem <= 200 * 1024) {
         defs.push_back("IMX_PIPE_STAGES=" + std::to_string(pipe_stages_for(e, L)));
@@ -515,7 +552,7 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
         sp.name[3] = "imx::step_kernel_pipe" + targs;
     }
     sp.name[4] = "";
-    if (variant >= JIT_EPISODE) {
+    if (jit_is_episode(variant)) {
         for (int k = 0; k < 4; ++k) sp.name[k] = "";
         sp.name[4] = "imx::step_kernel_tma_episode" + targs;
     }
@@ -542,7 +579,8 @@ static void ensure_jit(imx_env* e, int variant) {
         ensure_jit(e, JIT_STEP);                           // the other variants serve only where the step module does
         if (e->jit_state[JIT_STEP] != 1) return;
         if (variant == JIT_CC && (!e->multi || e->tile_cc.total > 200 * 1024)) return;
-        if (variant >= JIT_EPISODE && episode_layout_max(e, variant) > 200 * 1024) return;
+        if (jit_is_episode(variant) && episode_layout_max(e, variant) > 200 * 1024) return;
+        if (jit_has_eval(variant) && step_eval_layout_max(e) > 200 * 1024) return;
     }
     imxjit::Spec sp;
     int smem[imxjit::N_KERNELS];
@@ -1297,6 +1335,122 @@ extern "C" int imx_step_cc(imx_env* e, const void* actions_dev, void* obs_dev, v
     return imx_cc_observe(e, obs, fill_actions ? actions_dev : nullptr, clip_lo, clip_hi, cc_dev, obs_type_of(e->cfg), stream);
 }
 
+// step() with the period's bookkeeping of a closed-loop evaluation: the returns, the evaluation-loop accumulators and the
+// diagnostics.  One launch of imx_step_eval's specialised kernels (one-tile or pipelined, as for the plain step) wherever the
+// whole batch sits in whole tiles of the specialised layout; otherwise the composition it is bit-identical to: imx_step (with
+// the profits in scratch when the accumulators want them), returns_add_kernel, imx_eval_accumulate.
+extern "C" int imx_step_eval(imx_env* e, const void* actions_dev, void* obs_dev, double* reward_dev, const imx_info_out* info,
+                             double* return_dev, double* eval_acc_dev, void* stream) {
+    IMX_NVTX("imx_step_eval");
+
+    if (!e || !actions_dev) return fail(-1, "null argument");
+    if (e->t >= e->T) return fail(-6, "step() past the end of the episode (period %d of %d)", e->t, e->T);
+    IMX_CUDA(cudaSetDevice(e->cfg.device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const bool capturing = stream_is_capturing(s);
+    const int64_t N = e->N;
+    const int m = e->m, t0 = e->t;
+    const size_t cols = e->multi ? m : 1, cells = (size_t)N * m;
+    imx_info_out I;
+    memset(&I, 0, sizeof(I));
+    if (info) I = *info;
+    const int variant = obs_dev ? JIT_STEP_EVAL : JIT_STEP_EVAL_NOOBS;
+    // under capture nothing compiles, and a module never tried does not silently hand the call to the composition
+    if (capturing && e->jit_state[variant] == 0)
+        return fail(-1, "imx_step_eval under stream capture: call imx_prepare(IMX_PREPARE_EVAL) first");
+    const imxjit::Kernels* jk = jit_module(e, variant, s);
+    StepEvalArgs EV;
+    memset(&EV, 0, sizeof(EV));
+    EV.ret = return_dev;
+    EV.eval = eval_acc_dev;
+    EV.info = I;
+    EV.rescaled = (e->cfg.kind == IMX_KIND_MAIM_DIV || e->cfg.standardise_state) ? 1 : 0;
+    const int64_t tile_bytes = step_eval_layout(e, EV, false);
+    const int64_t E = e->tile_jit.E;
+    const auto aligned16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
+    // the plain step's rules for the specialised kernels (whole tiles only, N % 4, 16-byte aligned buffers, whole 16-byte units per
+    // bulk copy: E * m * 4 bytes for a diagnostics tile, E * 8 for an IM kind's returns), plus every new pointer aligned
+    // measured (profiles/r3_step_eval.jsonl): with the returns as the only bookkeeping, the env-per-thread body (div2) on a launch
+    // that streams more than half of L2 (262 144 envs) ran as fast as (float64 observations) or 7 % slower than (bfloat16) the
+    // plain specialised step + the returns add, so the composition serves it; with accumulators or diagnostics, below that size
+    // and on the lane-mapped networks the fused kernels were ahead or level (DESIGN.md §3.13)
+    const bool returns_only = !eval_acc_dev && !(I.demand_dev || I.ship_dev || I.acquisition_dev || I.order_dev || I.profit_dev);
+    int l2_bytes = 0;
+    if (returns_only && e->step_et && cudaDeviceGetAttribute(&l2_bytes, cudaDevAttrL2CacheSize, e->cfg.device) != cudaSuccess) cudaGetLastError();
+    const bool pays = !(returns_only && e->step_et && bytes_per_env(e) * N > (int64_t)(l2_bytes > 0 ? l2_bytes : 126 << 20) / 2);
+    const bool fused = pays && jk && jk->step && e->step_path != 1 && N % 4 == 0 && N % E == 0 && E % 2 == 0 && (E * m * 4) % 16 == 0 &&
+                       tile_bytes <= 200 * 1024 && tile_io_whole16(e, e->tile_jit, false) && aligned16(actions_dev) && aligned16(obs_dev) &&
+                       aligned16(reward_dev) && aligned16(return_dev) && aligned16(eval_acc_dev) && aligned16(I.demand_dev) &&
+                       aligned16(I.ship_dev) && aligned16(I.acquisition_dev) && aligned16(I.order_dev) && aligned16(I.profit_dev);
+    if (fused) {
+        StepArgs A;
+        fill_args(e, A);
+        A.periods = 1;
+        A.act_stride = (int64_t)cells;
+        A.obs_stride_bytes = (int64_t)(cells * e->O * obs_elem_bytes(e));
+        A.rew_stride = (int64_t)(N * cols);
+        A.actions = actions_dev;
+        A.obs = (double*)obs_dev;
+        A.reward = reward_dev;
+        TileLayout TL = e->tile_jit;                        // (the kernels address the bookkeeping regions through EV)
+        PipeArgs PA;
+        PA.n_tiles = (int32_t)(N / E);
+        TileLayout TL_stage = e->tile_jit;
+        TL_stage.total = EV.total;
+        const bool pipe = jk->step_pipe && e->pipe_mode >= 0 && (e->pipe_mode == 1 || pipe_pays(e));
+        TileLayout TL_max = e->tile_jit;
+        TL_max.total = (int32_t)step_eval_layout_max(e);
+        PA.stages = pipe_stages_for(e, TL_max);            // = the module's IMX_PIPE_STAGES
+        void* params_tile[] = {(void*)&A, (void*)&TL, (void*)&EV};
+        void* params_pipe[] = {(void*)&A, (void*)&TL, (void*)&PA, (void*)&EV};
+        unsigned grid = (unsigned)PA.n_tiles, block = (unsigned)e->jit_threads, smem = (unsigned)EV.total;
+        if (pipe) {
+            const int64_t resident = (int64_t)e->sm_count * pipe_ctas_for(e, TL_stage);
+            grid = (unsigned)(PA.n_tiles < resident ? PA.n_tiles : resident);
+            block += 32;
+            smem = (unsigned)(PA.stages * EV.total);
+        }
+        const CUresult cr = launch_dependent_jit(pipe ? jk->step_pipe : jk->step, grid, block, smem, s, e->use_pdl, pipe ? params_pipe : params_tile);
+        if (cr != CUDA_SUCCESS) return fail(-3, "launch of the specialised step kernel with bookkeeping failed (CUresult %d)", (int)cr);
+        e->last_variant = pipe ? 3 : 2;
+        e->t += 1;
+        return 0;
+    }
+    // the composition; scratch for what the caller did not pass (allocated here, never under capture)
+    auto scratch = [&](void** p, size_t bytes) -> int {
+        if (*p) return 0;
+        if (capturing) return fail(-1, "imx_step_eval needs an internal buffer under stream capture: call imx_prepare(IMX_PREPARE_EVAL) first");
+        IMX_CUDA(cudaMalloc(p, bytes));
+        return 0;
+    };
+    int rc = 0;
+    double* rew = reward_dev;
+    if (!rew) {
+        if ((rc = scratch((void**)&e->d_ep_ret, (size_t)N * cols * sizeof(double)))) return rc;
+        rew = e->d_ep_ret;
+    }
+    void* ob = obs_dev;
+    if (eval_acc_dev) {
+        if (!ob) {
+            if ((rc = scratch(&e->d_obs_scratch, cells * e->O * obs_elem_bytes(e)))) return rc;
+            ob = e->d_obs_scratch;
+        }
+        if (!I.profit_dev) {
+            if ((rc = scratch((void**)&e->d_ep_profit, cells * sizeof(double)))) return rc;
+            I.profit_dev = e->d_ep_profit;
+        }
+    }
+    const bool any_info = I.demand_dev || I.ship_dev || I.acquisition_dev || I.order_dev || I.profit_dev;
+    if ((rc = launch_step(e, actions_dev, (double*)ob, rew, any_info ? &I : nullptr, s))) return rc;
+    if (return_dev) {
+        const int64_t n = N * (int64_t)cols;
+        returns_add_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(return_dev, rew, n, t0 == 0 ? 1 : 0);
+        IMX_CHECK_LAUNCH("returns_add_kernel");
+    }
+    if (eval_acc_dev) return imx_eval_accumulate(e, ob, rew, I.profit_dev, eval_acc_dev, t0 == 0, stream);
+    return 0;
+}
+
 static int ensure_host_path(imx_env* e);
 
 extern "C" int imx_prepare(imx_env* e, int flags) {
@@ -1320,6 +1474,14 @@ extern "C" int imx_prepare(imx_env* e, int flags) {
     if (flags & IMX_PREPARE_RECORDS) {                     // both episode modules with records
         ensure_jit(e, JIT_EPISODE_REC);
         ensure_jit(e, JIT_EPISODE_REC_NOOBS);
+    }
+    if (flags & IMX_PREPARE_EVAL) {                        // imx_step_eval's two modules + the scratch of its composition
+        ensure_jit(e, JIT_STEP_EVAL);
+        ensure_jit(e, JIT_STEP_EVAL_NOOBS);
+        const size_t cols = e->multi ? e->m : 1, cells = (size_t)e->N * e->m;
+        if (!e->d_ep_ret) IMX_CUDA(cudaMalloc(&e->d_ep_ret, (size_t)e->N * cols * sizeof(double)));
+        if (!e->d_ep_profit) IMX_CUDA(cudaMalloc(&e->d_ep_profit, cells * sizeof(double)));
+        if (!e->d_obs_scratch) IMX_CUDA(cudaMalloc(&e->d_obs_scratch, cells * e->O * obs_elem_bytes(e)));
     }
     if (flags & (IMX_PREPARE_EPISODE | IMX_PREPARE_RECORDS)) {   // + every scratch buffer of the unfused form
         const size_t cols = e->multi ? e->m : 1, cells = (size_t)e->N * e->m;
@@ -1788,9 +1950,10 @@ extern "C" const char* imx_jit_log(void) { return imxjit::g_last_log.c_str(); }
 
 extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* log, int cap) {
     if (!cfg) return fail(-1, "null argument");
-    if (variant < 0 || variant >= JIT_VARIANTS)
+    if (variant < 0 || variant >= JIT_VARIANTS || variant == JIT_UNASSIGNED_7)
         return fail(-1, "variant must be 0 (step), 1 (no observations), 2 (critic rows), 3 (episode), 4 (episode without observations), "
-                        "5 (episode with records) or 6 (episode with records, without observations)");
+                        "5 (episode with records), 6 (episode with records, without observations), 8 (step with returns, accumulators "
+                        "and diagnostics) or 9 (the same without observations)");
     imx_env tmp;
     tmp.cfg = *cfg;
     const int rc = derive(&tmp);
@@ -1798,7 +1961,8 @@ extern "C" int imx_jit_compile_check(const imx_config* cfg, int variant, char* l
     plan_handle(&tmp, 148, 0);
     build_tables(&tmp, &tmp.TL);
     if (variant == JIT_CC && !tmp.multi) return fail(-1, "the critic rows exist for the multi-agent kinds only");
-    if (variant >= JIT_EPISODE && episode_layout_max(&tmp, variant) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
+    if (jit_is_episode(variant) && episode_layout_max(&tmp, variant) > 200 * 1024) return fail(-1, "the episode kernel's layout exceeds 200 KB of shared memory");
+    if (jit_has_eval(variant) && step_eval_layout_max(&tmp) > 200 * 1024) return fail(-1, "the bookkeeping step's layout exceeds 200 KB of shared memory");
     imxjit::Spec sp;
     int smem[imxjit::N_KERNELS];
     jit_spec(&tmp, variant, sp, smem);

@@ -201,4 +201,11 @@ __global__ void __launch_bounds__(STATS_THREADS) stats_final_kernel(const double
     }
 }
 
+// imx_step_eval's composition: one period's rewards into the episode returns in stats_slice_kernel<true>'s order,
+// ret[k] = (fresh ? 0.0 : ret[k]) + rew[k] (fresh: period 0, so a reward of -0.0 starts the return at +0.0, as there).
+__global__ void __launch_bounds__(256) returns_add_kernel(double* __restrict__ ret, const double* __restrict__ rew, int64_t n, int fresh) {
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k < n) ret[k] = __dadd_rn(fresh ? 0.0 : ret[k], rew[k]);
+}
+
 }  // namespace imx

@@ -46,7 +46,7 @@ __device__ __forceinline__ void bulk_wait_read_but_one() { asm volatile("cp.asyn
 
 template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV>
 __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArgs A, const __grid_constant__ TileLayout TLY,
-                                                 const __grid_constant__ PipeArgs PA) {
+                                                 const __grid_constant__ PipeArgs PA IMX_EVAL_PARAM) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t full[PIPE_MAX_STAGES], done[PIPE_MAX_STAGES];
     constexpr int S = IMX_PIPE_STAGES;
@@ -56,6 +56,11 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     const int es = obs_elem_bytes(KF(obs_type));
     const int aes = KF(act_f32) ? 4 : 8;
     const int n_my = (PA.n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;   // tiles blockIdx.x, + gridDim.x, ...
+#if IMX_EVAL
+    const int32_t stage_bytes = EV.total;            // a stage reserves only the bookkeeping regions this call uses
+#else
+    constexpr int32_t stage_bytes = KT(total);
+#endif
 
     pdl_launch_dependents();
     if (tid == CT) {
@@ -74,6 +79,13 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     if (KF(need_ho)) b_in += b_hist;
     if (KF(has_carry)) b_in += b_cell4;
     if (DIV && KF(NB) > 0) b_in += b_bt;
+#if IMX_EVAL
+    const int cols = KF(multi) ? m : 1;
+    const uint32_t b_ret = (uint32_t)E * cols * 8u, b_eval = (uint32_t)E * (4 + m) * 8u;
+    const bool se_load = A.t > 0;                    // returns / accumulators continue the episode (period 0 starts them at 0.0)
+    if (se_load && EV.ret) b_in += b_ret;
+    if (se_load && EV.eval) b_in += b_eval;
+#endif
     auto first_env = [&](int k) { return ((int64_t)blockIdx.x + (int64_t)k * gridDim.x) * E; };
 #if defined(IMX_L2_HINTS) && IMX_L2_HINTS
     const uint64_t pol_stream = l2_policy_evict_first(), pol_keep = l2_policy_evict_last();
@@ -105,7 +117,7 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     };
     auto issue_loads = [&](int k) {
         const int s = k % S;
-        unsigned char* st = smem + (size_t)s * KT(total);
+        unsigned char* st = smem + (size_t)s * stage_bytes;
         const int64_t n0 = first_env(k);
         uint64_t* bar = &full[s];
         mbar_expect_tx(bar, b_in);
@@ -120,6 +132,10 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
         if (KF(need_ho)) PIPE_LOAD_KEEP(st + KT(off_ho), A.hist_o + n0 * m * KF(P), b_hist, bar);
         if (KF(has_carry)) PIPE_LOAD_KEEP(st + KT(off_carry), A.carry + n0 * m, b_cell4, bar);
         if (DIV && KF(NB) > 0) PIPE_LOAD_KEEP(st + KT(off_bt), A.bt + n0 * KF(NB), b_bt, bar);
+#if IMX_EVAL
+        if (se_load && EV.ret) PIPE_LOAD_KEEP(st + EV.off_ret, EV.ret + n0 * cols, b_ret, bar);
+        if (se_load && EV.eval) PIPE_LOAD_KEEP(st + EV.off_eval, EV.eval + n0 * (4 + m), b_eval, bar);
+#endif
     };
 
     // The first ring fill is the launch's critical path: one thread issuing S tiles x 7-10 bulk loads one after the other
@@ -133,11 +149,11 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
         // ---------------------------------------------------------------- producer ---------------------------------
         auto issue_stores = [&](int k) {
             const int s = k % S;
-            const unsigned char* st = smem + (size_t)s * KT(total);
+            const unsigned char* st = smem + (size_t)s * stage_bytes;
             const int64_t n0 = first_env(k);
             if (KHAS(cc)) PIPE_STORE_STREAM(reinterpret_cast<unsigned char*>(A.cc) + n0 * m * A.cc_W * es, st + KT(off_cc), (uint32_t)E * m * A.cc_W * es);
             if (KHAS(obs)) PIPE_STORE_STREAM(reinterpret_cast<unsigned char*>(A.obs) + n0 * m * O * es, st + KT(off_obs), (uint32_t)E * m * O * es);
-            PIPE_STORE_KEEP(A.reward + (KF(multi) ? n0 * m : n0), st + KT(off_rew), KF(multi) ? b_cell8 : (uint32_t)E * 8u);
+            if (!IMX_EVAL || A.reward) PIPE_STORE_KEEP(A.reward + (KF(multi) ? n0 * m : n0), st + KT(off_rew), KF(multi) ? b_cell8 : (uint32_t)E * 8u);
             PIPE_STORE_STATE(A.inv + n0 * m, st + KT(off_inv), b_cell4);
             PIPE_STORE_STATE(A.backlog + n0 * m, st + KT(off_bl), b_cell4);
             PIPE_STORE_STATE(A.order_u + n0 * m, st + KT(off_ou), b_cell4);
@@ -146,6 +162,16 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
             if (KF(need_ho)) PIPE_STORE_STATE(A.hist_o + n0 * m * KF(P), st + KT(off_ho), b_hist);
             if (KF(has_carry)) PIPE_STORE_STATE(A.carry + n0 * m, st + KT(off_carry), b_cell4);
             if (DIV && KF(NB) > 0) PIPE_STORE_STATE(A.bt + n0 * KF(NB), st + KT(off_bt), b_bt);
+#if IMX_EVAL
+            // returns and accumulators travel like state, the diagnostics like the observation stream (one commit group per tile)
+            if (EV.ret) PIPE_STORE_STATE(EV.ret + n0 * cols, st + EV.off_ret, b_ret);
+            if (EV.eval) PIPE_STORE_STATE(EV.eval + n0 * (4 + m), st + EV.off_eval, b_eval);
+            if (EV.info.demand_dev) PIPE_STORE_STREAM(EV.info.demand_dev + n0 * m, st + EV.off_idem, b_cell4);
+            if (EV.info.ship_dev) PIPE_STORE_STREAM(EV.info.ship_dev + n0 * m, st + EV.off_iship, b_cell4);
+            if (EV.info.acquisition_dev) PIPE_STORE_STREAM(EV.info.acquisition_dev + n0 * m, st + EV.off_iacq, b_cell4);
+            if (EV.info.order_dev) PIPE_STORE_STREAM(EV.info.order_dev + n0 * m, st + EV.off_iord, b_cell4);
+            if (EV.info.profit_dev) PIPE_STORE_STREAM(EV.info.profit_dev + n0 * m, st + EV.off_prof, b_cell8);
+#endif
             bulk_commit();
         };
         for (int k = 0; k < pre; k += NW) prefetch_inputs(k);
@@ -175,21 +201,39 @@ __global__ void IMX_PIPE_BOUNDS step_kernel_pipe(const __grid_constant__ StepArg
     // (prefetching the rescale table into L1 here was measured: 5.5 -> 8.3 us per launch at 65 536 envs, profiles/r2_act_prefetch_ab.txt)
     for (int k = 0; k < n_my; ++k) {
         const int s = k % S;
-        unsigned char* st = smem + (size_t)s * KT(total);
+        unsigned char* st = smem + (size_t)s * stage_bytes;
         const TileSmem T = {st + KT(off_act), reinterpret_cast<const int32_t*>(st + KT(off_dem)),
                             reinterpret_cast<int32_t*>(st + KT(off_inv)), reinterpret_cast<int32_t*>(st + KT(off_bl)),
                             reinterpret_cast<int32_t*>(st + KT(off_ou)), reinterpret_cast<int32_t*>(st + KT(off_pipe)),
                             reinterpret_cast<int32_t*>(st + KT(off_hd)), reinterpret_cast<int32_t*>(st + KT(off_ho)),
                             reinterpret_cast<int32_t*>(st + KT(off_carry)), reinterpret_cast<int32_t*>(st + KT(off_bt)),
-                            st + KT(off_obs), reinterpret_cast<double*>(st + KT(off_rew))};
+                            st + KT(off_obs), reinterpret_cast<double*>(st + KT(off_rew))
+#if IMX_EVAL
+                            , (EV.eval || EV.info.profit_dev) ? reinterpret_cast<double*>(st + EV.off_prof) : nullptr,
+                            EV.ret ? reinterpret_cast<double*>(st + EV.off_ret) : nullptr,
+                            EV.info.demand_dev ? reinterpret_cast<int32_t*>(st + EV.off_idem) : nullptr,
+                            EV.info.ship_dev ? reinterpret_cast<int32_t*>(st + EV.off_iship) : nullptr,
+                            EV.info.acquisition_dev ? reinterpret_cast<int32_t*>(st + EV.off_iacq) : nullptr,
+                            EV.info.order_dev ? reinterpret_cast<int32_t*>(st + EV.off_iord) : nullptr
+#endif
+                            };
         const int64_t n0 = ((int64_t)blockIdx.x + (int64_t)k * gridDim.x) * E;
         mbar_wait(&full[s], (uint32_t)((k / S) & 1));
 #if IMX_USE_STEP_ET
-        tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV>(A, TLY, T, tid, A.t, n0, []() {});
+        tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV, false, (bool)IMX_EVAL>(A, TLY, T, tid, A.t, n0, []() {});
+#if IMX_EVAL
+        if (EV.eval) step_eval_env_pass(A, TLY, EV, st, tid);           // this thread simulated env tid
+#endif
 #else
         // replayed / Philox noisy-delay outcome of this lane's (env, stage) for this period (written by reset(), long complete)
         const bool delayed = (KF(noisy) && L.ok) ? (A.mask_T[((int64_t)A.t * A.N + n0 + L.e_loc) * m + L.i] != 0) : false;
-        tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, false>(A, TLY, T, L, A.t, 0, n0, delayed, []() {});
+        tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, false, false, (bool)IMX_EVAL>(A, TLY, T, L, A.t, 0, n0, delayed, []() {});
+#if IMX_EVAL
+        if (EV.eval) {                               // the env's cells sit in this warp: no barrier across compute warps
+            __syncwarp();
+            if (L.ok && L.i == 0) step_eval_env_pass(A, TLY, EV, st, L.e_loc);
+        }
+#endif
 #endif
         if (KHAS(cc)) cc_build<MAXC>(A, TLY, T, st, L, CT);
         fence_proxy_async_smem();                    // this thread's tile writes, before the bulk engine reads them

@@ -47,6 +47,27 @@ struct TileLayout {
 #define IMX_REC 0
 #endif
 
+// One step with its period's bookkeeping (imx_step_eval): a compile-time flag of the specialised build, so the modules without
+// it (IMX_K_has_eval undefined) contain none of this code.
+#if defined(IMX_JIT) && defined(IMX_K_has_eval) && IMX_K_has_eval
+#define IMX_EVAL 1
+#else
+#define IMX_EVAL 0
+#endif
+
+// imx_step_eval's outputs beyond StepArgs.  For one episode the returns and the accumulators are per-env state: their tiles are
+// loaded with the state tile (not at period 0, where they start at 0.0) and stored with it.  The regions sit behind
+// TileLayout.total, each reserved only when its output is asked for; `total` is the stage size of the call.
+struct StepEvalArgs {
+    double* __restrict__ ret;             // [N][m] / [N] episode returns, or null
+    double* __restrict__ eval;            // [N][4 + m] evaluation-loop accumulators, or null
+    imx_info_out info;                    // [N][m] diagnostics of the period; NULL fields are not written
+    int32_t off_ret, off_eval, off_prof;  // [E][m] / [E] float64, [E][4 + m] float64, [E][m] float64 (eval or info.profit_dev)
+    int32_t off_idem, off_iship, off_iacq, off_iord;   // [E][m] int32 diagnostics tiles
+    int32_t total;                        // dynamic shared memory bytes of one tile (one ring stage)
+    int32_t rescaled;                     // the state is standardised: the accumulators undo the scaling (rev_scale)
+};
+
 // One whole stored-plan episode per launch (imx_replay_episode, step_kernel_tma_episode): what the kernel needs beyond the
 // multi-period StepArgs.  The episode regions of shared memory sit behind TileLayout.total2 (the per-period demand rows of
 // that layout are unused: the episode's whole trace is resident instead).
@@ -245,8 +266,10 @@ __device__ __forceinline__ LaneCtx<MAXC> make_lane_ctx(const StepArgs& A, int ti
 // writes (a multi-period launch waits there for the previous period's bulk stores).  No barriers or fences in here:
 // the caller orders the tile's loads before and its stores after.
 //   j = period index inside the launch (diagnostics block, MANY only), t = period being simulated, n0 = first env of the tile
-//   EP: episode kernel — S.dem is the tile's whole [E][R][T] trace, and the profits go to S.prof when it is set
-template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, bool EP = false, typename BeforeStore>
+//   EP: episode kernel — S.dem is the tile's whole [E][R][T] trace
+//   OUT: the period's bookkeeping tiles — profits to S.prof, the diagnostics tiles (records or imx_step_eval's info), the reward
+//        added into S.ret (from 0.0 at period 0 outside the episode kernel, whose returns start zeroed) — each when it is set
+template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, bool EP = false, bool OUT = EP, typename BeforeStore>
 __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout& TLY, const TileSmem& S, const LaneCtx<MAXC>& L,
                                             int t, int j, int64_t n0, bool delayed, BeforeStore&& before_store) {
     const NodeParams& np = L.np;
@@ -425,16 +448,17 @@ __device__ __forceinline__ void tile_period(const StepArgs& A, const TileLayout&
         }
         if (KF(multi)) S.rew[cell] = reward_out;
         else if (i == 0) S.rew[e_loc] = reward_out;
-        if (EP && S.prof) S.prof[cell] = profit;
-        if (EP && IMX_REC) {                         // records: the period's diagnostics into their tiles (stored by the caller)
+        if (OUT && S.prof) S.prof[cell] = profit;
+        if (OUT && (IMX_REC || IMX_EVAL)) {          // the period's diagnostics into their tiles (stored by the caller)
             if (S.rdem) S.rdem[cell] = demand;
             if (S.rship) S.rship[cell] = ship;
             if (S.racq) S.racq[cell] = acq;
             if (S.rord) S.rord[cell] = order;
         }
-        if (EP && S.ret) {                           // stats_slice_kernel<true>'s order: from 0, period by period
-            if (KF(multi)) S.ret[cell] = __dadd_rn(S.ret[cell], reward_out);
-            else if (i == 0) S.ret[e_loc] = __dadd_rn(S.ret[e_loc], reward_out);
+        if (OUT && S.ret) {                          // stats_slice_kernel<true>'s order: from 0, period by period
+            const bool fresh = !EP && t == 0;        // (the returns tile is not loaded at period 0)
+            if (KF(multi)) S.ret[cell] = __dadd_rn(fresh ? 0.0 : S.ret[cell], reward_out);
+            else if (i == 0) S.ret[e_loc] = __dadd_rn(fresh ? 0.0 : S.ret[e_loc], reward_out);
         }
 #ifdef IMX_OBS_ROTATE
         {
@@ -553,8 +577,8 @@ __device__ __forceinline__ void cc_build(const StepArgs& A, const TileLayout& TL
 // Used for the divergent networks, whose lanes = nodes kernels are issue-bound (profiles/r2_ncu_div2_step_kernel_lanes.txt).
 #if defined(IMX_JIT) && defined(IMX_STEP_ET) && IMX_STEP_ET
 #define IMX_USE_STEP_ET 1
-// EP: episode kernel (as in tile_period; the noisy-delay outcomes come from episode_delayed)
-template <int M, int DMAX, int PMAX, int MAXC, bool DIV, bool EP = false, typename BeforeStore>
+// EP: episode kernel (as in tile_period; the noisy-delay outcomes come from episode_delayed); OUT: as in tile_period
+template <int M, int DMAX, int PMAX, int MAXC, bool DIV, bool EP = false, bool OUT = EP, typename BeforeStore>
 __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayout& TLY, const TileSmem& S, int e, int t, int64_t n0,
                                                BeforeStore&& before_store, const EpisodeArgs* EA = nullptr) {
     constexpr int INV_MAX[M] = {IMX_L_inv_max}, ORDER_MAX[M] = {IMX_L_order_max}, DEMAND_MAX[M] = {IMX_L_demand_max};
@@ -702,8 +726,8 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
                 if (k < NCHILD[j]) S.bt[e * KF(NB) + BT_OFF[j] + k] = bt[j][k];
         }
         if (KF(multi)) S.rew[c0 + j] = reward[j];
-        if (EP && S.prof) S.prof[c0 + j] = profit[j];
-        if (EP && IMX_REC) {                         // records, as in tile_period
+        if (OUT && S.prof) S.prof[c0 + j] = profit[j];
+        if (OUT && (IMX_REC || IMX_EVAL)) {          // diagnostics tiles, as in tile_period
             if (S.rdem) S.rdem[c0 + j] = demand[j];
             if (S.rship) S.rship[c0 + j] = ship[j];
             if (S.racq) S.racq[c0 + j] = acq[j];
@@ -717,9 +741,11 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
         }
     }
     if (!KF(multi)) S.rew[e] = reward[0];
-    if (EP && S.ret) {                               // stats_slice_kernel<true>'s order: from 0, period by period
+    if (OUT && S.ret) {                              // stats_slice_kernel<true>'s order: from 0, period by period
+        const bool fresh = !EP && t == 0;            // (as in tile_period)
 #pragma unroll
-        for (int j = 0; j < (KF(multi) ? M : 1); ++j) S.ret[e * (KF(multi) ? M : 1) + j] = __dadd_rn(S.ret[e * (KF(multi) ? M : 1) + j], reward[j]);
+        for (int j = 0; j < (KF(multi) ? M : 1); ++j)
+            S.ret[e * (KF(multi) ? M : 1) + j] = __dadd_rn(fresh ? 0.0 : S.ret[e * (KF(multi) ? M : 1) + j], reward[j]);
     }
     if (DIV && err_code != 0) A.err[n0 + e] = err_code;
 }
@@ -727,18 +753,20 @@ __device__ __forceinline__ void tile_period_et(const StepArgs& A, const TileLayo
 #define IMX_USE_STEP_ET 0
 #endif
 
-// Episode kernel with evaluation accumulators, after each period: thread e repeats eval_accumulate_kernel's float64 operations
-// in its order on the observation elements the step writes (obs[i][0] = inventory, obs[i][1] = backlog: rounded to the
-// observation element type and widened back) and on the period's profits.
-__device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs& EA, unsigned char* smem, int e) {
+// Evaluation accumulators after a period (episode kernel, imx_step_eval): thread e repeats eval_accumulate_kernel's float64
+// operations in its order on the observation elements the step writes (obs[i][0] = inventory, obs[i][1] = backlog: rounded to
+// the observation element type and widened back) and on the period's profits.  `smem` is the tile's base; off_eval / off_prof
+// its accumulator and profit regions.
+__device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLayout& TLY, unsigned char* smem, int32_t off_eval,
+                                                 int32_t off_prof, int32_t rescaled, int e) {
     const int m = KF(m);
     const int cols = KF(multi) ? m : 1;
     const double* rew = reinterpret_cast<const double*>(smem + KT(off_rew)) + e * cols;
     {
-        double* row = reinterpret_cast<double*>(smem + EA.off_eval) + e * (4 + m);
+        double* row = reinterpret_cast<double*>(smem + off_eval) + e * (4 + m);
         const int32_t* inv = reinterpret_cast<const int32_t*>(smem + KT(off_inv)) + e * m;
         const int32_t* bl = reinterpret_cast<const int32_t*>(smem + KT(off_bl)) + e * m;
-        const double* prof = reinterpret_cast<const double*>(smem + EA.off_prof) + e * m;
+        const double* prof = reinterpret_cast<const double*>(smem + off_prof) + e * m;
         double ep = row[0], step_inv = 0.0, step_bl = 0.0, cust = 0.0;
         if (!KF(multi)) ep = __dadd_rn(ep, rew[0]);
         for (int i = 0; i < m; ++i) {
@@ -754,7 +782,7 @@ __device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLa
             }
             x0 = obs_stored(KF(obs_type), x0);
             x1 = obs_stored(KF(obs_type), x1);
-            if (EA.rescaled) {
+            if (rescaled) {
                 x0 = rev_scale_dev(x0, inv_max, A.a, A.bma);         // the loops use inv_max for BOTH fields
                 x1 = rev_scale_dev(x1, inv_max, A.a, A.bma);
             }
@@ -771,13 +799,33 @@ __device__ __forceinline__ void episode_env_pass(const StepArgs& A, const TileLa
     }
 }
 
+#if IMX_EVAL
+// imx_step_eval's accumulator pass for env e of the tile at `smem`: at period 0 the row starts at 0.0 (its tile was not loaded),
+// which is imx_eval_accumulate(reset = 1).  The caller has made the env's tiles of this period visible to this thread.
+__device__ __forceinline__ void step_eval_env_pass(const StepArgs& A, const TileLayout& TLY, const StepEvalArgs& EV, unsigned char* smem,
+                                                   int e) {
+    if (A.t == 0) {
+        double* row = reinterpret_cast<double*>(smem + EV.off_eval) + e * (4 + KF(m));
+#pragma unroll
+        for (int c = 0; c < 4 + KF(m); ++c) row[c] = 0.0;
+    }
+    episode_env_pass(A, TLY, smem, EV.off_eval, EV.off_prof, EV.rescaled, e);
+}
+#define IMX_EVAL_PARAM , const __grid_constant__ StepEvalArgs EV
+#else
+#define IMX_EVAL_PARAM
+#endif
+
 // MANY = false: one period per launch (the loop below folds away); MANY = true: A.periods periods per launch with the
 // tile's state resident in shared memory (imx_step_many) — separate kernels because the loop costs registers.
 // EPISODE (with MANY): a whole episode from period 0 (imx_replay_episode) — the state starts as reset_kernel writes it instead
 // of being loaded, the tile's demand trace is resident for the whole episode, rewards are stored only when A.reward is set,
 // and returns / evaluation accumulators are kept in shared memory and stored once.
+// EV (one period, imx_step_eval modules only): returns / accumulator tiles travel with the state, diagnostics tiles are stored
+// next to it, and the rewards are stored only when A.reward is set.
 template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV, bool MANY, bool EPISODE = false>
-__device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs* EA = nullptr) {
+__device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& TLY, const EpisodeArgs* EA = nullptr,
+                                          const StepEvalArgs* EV = nullptr) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) uint64_t bar[2];         // bar[b]: inputs of the periods with parity b (bar[0] also the state)
 
@@ -794,6 +842,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     const int64_t n0 = (int64_t)blockIdx.x * E;      // first env of the tile
     const int K = MANY ? A.periods : 1;              // periods this launch advances
     constexpr bool REC = EPISODE && IMX_REC;         // the episode kernel streams out per-period records
+    constexpr bool SE = IMX_EVAL && !MANY && !EPISODE;   // imx_step_eval's bookkeeping
 
     int32_t* s_inv = reinterpret_cast<int32_t*>(smem + KT(off_inv));
     int32_t* s_bl = reinterpret_cast<int32_t*>(smem + KT(off_bl));
@@ -847,7 +896,13 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
         if (KF(need_ho)) bytes += b_hist;
         if (KF(has_carry)) bytes += b_cell4;
         if (DIV && KF(NB) > 0) bytes += b_bt;
+        const uint32_t b_ret = (uint32_t)E * (KF(multi) ? m : 1) * 8u, b_eval = (uint32_t)E * (4 + m) * 8u;
+        const bool se_load = SE && A.t > 0;          // returns / accumulators continue the episode
+        if (se_load && EV->ret) bytes += b_ret;
+        if (se_load && EV->eval) bytes += b_eval;
         mbar_expect_tx(&bar[0], bytes);
+        if (se_load && EV->ret) bulk_load_g2s(smem + EV->off_ret, EV->ret + n0 * (KF(multi) ? m : 1), b_ret, &bar[0]);
+        if (se_load && EV->eval) bulk_load_g2s(smem + EV->off_eval, EV->eval + n0 * (4 + m), b_eval, &bar[0]);
         load_inputs(0);
         bulk_load_g2s(s_inv, A.inv + n0 * m, b_cell4, &bar[0]);
         bulk_load_g2s(s_bl, A.backlog + n0 * m, b_cell4, &bar[0]);
@@ -912,12 +967,17 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     mbar_wait(&bar[b], (uint32_t)((j >> 1) & 1));
 
     auto rec_tile = [&](const void* out, int32_t off) { return (REC && out) ? reinterpret_cast<int32_t*>(smem + off) : nullptr; };
+    auto se_tile = [&](const void* out, int32_t off) { return (SE && out) ? reinterpret_cast<int32_t*>(smem + off) : nullptr; };
     const TileSmem S = {s_act, EPISODE ? reinterpret_cast<const int32_t*>(smem + EA->off_edem) : s_dem, s_inv, s_bl, s_ou, s_pipe, s_hd,
                         s_ho, s_carry, s_bt, s_obs, s_rew,
-                        (EPISODE && (EA->eval || (REC && EA->rec.profit_dev))) ? reinterpret_cast<double*>(smem + EA->off_prof) : nullptr,
-                        (EPISODE && EA->ret) ? reinterpret_cast<double*>(smem + EA->off_ret) : nullptr,
-                        REC ? rec_tile(EA->rec.demand_dev, EA->off_rdem) : nullptr, REC ? rec_tile(EA->rec.ship_dev, EA->off_rship) : nullptr,
-                        REC ? rec_tile(EA->rec.acquisition_dev, EA->off_racq) : nullptr, REC ? rec_tile(EA->rec.order_dev, EA->off_rord) : nullptr};
+                        (EPISODE && (EA->eval || (REC && EA->rec.profit_dev))) ? reinterpret_cast<double*>(smem + EA->off_prof)
+                        : (SE && (EV->eval || EV->info.profit_dev)) ? reinterpret_cast<double*>(smem + EV->off_prof) : nullptr,
+                        (EPISODE && EA->ret) ? reinterpret_cast<double*>(smem + EA->off_ret)
+                        : (SE && EV->ret) ? reinterpret_cast<double*>(smem + EV->off_ret) : nullptr,
+                        REC ? rec_tile(EA->rec.demand_dev, EA->off_rdem) : SE ? se_tile(EV->info.demand_dev, EV->off_idem) : nullptr,
+                        REC ? rec_tile(EA->rec.ship_dev, EA->off_rship) : SE ? se_tile(EV->info.ship_dev, EV->off_iship) : nullptr,
+                        REC ? rec_tile(EA->rec.acquisition_dev, EA->off_racq) : SE ? se_tile(EV->info.acquisition_dev, EV->off_iacq) : nullptr,
+                        REC ? rec_tile(EA->rec.order_dev, EA->off_rord) : SE ? se_tile(EV->info.order_dev, EV->off_iord) : nullptr};
     // The state tiles are rewritten in place, and with records they are also the source of bulk stores (row 0 from the
     // prologue, row t + 1 after period t), as are the record and profit tiles.  tile_period / tile_period_et write all of them
     // only after this hook, whose bulk_wait_read_all drains every earlier bulk read of the tile: keep it that way.  Period 0
@@ -929,10 +989,19 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
         }
     };
 #if IMX_USE_STEP_ET
-    tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV, EPISODE>(A, TLY, S, tid, t, n0, before_store, EA);
+    tile_period_et<IMX_K_m, DMAX, PMAX, MAXC, DIV, EPISODE, EPISODE || SE>(A, TLY, S, tid, t, n0, before_store, EA);
     (void)L; (void)delayed;
+#if IMX_EVAL
+    if (SE && EV->eval) step_eval_env_pass(A, TLY, *EV, smem, tid);     // this thread simulated env tid
+#endif
 #else
-    tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, MANY, EPISODE>(A, TLY, S, L, t, j, n0, delayed, before_store);
+    tile_period<M_PAD, DMAX, PMAX, MAXC, DIV, MANY, EPISODE, EPISODE || SE>(A, TLY, S, L, t, j, n0, delayed, before_store);
+#if IMX_EVAL
+    if (SE && EV->eval) {                            // the env's cells sit in this warp: no barrier across warps
+        __syncwarp();
+        if (ok && i == 0) step_eval_env_pass(A, TLY, *EV, smem, e_loc);
+    }
+#endif
 #endif
     if (!MANY && KHAS(cc)) cc_build<MAXC>(A, TLY, S, smem, L, (int)blockDim.x);
     fence_proxy_async_smem();          // every writer orders its generic-proxy stores before the bulk copies
@@ -940,8 +1009,18 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
     if (tid == 0) {
         if (!MANY && KHAS(cc)) bulk_store_only(reinterpret_cast<unsigned char*>(A.cc) + n0 * m * A.cc_W * es, smem + KT(off_cc), (uint32_t)E * m * A.cc_W * es);
         if (KHAS(obs)) bulk_store_only(reinterpret_cast<unsigned char*>(A.obs) + (int64_t)j * A.obs_stride_bytes + n0 * m * O * es, s_obs, (uint32_t)E * m * O * es);
-        if (!EPISODE || A.reward)
+        if (!(EPISODE || SE) || A.reward)
             bulk_store_only(A.reward + (int64_t)j * A.rew_stride + (KF(multi) ? n0 * m : n0), s_rew, KF(multi) ? b_cell8 : (uint32_t)E * 8u);
+        if (SE) {                      // returns and accumulators leave with the state, the diagnostics next to them
+            const imx_info_out& I = EV->info;
+            if (EV->ret) bulk_store_only(EV->ret + n0 * (KF(multi) ? m : 1), smem + EV->off_ret, (uint32_t)E * (KF(multi) ? m : 1) * 8u);
+            if (EV->eval) bulk_store_only(EV->eval + n0 * (4 + m), smem + EV->off_eval, (uint32_t)E * (4 + m) * 8u);
+            if (I.demand_dev) bulk_store_only(I.demand_dev + n0 * m, smem + EV->off_idem, b_cell4);
+            if (I.ship_dev) bulk_store_only(I.ship_dev + n0 * m, smem + EV->off_iship, b_cell4);
+            if (I.acquisition_dev) bulk_store_only(I.acquisition_dev + n0 * m, smem + EV->off_iacq, b_cell4);
+            if (I.order_dev) bulk_store_only(I.order_dev + n0 * m, smem + EV->off_iord, b_cell4);
+            if (I.profit_dev) bulk_store_only(I.profit_dev + n0 * m, smem + EV->off_prof, b_cell8);
+        }
         if (j == K - 1) {              // the tile's state leaves the SM once per launch
             bulk_store_only(A.inv + n0 * m, s_inv, b_cell4);
             bulk_store_only(A.backlog + n0 * m, s_bl, b_cell4);
@@ -971,7 +1050,7 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
         }
     }
     // (reads this period's reward / state / profit tiles: the next period overwrites them only behind its before_store barrier)
-    if (EPISODE && EA->eval && tid < E) episode_env_pass(A, TLY, *EA, smem, tid);
+    if (EPISODE && EA->eval && tid < E) episode_env_pass(A, TLY, smem, EA->off_eval, EA->off_prof, EA->rescaled, tid);
     }   // periods
     if (EPISODE && (EA->ret || EA->eval)) {      // returns and accumulator rows leave the SM once per episode
         fence_proxy_async_smem();
@@ -993,8 +1072,12 @@ __device__ __forceinline__ void step_tile(const StepArgs& A, const TileLayout& T
 #define IMX_STEP_BOUNDS __launch_bounds__(TMA_THREADS)
 #endif
 template <int M_PAD, int DMAX, int PMAX, int MAXC, bool DIV>
-__global__ void IMX_STEP_BOUNDS step_kernel_tma(const __grid_constant__ StepArgs A, const __grid_constant__ TileLayout TLY) {
+__global__ void IMX_STEP_BOUNDS step_kernel_tma(const __grid_constant__ StepArgs A, const __grid_constant__ TileLayout TLY IMX_EVAL_PARAM) {
+#if IMX_EVAL
+    step_tile<M_PAD, DMAX, PMAX, MAXC, DIV, false>(A, TLY, nullptr, &EV);
+#else
     step_tile<M_PAD, DMAX, PMAX, MAXC, DIV, false>(A, TLY);
+#endif
 }
 
 // A.periods periods per launch (imx_step_many).  The runtime-specialised build bounds its registers (IMX_MANY_MAXNREG,

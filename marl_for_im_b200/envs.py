@@ -731,6 +731,81 @@ class _ImxEnvBase:
             self.last_reward = rew[T - 1]
         return {"returns": ret, "stats": stats, "obs": obs, "rewards": rew, "eval": ev, "records": recs}
 
+    # step_eval(return_info=True): info key -> field of imx_info_out, dtype
+    INFO_FIELDS = {"demand": ("demand_dev", torch.int32), "ship": ("ship_dev", torch.int32),
+                   "acquisition": ("acquisition_dev", torch.int32), "actual order": ("order_dev", torch.int32),
+                   "profit": ("profit_dev", torch.float64)}
+
+    def _f64_out(self, x, shape, name):
+        if x is not None and (not isinstance(x, torch.Tensor) or x.dtype != torch.float64 or not x.is_contiguous()
+                              or tuple(x.shape) != tuple(shape) or x.device.type != self.device.type
+                              or (self.device.index is not None and x.device.index != self.device.index)):
+            raise ValueError(f"{name} must be a contiguous float64 tensor of shape {list(shape)} on {self.device}")
+        return x
+
+    def step_eval(self, action, returns=None, eval_acc=None, want_obs=True, want_rewards=True, return_info=False,
+                  _out=None):
+        """``step()`` with the bookkeeping of a closed-loop evaluation period (the evaluation loops that step a policy one period
+        at a time, MA_inv_management.py:517-587, inv_management.py:567-606): the reward is added into ``returns`` ([N, m] /
+        [N]) and ``eval_acc`` ([N, 4 + m]) accumulates what ``eval_accumulate`` would, both starting afresh at period 0 —
+        after T calls on a stored plan they equal ``replay_episode``'s ``returns`` / ``eval``.  Both are caller-owned contiguous
+        float64 tensors on the env's device (or None).  One kernel launch where the batch allows it.
+        Returns ``(obs [N, m, O], reward [N, m] / [N], done, info)`` as packed tensors, None for what was not asked for; ``info``
+        is a dict of ``[N, m]`` tensors with the keys of ``step_many(return_info=True)``."""
+        if not self.batched:
+            raise _lib.ImxError("step_eval is a batched-mode call (construct the env with num_envs=N)")
+        N, m = self.num_envs, self.num_nodes
+        self._f64_out(returns, (N, m) if self.MULTI else (N,), "returns")
+        self._f64_out(eval_acc, (N, 4 + m), "eval_acc")
+        act = self._actions_to_device(action)
+        obs_buf, rew_buf, info = _out if _out is not None else (
+            self._new_obs() if want_obs else None, self._new_reward() if want_rewards else None,
+            {k: torch.empty((N, m), dtype=dt, device=self.device) for k, (_, dt) in self.INFO_FIELDS.items()} if return_info else None)
+        info_struct = _lib.ImxInfoOut(**{f: info[k].data_ptr() for k, (f, _) in self.INFO_FIELDS.items()}) if info is not None else None
+        p = lambda x: C.c_void_p(x.data_ptr()) if x is not None else None   # noqa: E731
+        _lib.check(self._lib.imx_step_eval(self._handle, p(act), p(obs_buf), p(rew_buf),
+                                           C.byref(info_struct) if info_struct is not None else None, p(returns), p(eval_acc),
+                                           self._stream()))
+        self._keepalive_eval_step = act
+        if obs_buf is not None:
+            self.last_obs = obs_buf
+        if rew_buf is not None:
+            self.last_reward = rew_buf
+        return obs_buf, rew_buf, self.period >= self.num_periods, info
+
+    def evaluate_policy(self, policy, customer_demand=None, delay_mask=None, noisy_delay=None, stats=None, accumulate=False,
+                        eval_acc=False, want_rewards=False, return_info=False):
+        """One closed-loop evaluation episode of the whole batch: ``reset(customer_demand, ...)``, then for t < T
+        ``actions = policy(obs, t)`` on the packed observation ``[N, m, O]`` and ``step_eval`` (one launch per period: the policy
+        needs each period's observation).  ``noisy_delay`` / ``delay_mask`` as in ``reset()``; ``stats`` / ``accumulate`` as in
+        ``replay_episode``.  Returns ``dict(returns, stats, eval [N, 4 + m], rewards [T, N(, m)], info)`` with None for what
+        was not asked; ``info`` holds ``[T, N, m]`` tensors with the keys of ``step_many(return_info=True)``.  With
+        ``policy = lambda obs, t: plan[t]`` the results equal ``replay_episode(plan, ...)``'s."""
+        if not self.batched:
+            raise _lib.ImxError("evaluate_policy is a batched-mode call (construct the env with num_envs=N)")
+        N, m, T = self.num_envs, self.num_nodes, self.num_periods
+        cols = (m,) if self.MULTI else ()
+        f64 = dict(dtype=torch.float64, device=self.device)
+        if stats is True:
+            stats = torch.zeros(3 + (2 * m if self.MULTI else 0), **f64)
+        elif stats is False:
+            stats = None
+        if stats is not None:
+            self._f64_out(stats, (3 + (2 * m if self.MULTI else 0),), "stats")
+        ret = torch.empty((N,) + cols, **f64)
+        ev = torch.empty((N, 4 + m), **f64) if eval_acc else None
+        rew = torch.empty((T, N) + cols, **f64) if want_rewards else None
+        info = {k: torch.empty((T, N, m), dtype=dt, device=self.device) for k, (_, dt) in self.INFO_FIELDS.items()} if return_info else None
+        self.reset(customer_demand, noisy_delay=bool(noisy_delay), noisy_delay_threshold=self.noisy_delay_threshold,
+                   delay_mask=delay_mask)
+        obs = self.last_obs
+        for t in range(T):
+            out = (self._new_obs(), rew[t] if rew is not None else None, {k: v[t] for k, v in info.items()} if info is not None else None)
+            obs, _, _, _ = self.step_eval(policy(obs, t), returns=ret, eval_acc=ev, _out=out)
+        if stats is not None:
+            self.episode_stats(ret.unsqueeze(0), stats=stats, accumulate=accumulate)
+        return {"returns": ret, "stats": stats, "eval": ev, "rewards": rew, "info": info}
+
     # ------------------------------------------------------------------ drop-in mode histories
     def _alloc_histories(self):
         T, m = self.num_periods, self.num_nodes

@@ -342,9 +342,10 @@ int imx_eval_stats(imx_env* env, const double* acc_dev, double* stats_dev, int a
  * observation of CC_inv_management.py:516-528): for every agent the flat vector
  * [opponent_action (m-1) | opponent_obs (m-1)*O | own_obs O], W = imx_cc_obs_len() values.
  *   obs_dev      [N][m][O] in the element type this env writes (float64, float32 with cfg.obs_f32, bfloat16 with IMX_IO_OBS_BF16)
- *   actions_dev  [N][m] actions of the same step in the handle's action type, clipped to [clip_lo, clip_hi]; NULL = zeros
+ *   actions_dev  [N][m] actions of the same step in the handle's action type, clipped to [clip_lo, clip_hi] as np.clip clips
+ *                (a NaN action stays NaN, -0.0 stays -0.0, clip_lo > clip_hi gives clip_hi); NULL = zeros
  *   out_dev      [N][m][W] float64 (out_is_f32 = 0), float32 (1: RLlib casts observations to float32) or bfloat16 (2: the
- *                round-to-nearest-even of the float32 value) */
+ *                round-to-nearest-even of the float32 value; a NaN action becomes the NaN 0x7FFF) */
 int imx_cc_obs_len(const imx_env* env);
 int imx_cc_observe(imx_env* env, const void* obs_dev, const void* actions_dev, double clip_lo, double clip_hi,
                    void* out_dev, int out_is_f32, void* stream);
@@ -354,9 +355,10 @@ int imx_cc_observe(imx_env* env, const void* obs_dev, const void* actions_dev, d
  * writes them with one bulk store per tile next to obs / reward / state (no second pass over [N][m][O]).
  *   obs_dev     [N][m][O] or NULL (the rows still contain every agent's observation)
  *   cc_dev      [N][m][W], W = imx_cc_obs_len(), in the observation element type (float64, float32 or bfloat16)
- *   fill_actions non-zero: opponent-action slots = this step's actions clipped to [clip_lo, clip_hi] (FillInActions,
- *               models/CC_Model.py:165-193; the evaluation loops' hand-built rows, CC_inv_management.py:516-528); zero: zeros, as
- *               central_critic_observer leaves them at sampling time (:196-214)
+ *   fill_actions non-zero: opponent-action slots = this step's actions clipped to [clip_lo, clip_hi] as imx_cc_observe clips
+ *               them, like np.clip: a NaN action stays NaN (FillInActions, models/CC_Model.py:165-193; the evaluation loops'
+ *               hand-built rows, CC_inv_management.py:516-528); zero: zeros, as central_critic_observer leaves them at
+ *               sampling time (:196-214)
  * Fused wherever the runtime-specialised TMA kernels serve the whole batch (N a multiple of the tile size, 16-byte aligned
  * buffers); otherwise imx_step followed by imx_cc_observe — same bytes either way.  Multi-agent kinds only. */
 int imx_step_cc(imx_env* env, const void* actions_dev, void* obs_dev, void* cc_dev, int fill_actions, double clip_lo,

@@ -547,8 +547,14 @@ static void jit_spec(const imx_env* e, int variant, imxjit::Spec& sp, int smem[i
     const int64_t pipe_smem = (int64_t)pipe_stages_for(e, L) * L.total;
     if (e->pipe_mode >= 0 && pipe_smem <= 200 * 1024) {
         defs.push_back("IMX_PIPE_STAGES=" + std::to_string(pipe_stages_for(e, L)));
+        // the critic-row kernel of the 2-wide tile (config 5): left alone, ptxas keeps values of the 2-stage chain's tile loop in
+        // local memory (8-16 bytes of stack, a load after every stage wait); 56 registers keep them in registers.  us per period
+        // at 65 536 envs, B200 at 1000 W, bound / none: 2 stages float64 9.06 / 9.12, float32 5.19 / 5.32, bfloat16 5.12 / 5.33;
+        // 1 stage (no spill either way) float64 3.83 / 3.89, float32 3.07 / 3.07, bfloat16 3.11 / 3.13.
+        // IMX_PIPE_MAXNREG overrides (0: no bound).
         const char* pr = getenv("IMX_PIPE_MAXNREG");
-        if (pr && atoi(pr) > 0) defs.push_back("IMX_PIPE_MAXNREG=" + std::to_string(atoi(pr)));
+        const int pbound = pr ? atoi(pr) : (has_cc && m_pad_of(e) == 2 ? 56 : 0);
+        if (pbound > 0) defs.push_back("IMX_PIPE_MAXNREG=" + std::to_string(pbound));
         sp.name[3] = "imx::step_kernel_pipe" + targs;
     }
     sp.name[4] = "";

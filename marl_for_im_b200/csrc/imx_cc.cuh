@@ -35,7 +35,7 @@ __global__ void __launch_bounds__(256) cc_observer_kernel(const InT* __restrict_
         double v;
         if (w < m - 1) {
             const int j = w < i ? w : w + 1;
-            v = actions ? fmin(fmax(load_action(actions, n * m + j, act_f32 != 0), lo), hi) : 0.0;
+            v = actions ? clip_np(load_action(actions, n * m + j, act_f32 != 0), lo, hi) : 0.0;
         } else if (w < (m - 1) * (1 + O)) {
             const int q = w - (m - 1);
             const int slot = q / O, k = q - slot * O;

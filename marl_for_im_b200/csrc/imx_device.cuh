@@ -230,7 +230,8 @@ __device__ __forceinline__ double div_by_m(double s, int m, double inv_m, bool m
 enum : int { OBS_F64 = 0, OBS_F32 = 1, OBS_BF16 = 2 };
 __host__ __device__ constexpr int obs_elem_bytes(int type) { return type == OBS_BF16 ? 2 : type == OBS_F32 ? 4 : 8; }
 
-// float32 -> bfloat16 bits, round to nearest even (one F2FP; observations are never NaN)
+// float32 -> bfloat16 bits, round to nearest even (one F2FP; a NaN, which only a critic row's opponent action can be,
+// becomes the canonical NaN 0x7FFF)
 __device__ __forceinline__ uint16_t f32_to_bf16(float x) {
     uint16_t r;
     asm("cvt.rn.bf16.f32 %0, %1;" : "=h"(r) : "f"(x));
@@ -246,6 +247,13 @@ __device__ __forceinline__ double obs_stored(int type, double x) {
 // One action element, widened to float64 (exact for float32, so decode_order sees the same value a float64 caller passes)
 __device__ __forceinline__ double load_action(const void* __restrict__ p, int64_t k, bool f32) {
     return f32 ? (double)reinterpret_cast<const float*>(p)[k] : reinterpret_cast<const double*>(p)[k];
+}
+// v clipped to [lo, hi] as the oracle's min(max(v, lo), hi) and np.clip do, operands in that order: a NaN stays NaN, -0.0
+// stays -0.0 against a bound of +0.0, and lo > hi gives hi.  (fmax returns the other operand when one is NaN, and picks
+// +0.0 over -0.0.)
+__device__ __forceinline__ double clip_np(double v, double lo, double hi) {
+    const double t = (lo > v) ? lo : v;
+    return (hi < t) ? hi : t;
 }
 
 // Reduced-precision observations: the table entry rounded on the host (float32: (float)tab[v] == np.float32(obs64); bfloat16:

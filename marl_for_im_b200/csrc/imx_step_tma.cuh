@@ -529,7 +529,7 @@ __device__ __forceinline__ void cc_build_row(const StepArgs& A, const TileSmem& 
 #pragma unroll
     for (int q = 0; q < m - 1; ++q) {
         const int j = q + (q >= L.i ? 1 : 0);
-        const double v = A.cc_fill ? fmin(fmax(load_action(S.act, e0 + j, KF(act_f32) != 0), A.cc_lo), A.cc_hi) : 0.0;
+        const double v = A.cc_fill ? clip_np(load_action(S.act, e0 + j, KF(act_f32) != 0), A.cc_lo, A.cc_hi) : 0.0;
         if constexpr (sizeof(ObsT) == 2) row[k++] = f32_to_bf16((float)v);
         else if constexpr (sizeof(ObsT) == 4) row[k++] = __float_as_uint((float)v);
         else row[k++] = (unsigned long long)__double_as_longlong(v);
